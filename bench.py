@@ -2,7 +2,7 @@
 """Benchmarks of the DRMNet rendering hot path on B200 -- BASELINE.json metric and configs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload render|img2refmap|synth|sampling] [--batch B] [--footprint auto|S]
+                    [--workload render|img2refmap|synth|sampling] [--batch B] [--footprint auto|S] [--dump-outputs DIR]
 
 workload  (a step is one pass of the hot path over one batch of synthetic input, per GPU; weak scaling over ranks)
   render      BASELINE config[1] -- THE HEADLINE: 64 synthetic 2000x1000 envmaps x random BRDF parameters
@@ -23,6 +23,12 @@ cpu_baseline  render: the fp64 oracle port (C + OpenMP, all host cores) on a bou
               img2refmap: the numpy oracle port on one image of the batch (rank 0 only)
 Multi-GPU: every rank owns its own envmaps; the rendered refmaps are gathered by ONE equal-count all_gather on a side
 stream (drmnet_b200.dist.RefmapGather); `rank_ms` lists every rank's own step time.
+
+--dump-outputs DIR  (e.g. bench_outputs, which git ignores) after the timed steps, rank 0 writes what the last timed
+              step returned (the gathered refmaps under multi-GPU) as DIR/<name>.npy, float32 (float64 stays float64).
+              The inputs are seeded, so two builds run with the same arguments can be compared array for array.  Past
+              64 MB in all, every array is cut to the same seeded sample of its flattened elements and
+              DIR/<name>.sample_index.npy holds their positions.
 """
 from __future__ import annotations
 
@@ -38,6 +44,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 HE, WE, RES = 1000, 2000, 128
 ALG_BYTES_PER_REFMAP = HE * WE * 3 * 4 + RES * RES * 3 * 4 + 40  # SURVEY 8d: 24 196 648
@@ -163,7 +170,7 @@ def wl_render(args, rank, dev):
 
     return dict(step=step, e2e_step=e2e_step, units=batch, alg_bytes=batch * ALG_BYTES_PER_REFMAP, gather=True,
                 h2d=host_envs.numel() * 4 + host_z.numel() * 4 + host_view.numel() * 4, d2h=host_out.numel() * 4,
-                dtype="f32",
+                dtype="f32", outputs=lambda r: {"refmaps": r},
                 config={"workload": "config[1]: batched parametric refmap render, 64 synthetic 2000x1000 envmaps x random "
                                     "BRDF params -> 128x128 refmaps per GPU (each rank: its own envmaps, the same BRDF / view draws)",
                         "batch_per_gpu": batch,
@@ -193,7 +200,7 @@ def wl_img2refmap(args, rank, dev):
     h_mask = torch.empty((batch, res, res), dtype=torch.bool).pin_memory()
 
     def step():
-        return img2refmap_batch(colors, normals, offsets, res, thr)[0]
+        return img2refmap_batch(colors, normals, offsets, res, thr)
 
     def e2e_step():
         o = img2refmap_batch(h_col.to(dev, non_blocking=True), h_nrm.to(dev, non_blocking=True), offsets, res, thr)
@@ -213,6 +220,7 @@ def wl_img2refmap(args, rank, dev):
     return dict(step=step, e2e_step=e2e_step, units=batch, alg_bytes=24 * total_n + batch * res * res * (13 + 8),
                 gather=False, h2d=(h_col.numel() + h_nrm.numel()) * 4, d2h=h_map.numel() * 4 + h_mask.numel(),
                 dtype="f32 compare / u32 keys",
+                outputs=lambda r: {"refmap": r[0], "refmask": r[1], "counts": r[2], "sel_index": r[3]},
                 config={"workload": "img2refmap: 64 sphere images of 512x512 (SURVEY 8d inputs (b),(c)) -> 64 refmaps, "
                                     "res 128, thr pi/256", "batch_per_gpu": batch, "pixels_per_image": total_n // batch,
                         "l2": "inputs larger than L2 (317 MB of pixels per GPU)"},
@@ -236,7 +244,8 @@ def wl_synth(args, rank, dev):
     h_out = torch.empty((3, B, 3, RES, RES), dtype=torch.float32).pin_memory()
 
     def step():
-        return torch.stack(synthesize_refmaps(r, stacked_z, envs, views)[0])
+        post, scale, raw = synthesize_refmaps(r, stacked_z, envs, views)
+        return torch.stack(post), scale, raw
 
     def e2e_step():
         o = synthesize_refmaps(r, stacked_z, h_env.to(dev, non_blocking=True), views)[0]
@@ -245,6 +254,7 @@ def wl_synth(args, rank, dev):
 
     return dict(step=step, e2e_step=e2e_step, units=3 * B, alg_bytes=B * HE * WE * 12 + 3 * B * (RES * RES * 12 + 40),
                 gather=False, h2d=h_env.numel() * 4, d2h=h_out.numel() * 4, dtype="f32",
+                outputs=lambda o: {"refmaps": o[0], "normalizing_scale": o[1], "raw": o[2]},
                 config={"workload": "config[2]: training-data synthesis, batch 20 x {LrK, Lrk, Lrkm1} sharing envmap and "
                                     "view, render + luminance normalisation + log transform", "batch_per_gpu": B,
                         "renders_per_step_per_gpu": 3 * B, "l2": "inputs larger than L2 (480 MB of envmaps per GPU)"},
@@ -279,7 +289,7 @@ def wl_sampling(args, rank, dev):
         torch.cuda.synchronize()
 
     return dict(step=step, e2e_step=e2e_step, units=B, alg_bytes=B * (RES * RES * 12 * 2 + 128 * 256 * 12 * 2), gather=True,
-                h2d=h_r0.numel() * 4, d2h=h_out.numel() * 4, dtype="f32",
+                h2d=h_r0.numel() * 4, d2h=h_out.numel() * 4, dtype="f32", outputs=lambda r: {"refmaps": r},
                 config={"workload": "config[3]: per-step re-render of a sampling batch of 32 (r0toenvmap -> 128x256 envmap -> "
                                     "render at the current z); the U-Nets are stock PyTorch and not part of the step",
                         "batch_per_gpu": B, "l2": "flushed between steps (a 256 MB buffer is written)"},
@@ -355,6 +365,33 @@ def run_reference(args):
     }), file=JSON_OUT, flush=True)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(arrays, out_dir):
+    """Write {name: tensor} as out_dir/<name>.npy in float32 (float64 kept).  When the arrays exceed DUMP_LIMIT_BYTES
+    together, each keeps the same fraction of its flattened elements, drawn with a fixed seed, and
+    out_dir/<name>.sample_index.npy (float64) lists which."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    frac = 1.0
+    if sum(a.nbytes for a in host.values()) > DUMP_LIMIT_BYTES:
+        # a sampled element costs its value plus a float64 index; 4 KB per file covers the .npy headers
+        budget = DUMP_LIMIT_BYTES - 4096 * 2 * len(host)
+        frac = budget / sum(a.size * (a.itemsize + 8) for a in host.values())
+    for name, a in host.items():
+        if frac < 1.0:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, max(1, int(a.size * frac)), replace=False))
+            np.save(out_dir / f"{name}.sample_index.npy", idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -366,7 +403,10 @@ def main():
     ap.add_argument("--footprint", default="auto", help="'auto' (per render, from its roughness) or 1, 2, 4, 8, 16")
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries the JSON line and nothing else: whatever libraries print there (NCCL's version banner at init)
     # goes to stderr
     global JSON_OUT
@@ -411,7 +451,7 @@ def main():
         torch.cuda.synchronize()
 
     for _ in range(max(args.warmup, 3)):
-        step()
+        last = step()  # held like the timed loop holds it, so the allocator is warmed for the same footprint
     if gather is not None:
         gather.result()
     barrier()
@@ -421,16 +461,19 @@ def main():
         barrier()
         ev[0].record()
         for i in range(args.steps):
-            step()
+            last = step()
             ev[i + 1].record()
         if gather is not None:
-            gather.result()
+            last = gather.result()
             end = torch.cuda.Event(enable_timing=True)
             end.record()
         else:
             end = ev[-1]
         barrier()
     launches = L.drm_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        # before anything else runs: the render writes every step into the same buffer
+        dump_outputs(W["outputs"](last), args.dump_outputs)
     clock_info = clocks.summary()
     if clock_info["samples"] < 2:
         # the timed region was shorter than nvidia-smi's sampling period: keep the same load running until it has sampled
