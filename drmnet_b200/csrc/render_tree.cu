@@ -82,7 +82,7 @@ struct TreeArgs {
     int* item_ctr;         // work counter of this pass's persistent CTAs
     int pool_cap;          // chunks in pool_out
     PyrGeom gs, gd;
-    int B, He, We, N, res, pk, p, channel_first, pixcov;
+    int B, He, We, N, res, pk, channel_first, pixcov;
     float cell, domega_k, kappa, rcap, rcap_simple, hz, hz_in, hz_nv, hz_fin, kappa_d, hz_d, hand, limb_nv, limb_boost, limb_x, limb_hand, limb_ramp, limb_sub, limb_cells;
     float glx[TREE_MAX_P + 1][16], glw[TREE_MAX_P + 1][16];  // Gauss-Legendre lattices 1, 2, 4, 8, 16
     int stats;                   // debug: count visits / accepted records per pass into status[16..]
@@ -504,7 +504,10 @@ __device__ __forceinline__ bool warp_cone(const TreeArgs& g, int p, const NodeT&
     const float inv = rsqrtf(fmaxf(ax * ax + ay * ay + az * az, 1e-30f));
     ax *= inv; ay *= inv; az *= inv;
     const float dx = nd.nx - ax, dy = nd.ny - ay, dz = nd.nz - az;
-    beta = warp_max(nd.active ? chord_angle(dx * dx + dy * dy + dz * dz) : 0.f) + 0.75f * g.cell / (float)(1 << p);
+    // rounded term by term: with p known at compile time (p = 0) the compiler would otherwise fuse 0.75 cell + max into
+    // one FMA and move cone decisions by an ulp against the same cone at a run-time p
+    beta = __fadd_rn(warp_max(nd.active ? chord_angle(dx * dx + dy * dy + dz * dz) : 0.f),
+                     __fmul_rn(0.75f, g.cell) / (float)(1 << p));
     return true;
 }
 
@@ -548,8 +551,33 @@ __device__ __forceinline__ void tile_writeback(const TreeArgs& g, int p, float* 
     }
 }
 
-// ---- specular lobe, pass p ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(TREE_THREADS, 2) tree_spec_pass_kernel(const TreeArgs g) {
+// t-th tile of a tiles_x x tiles_x tile grid in the order the passes hand them out: the perimeter first (top row, bottom
+// row, left column, right column), then the interior row by row.  The perimeter tiles hold the rim of the refmap (n.v -> 0
+// on all four edges), whose blocks run several times longer than the others: started first, they no longer form the
+// tail of the pass.
+__device__ __forceinline__ void tile_of(int t, int tiles_x, int& ti, int& tj) {
+    const int m = tiles_x - 1;
+    if (tiles_x <= 2) { ti = t / tiles_x; tj = t - ti * tiles_x; }
+    else if (t < tiles_x) { ti = 0; tj = t; }
+    else if (t < 2 * tiles_x) { ti = m; tj = t - tiles_x; }
+    else if (t < 2 * tiles_x + (m - 1)) { ti = 1 + t - 2 * tiles_x; tj = 0; }
+    else if (t < 4 * m) { ti = 1 + t - 2 * tiles_x - (m - 1); tj = m; }
+    else { const int q = t - 4 * m; ti = 1 + q / (m - 1); tj = 1 + q - (ti - 1) * (m - 1); }
+}
+
+// Resident CTAs per SM (`__launch_bounds__` minimum), measured on a B200 with the bench batch: the specular passes keep
+// 2 (at 3 the compiler has 80 registers a thread, spills 128-200 bytes and every pass runs 4-10 % slower); the diffuse
+// pass takes 3 (80 registers, 12 bytes of spill: 16.2 -> 13.8 ms a step).
+static constexpr int SPEC_MINB = 2, DIFF_MINB = 3;
+
+// collect_stats: per pass p, status[50 + p] += cycles (in units of 1024) the warps spent in the barriers of the item loop,
+// waiting for the slowest warp of their tile, and status[56 + p] += their cycles in the kernel.  Outside the 40 words
+// drm_render_status copies: scripts/tree_stats.py reads them from the workspace.
+static constexpr int STAT_TILE_WAIT = 50, STAT_WARP_CYCLES = 56;
+
+// ---- specular lobe, pass P (one instance per lattice 2^P) -------------------------------------------------------------
+template <int P>
+__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel(const TreeArgs g) {
     extern __shared__ __align__(16) unsigned char tree_smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int* stack = reinterpret_cast<int*>(tree_smem) + warp * STACK_CAP;
@@ -557,23 +585,32 @@ __global__ void __launch_bounds__(TREE_THREADS, 2) tree_spec_pass_kernel(const T
     float4* buf0 = reinterpret_cast<float4*>(tree_smem + TREE_WARPS * STACK_CAP * 4 + TREE_WARPS * (BUF1 / 2) * PAIR4 * 16) + warp * (BUF0 * 2);
     float* red = reinterpret_cast<float*>(tree_smem);  // reused after the traversal: [256][3]
 
-    const int p = g.p;
+    constexpr int p = P;
     const int NG = g.res << p;
     const int tiles_x = (NG + 15) / 16;
     const int n_items = g.nact[p] * tiles_x * tiles_x;
+    // barriers of the item loop; under collect_stats they also count the cycles the warp waits in them
+    const bool stats = g.stats;
+    long long t_warp = stats ? clock64() : 0, t_wait = 0;
+    auto tile_sync = [&]() {
+        const long long t = stats ? clock64() : 0;
+        __syncthreads();
+        if (stats) t_wait += clock64() - t;
+    };
     // persistent CTAs: items = (active render, tile of 16 x 16 lattice nodes), tile-major so that the renders interleave,
-    // handed out by a counter (the rim tiles take several times longer than the others)
+    // handed out by a counter in the order of tile_of (the rim tiles take several times longer than the others)
     __shared__ int next_item;
     while (true) {
     if (tid == 0) next_item = atomicAdd(g.item_ctr, 1);
-    __syncthreads();
+    tile_sync();
     const int item = next_item;
     if (item >= n_items) break;
     const int k = g.act[p * TREE_CHUNK + item % g.nact[p]];
     const int tile = item / g.nact[p];
     const TreeConst rc = g.rc[k];
     const int pk = rc.pk;
-    const int ti = tile / tiles_x, tj = tile - ti * tiles_x;
+    int ti, tj;
+    tile_of(tile, tiles_x, ti, tj);
     const int I0 = ti * 16 + (warp >> 1) * 4, J0 = tj * 16 + (warp & 1) * 8;
     float a0 = 0.f, a1 = 0.f, a2 = 0.f;
     const bool pixcov = g.pixcov && p == 0 && pk > 0;  // the 1x1 node of a finer footprint carries the cell's covariance
@@ -591,7 +628,7 @@ __global__ void __launch_bounds__(TREE_THREADS, 2) tree_spec_pass_kernel(const T
         const int bI = I0 >> 2, bJ = J0 >> 3;
         const int* in_list = nullptr;  // entries of the current chunk
         int in_n, in_pos = 0, in_next = -1;
-        if (p == 0) {
+        if constexpr (p == 0) {
             in_n = g.gs.H[g.gs.L] * g.gs.W[g.gs.L];
         } else {
             const int nbJp = ((g.res << (p - 1)) + 7) / 8;
@@ -976,15 +1013,19 @@ __global__ void __launch_bounds__(TREE_THREADS, 2) tree_spec_pass_kernel(const T
         const int bI = I0 >> 2, bJ = J0 >> 3;
         if (bI < nbI && bJ < nbJ) g.heads_out[(size_t)k * nbI * nbJ + (size_t)bI * nbJ + bJ] = -1;
     }
-    __syncthreads();  // stacks and buffers are dead: the reduction reuses the memory
+    tile_sync();  // stacks and buffers are dead: the reduction reuses the memory
     tile_writeback(g, p, red, k, ti, tj, a0, a1, a2, false);
-    __syncthreads();  // ... and the next item's traversal reuses it again
+    tile_sync();  // ... and the next item's traversal reuses it again
+    }
+    if (stats && lane == 0) {
+        atomicAdd(g.status + STAT_TILE_WAIT + p, (int)(t_wait >> 10));
+        atomicAdd(g.status + STAT_WARP_CYCLES + p, (int)((clock64() - t_warp) >> 10));
     }
 }
 
 // ---- diffuse lobe: one pass, writes `out`.  1x1 lattice whose node carries the covariance of the refmap cell (fourth
 // order in the cell size: cells up to 0.03 rad), or the render's own lattice for coarser refmaps ------------------------
-__global__ void __launch_bounds__(TREE_THREADS, 2) tree_diff_kernel(const TreeArgs g) {
+__global__ void __launch_bounds__(TREE_THREADS, DIFF_MINB) tree_diff_kernel(const TreeArgs g) {
     extern __shared__ __align__(16) unsigned char tree_smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int* stack = reinterpret_cast<int*>(tree_smem) + warp * STACK_CAP;
@@ -1266,6 +1307,32 @@ static constexpr size_t TREE_SMEM = (size_t)TREE_WARPS * STACK_CAP * 4 + (size_t
                                     (size_t)TREE_WARPS * BUF0 * 2 * 16;
 static_assert(BUF1 * SREC4 <= (BUF1 / 2) * PAIR4 + 8 * BUF0, "the diffuse pass stages its records in the same region");
 
+static constexpr int MAX_DEVICES = 64;
+
+// Pass P on a persistent grid of (SMs x resident CTAs of this instance), at most one CTA per item.  The grid size is
+// queried once per device and instance.
+template <int P>
+static cudaError_t launch_spec_pass(const TreeArgs& a, long items, cudaStream_t st) {
+    static int resident[MAX_DEVICES];
+    cudaError_t e = cudaFuncSetAttribute(tree_spec_pass_kernel<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM);
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(tree_spec_pass_kernel<P>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    int dev = 0;
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    int per_sm = 0, sms = 0;
+    int* slot = dev < MAX_DEVICES ? &resident[dev] : &per_sm;
+    if (*slot == 0) {
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tree_spec_pass_kernel<P>, TREE_THREADS, TREE_SMEM);
+        if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        if (e != cudaSuccess) return e;
+        *slot = max(per_sm, 1) * sms;
+    }
+    const int grid = (int)(items < *slot ? items : *slot);
+    tree_spec_pass_kernel<P><<<grid, TREE_THREADS, TREE_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
 }  // namespace drm
 
 using namespace drm;
@@ -1349,7 +1416,7 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
         }
     }
     DRM_CHECK_CUDA(cudaFuncSetAttribute(tree_diff_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM));
-    DRM_CHECK_CUDA(cudaFuncSetAttribute(tree_spec_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM));
+    DRM_CHECK_CUDA(cudaFuncSetAttribute(tree_diff_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     // ---- renders, TREE_CHUNK at a time: specular pyramids, diffuse lobe (writes out), specular passes (add) ------------
     const size_t per_render_out = (size_t)res * res * 3;
     for (int k0 = 0; k0 < N; k0 += TREE_CHUNK) {
@@ -1378,7 +1445,6 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
             count_launches(1);
         }
         for (int p = 0; p <= L.pk; ++p) {
-            a.p = p;
             a.pixcov = (o.pixel_covariance && p == 0) ? 1 : 0;
             a.pool_in = nullptr; a.heads_in = nullptr; a.pool_out = nullptr; a.heads_out = nullptr; a.pool_ctr = nullptr;
             if (p > 0) { a.pool_in = L.pool[(p - 1) & 1]; a.heads_in = L.heads[(p - 1) & 1]; }
@@ -1389,10 +1455,15 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
             }
             const int NG = res << p;
             const long items = (long)((NG + 15) / 16) * ((NG + 15) / 16) * n;  // upper bound: the active renders are fewer
-            const int grid = (int)(items < 148L * 2 ? items : 148L * 2);  // persistent CTAs: two resident per SM
             a.item_ctr = L.status + 44 + p;
             DRM_CHECK_CUDA(cudaMemsetAsync(a.item_ctr, 0, sizeof(int), st));
-            tree_spec_pass_kernel<<<grid, TREE_THREADS, TREE_SMEM, st>>>(a);
+            switch (p) {
+                case 0: DRM_CHECK_CUDA(launch_spec_pass<0>(a, items, st)); break;
+                case 1: DRM_CHECK_CUDA(launch_spec_pass<1>(a, items, st)); break;
+                case 2: DRM_CHECK_CUDA(launch_spec_pass<2>(a, items, st)); break;
+                case 3: DRM_CHECK_CUDA(launch_spec_pass<3>(a, items, st)); break;
+                default: DRM_CHECK_CUDA(launch_spec_pass<4>(a, items, st)); break;
+            }
             count_launches(1);
         }
     }
