@@ -565,19 +565,31 @@ __device__ __forceinline__ void tile_of(int t, int tiles_x, int& ti, int& tj) {
     else { const int q = t - 4 * m; ti = 1 + q / (m - 1); tj = 1 + q - (ti - 1) * (m - 1); }
 }
 
-// Resident CTAs per SM (`__launch_bounds__` minimum), measured on a B200 with the bench batch: the specular passes keep
-// 2 (at 3 the compiler has 80 registers a thread, spills 128-200 bytes and every pass runs 4-10 % slower); the diffuse
-// pass takes 3 (80 registers, 12 bytes of spill: 16.2 -> 13.8 ms a step).
-static constexpr int SPEC_MINB = 2, DIFF_MINB = 3;
+// Resident CTAs per SM (`__launch_bounds__` minimum) of each specular instance and of the diffuse pass, measured on a
+// B200 with the bench batch.  At 3 a thread has 80 registers.  The specular instances fit them without spilling because
+// the item's render record and the warp's cone and thresholds live in shared memory (rc, WarpUni) and the evaluation
+// loops load each staged float4 where they use it; 3 x (67 584 dynamic + 1 520 static) bytes of shared memory fit an
+// SM.  Every pass is faster at 3 than at 2 (render step 178 -> 168 ms).  The diffuse pass: 80 registers, 12 bytes of
+// spill, 16.2 -> 13.8 ms a step.  tests/test_kernel_resources.py holds the specular instances to these budgets.
+static constexpr int SPEC_MINB[TREE_MAX_P + 1] = {3, 3, 3, 3, 3}, DIFF_MINB = 3;
 
 // collect_stats: per pass p, status[50 + p] += cycles (in units of 1024) the warps spent in the barriers of the item loop,
 // waiting for the slowest warp of their tile, and status[56 + p] += their cycles in the kernel.  Outside the 40 words
 // drm_render_status copies: scripts/tree_stats.py reads them from the workspace.
 static constexpr int STAT_TILE_WAIT = 50, STAT_WARP_CYCLES = 56;
 
+// What a block's traversal decides with that is the same in every lane of its warp: its cone and the thresholds of this
+// pass.  It lives in a per-warp shared slot and is read where it is used, so that it does not hold registers through
+// the evaluation loops.
+struct WarpUni {
+    float ax, ay, az, beta;
+    float thr_p, hand_p, hz_p, xthr, rcap, kappa2;
+    int limb;
+};
+
 // ---- specular lobe, pass P (one instance per lattice 2^P) -------------------------------------------------------------
 template <int P>
-__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel(const TreeArgs g) {
+__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_kernel(const TreeArgs g) {
     extern __shared__ __align__(16) unsigned char tree_smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int* stack = reinterpret_cast<int*>(tree_smem) + warp * STACK_CAP;
@@ -599,15 +611,30 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
     };
     // persistent CTAs: items = (active render, tile of 16 x 16 lattice nodes), tile-major so that the renders interleave,
     // handed out by a counter in the order of tile_of (the rim tiles take several times longer than the others)
-    __shared__ int next_item;
+    // the item's render record is read from shared memory where it is used: one copy per CTA instead of 34 registers
+    __shared__ int next_item, next_k;
+    __shared__ TreeConst rc;
+    __shared__ WarpUni wu_s[TREE_WARPS];
+    WarpUni& wu = wu_s[warp];
     while (true) {
-    if (tid == 0) next_item = atomicAdd(g.item_ctr, 1);
+    if (warp == 0) {
+        int it = 0;
+        if (lane == 0) it = atomicAdd(g.item_ctr, 1);
+        it = __shfl_sync(0xffffffffu, it, 0);
+        if (it < n_items) {
+            const int kk = g.act[p * TREE_CHUNK + it % g.nact[p]];
+            const int* src = reinterpret_cast<const int*>(g.rc + kk);
+            int* dst = reinterpret_cast<int*>(&rc);
+            for (int i = lane; i < (int)(sizeof(TreeConst) / 4); i += 32) dst[i] = src[i];
+            if (lane == 0) next_k = kk;
+        }
+        if (lane == 0) next_item = it;
+    }
     tile_sync();
     const int item = next_item;
     if (item >= n_items) break;
-    const int k = g.act[p * TREE_CHUNK + item % g.nact[p]];
+    const int k = next_k;
     const int tile = item / g.nact[p];
-    const TreeConst rc = g.rc[k];
     const int pk = rc.pk;
     int ti, tj;
     tile_of(tile, tiles_x, ti, tj);
@@ -655,18 +682,20 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
         // the horizon ramp matters most where the lobe itself sits on it: n.v within a few lobe widths of zero
         const float hz_p = (limb || nv_min < g.hz_nv * sqrtf(rc.alpha2)) ? (p == pk && rc.full2 ? g.hz_fin : g.hz) : g.hz_in;
         const float xthr = g.limb_ramp * sqrtf(rc.alpha2);
-        const float alpha2 = rc.alpha2, kappa2 = g.kappa * g.kappa;
+        const float kappa2 = g.kappa * g.kappa;
         // wide cells need the second-order terms of G1(n.d) whatever the lobe: without them the cap is half as large
         const float rcap = rc.full2 ? g.rcap : g.rcap_simple;
+        if (lane == 0) wu = WarpUni{ax, ay, az, beta, thr_p, hand_p, hz_p, xthr, rcap, kappa2, limb};
+        __syncwarp();
 
         // Staged pairs: field f of records 2j, 2j+1 sits at buf1[(j * 26 + f) * 2 + {0,1}].  Fields: 0-2 mu, 3 tr Sigma,
         // 4-6 Sigma_xx,yy,zz, 7-9 2 Sigma_xy,xz,yz, 10 2 v.mu / |mu|^2, 11-13 w RGB, 14-16 m_R, 17-19 m_B,
         // 20 v.mu, 21 v Sigma v, 22-24 Sigma v (rough lobes only).
         const f2 NX = F2(nd.nx), NY = F2(nd.ny), NZ = F2(nd.nz), NV = F2(-nd.nv);
         const f2 Q0 = F2(nd.q0), Q1 = F2(nd.q1), Q2 = F2(nd.q2), Q3 = F2(0.5f * nd.q3), Q4 = F2(0.5f * nd.q4), Q5 = F2(0.5f * nd.q5);
-        const f2 CI = F2(rc.inv_a2m1), OMA = F2(rc.one_m_a2), A2 = F2(alpha2);
         const f2 TRP = F2(nd.P0 + nd.P1 + nd.P2);
         auto eval1 = [&]() {
+            const f2 CI = F2(rc.inv_a2m1), OMA = F2(rc.one_m_a2), A2 = F2(rc.alpha2);
             if (n1 & 1) {  // pad the last pair with a record of zero weight
                 float* s = buf1 + ((n1 >> 1) * 26) * 2 + 1;
                 if (lane < 26) s[lane * 2] = lane == 3 ? 1.f : 0.f;
@@ -678,7 +707,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
             if (!rc.full2) {
                 for (int j = 0; j < np; ++j) {
                     const float4* s = b4 + j * PAIR4;
-                    const float4 v0 = s[0], v1 = s[1], v2 = s[2], v3 = s[3], v4 = s[4], v5 = s[5], v6 = s[6], v7 = s[7], v8 = s[8], v9 = s[9];
+                    const float4 v0 = s[0], v1 = s[1];
                     const f2 ex = sub2(NX, lo(v0)), ey = sub2(NY, hi(v0)), ez = sub2(NZ, lo(v1));
                     f2 u = fma2(ez, ez, fma2(ey, ey, fma2(ex, ex, hi(v1))));
                     f2 nmu = fma2(u, F2(-0.5f), F2(1.f));
@@ -686,6 +715,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                         u = fma2(TRP, nmu, u);
                         nmu = fma2(u, F2(-0.5f), F2(1.f));
                     }
+                    const float4 v2 = s[2], v3 = s[3], v4 = s[4];
                     f2 nSn = mul2(Q0, lo(v2));
                     nSn = fma2(Q1, hi(v2), nSn); nSn = fma2(Q2, lo(v3), nSn);
                     nSn = fma2(Q3, hi(v3), nSn); nSn = fma2(Q4, lo(v4), nSn); nSn = fma2(Q5, hi(v4), nSn);
@@ -697,6 +727,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                         pp = fma2(mul2(my, mz), F2(nd.P5), pp);
                         nSn = add2(nSn, pp);
                     }
+                    const float4 v5 = s[5];
                     const f2 xm = max2(fma2(lo(v5), nmu, NV), 0.f);
                     const f2 sin2 = mul2(u, fma2(u, F2(-0.25f), F2(1.f)));
                     const f2 rq = rcp2(fma2(sin2, CI, F2(1.f)));
@@ -708,9 +739,11 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                     const f2 t = fma2(mul2(a, F2(6.f)), a, mul2(rq, CI));
                     const f2 K = mul2(Dg, fma2(mul2(nSn, t), F2(2.f), F2(1.f)));
                     const f2 cn = mul2(mul2(Dg, a), F2(4.f));
+                    const float4 v7 = s[7], v8 = s[8], v9 = s[9];
                     const f2 nmR = fma2(NZ, lo(v8), fma2(NY, hi(v7), mul2(NX, lo(v7))));
                     const f2 nmB = fma2(NZ, hi(v9), fma2(NY, lo(v9), mul2(NX, hi(v8))));
                     cR = fma2(cn, nmR, fma2(K, hi(v5), cR));
+                    const float4 v6 = s[6];
                     cG = fma2(K, lo(v6), cG);
                     cG = fma2(cn, make_float2(-nmR.x - nmB.x, -nmR.y - nmB.y), cG);
                     cB = fma2(cn, nmB, fma2(K, hi(v6), cB));
@@ -718,8 +751,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
             } else {
                 for (int j = 0; j < np; ++j) {
                     const float4* s = b4 + j * PAIR4;
-                    const float4 v0 = s[0], v1 = s[1], v2 = s[2], v3 = s[3], v4 = s[4], v5 = s[5], v6 = s[6], v7 = s[7], v8 = s[8], v9 = s[9],
-                                 v10 = s[10], v11 = s[11], v12 = s[12];
+                    const float4 v0 = s[0], v1 = s[1];
                     const f2 ex = sub2(NX, lo(v0)), ey = sub2(NY, hi(v0)), ez = sub2(NZ, lo(v1));
                     f2 u = fma2(ez, ez, fma2(ey, ey, fma2(ex, ex, hi(v1))));
                     f2 nmu = fma2(u, F2(-0.5f), F2(1.f));
@@ -727,6 +759,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                         u = fma2(TRP, nmu, u);
                         nmu = fma2(u, F2(-0.5f), F2(1.f));
                     }
+                    const float4 v2 = s[2], v3 = s[3], v4 = s[4];
                     f2 nSn = mul2(Q0, lo(v2));
                     nSn = fma2(Q1, hi(v2), nSn); nSn = fma2(Q2, lo(v3), nSn);
                     nSn = fma2(Q3, hi(v3), nSn); nSn = fma2(Q4, lo(v4), nSn); nSn = fma2(Q5, hi(v4), nSn);
@@ -739,6 +772,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                         pp = fma2(mul2(my, mz), F2(nd.P5), pp);
                         pS = add2(nSn, pp);
                     }
+                    const float4 v10 = s[10], v11 = s[11], v12 = s[12];
                     const f2 vmu = lo(v10), vSv = hi(v10);
                     const f2 nSv = fma2(NZ, lo(v12), fma2(NY, hi(v11), mul2(NX, lo(v11))));
                     // mean and variance of n.d over the cell; the clamp at the horizon acts on that distribution
@@ -776,9 +810,11 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                     T3.y = st1 ? 0.f : T3.y;
                     K = add2(K, add2(T2, T3));
                     const f2 cn = mul2(mul2(Dg, a), F2(4.f));
+                    const float4 v5 = s[5], v7 = s[7], v8 = s[8], v9 = s[9];
                     const f2 nmR = fma2(NZ, lo(v8), fma2(NY, hi(v7), mul2(NX, lo(v7))));
                     const f2 nmB = fma2(NZ, hi(v9), fma2(NY, lo(v9), mul2(NX, hi(v8))));
                     cR = fma2(cn, nmR, fma2(K, hi(v5), cR));
+                    const float4 v6 = s[6];
                     cG = fma2(K, lo(v6), cG);
                     cG = fma2(cn, make_float2(-nmR.x - nmB.x, -nmR.y - nmB.y), cG);
                     cB = fma2(cn, nmB, fma2(K, hi(v6), cB));
@@ -793,6 +829,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
         // (hx0,hx1,hy0,hy1) (hz0,hz1,2vh0,2vh1) (wR0,wR1,wG0,wG1) (wB0,wB1,-,-).
         const f2 NVp = F2(nd.nv);
         auto eval0 = [&]() {
+            const f2 CI = F2(rc.inv_a2m1), OMA = F2(rc.one_m_a2), A2 = F2(rc.alpha2);
             if (n0 & 1) {  // pad the last pair with a texel of zero weight
                 float* s = reinterpret_cast<float*>(buf0 + (n0 >> 1) * 4) + 1;
                 if (lane < 7) s[lane * 2] = lane < 3 ? (lane == 0 ? nd.nx : lane == 1 ? nd.ny : nd.nz) : 0.f;
@@ -848,13 +885,13 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
             // ---- decide ----
             int act = ACT_DROP;
             const int lev = (int)(ent >> 28), id = (int)(ent & 0x0fffffffu);
-            float4 r0, r1, r2, r3, r4;
             float h[3], vh = 0.f, w3[3];
             if (has) {
                 float mx, my, mz, rha, wsum, vmu, im;
                 if (lev > 0) {
+                    // the verdict needs the mean, radius and energy; staging reads the rest of the record again
                     const float4* rp = pyr + (g.gs.off[lev] + id) * REC4;
-                    r0 = rp[0]; r1 = rp[1]; r2 = rp[2]; r3 = rp[3]; r4 = rp[4];
+                    const float4 r0 = rp[0], r2 = rp[2], r3 = rp[3];
                     mx = r0.x; my = r0.y; mz = r0.z;
                     wsum = r2.z + r2.w + r3.x;
                     const float m2 = fmaxf(mx * mx + my * my + mz * mz, 1e-30f);
@@ -869,6 +906,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                     im = 1.f; rha = 0.f; vmu = vh;
                 }
                 if (wsum > 0.f) {
+                    const float ax = wu.ax, ay = wu.ay, az = wu.az, beta = wu.beta;
                     const float hx = mx * im - ax, hy = my * im - ay, hz = mz * im - az;
                     const float ang = fast_chord_angle(hx * hx + hy * hy + hz * hz);
                     const float dmin = fmaxf(ang - beta - rha, 0.f);
@@ -880,14 +918,14 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                     if (spread < 1.5607f && adc <= -ss) act = ACT_DROP;
                     // near for this lattice: small cells go to the child blocks, large ones are refined here so that
                     // their far parts stay on this lattice
-                    else if (p < pk && dmin < thr_p) act = (lev == 0 || rha <= hand_p * thr_p) ? ACT_HAND : ACT_REFINE;
+                    else if (p < pk && dmin < wu.thr_p) act = (lev == 0 || rha <= wu.hand_p * wu.thr_p) ? ACT_HAND : ACT_REFINE;
                     // rim blocks: what lies within the shadowing ramp of their horizon goes down as well, in pieces of
                     // at most 0.05 rad
-                    else if (p < pk && limb && spread < 1.5607f &&
-                             adc * __cosf(spread) - sqrtf(fmaxf(1.f - adc * adc, 0.f)) * ss < xthr)
+                    else if (p < pk && wu.limb && spread < 1.5607f &&
+                             adc * __cosf(spread) - sqrtf(fmaxf(1.f - adc * adc, 0.f)) * ss < wu.xthr)
                         act = (lev == 0 || rha <= 0.05f) ? ACT_HAND : ACT_REFINE;
-                    else if (lev > 0 && (rha > rcap || rha * rha > kappa2 * (alpha2 + dmin * dmin) ||
-                                         (2.f * rha > hz_p && fabsf(adc) < ss))) act = ACT_REFINE;
+                    else if (lev > 0 && (rha > wu.rcap || rha * rha > wu.kappa2 * (rc.alpha2 + dmin * dmin) ||
+                                         (2.f * rha > wu.hz_p && fabsf(adc) < ss))) act = ACT_REFINE;
                     else act = ACT_ACCEPT;
                 }
             }
@@ -965,6 +1003,8 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB) tree_spec_pass_kernel
                     if (lev > 0) {
                         const int slot = n1 + __popc(m1 & ((1u << lane) - 1u));
                         float* s = buf1 + ((slot >> 1) * 26) * 2 + (slot & 1);
+                        const float4* rp = pyr + (g.gs.off[lev] + id) * REC4;
+                        const float4 r0 = rp[0], r1 = rp[1], r2 = rp[2], r3 = rp[3], r4 = rp[4];
                         const float Sxx = r1.x, Syy = r1.y, Szz = r1.z, Sxy = r1.w, Sxz = r2.x, Syz = r2.y;
                         const float vx = rc.vhat[0], vy = rc.vhat[1], vz = rc.vhat[2];
                         const float vmu = vx * r0.x + vy * r0.y + vz * r0.z;
