@@ -14,7 +14,7 @@ from typing import List, Optional, Sequence, Tuple
 import torch
 
 from . import _lib
-from .renderer import B200RefMapRenderer, _slots, render_batch
+from .renderer import B200RefMapRenderer, _env_dtype, _slots, render_batch
 
 
 def _stream(device) -> int:
@@ -26,7 +26,8 @@ def rendering_refmaps(renderer: B200RefMapRenderer, envmaps, z: torch.Tensor,
                       new_scene: bool = False) -> torch.Tensor:
     """envmaps [B,He,We,3] (a tensor, or a list of [He,We,3] tensors), z [L,B,P] -> [L,B,3,res,res]: the L BRDF vectors
     of sample b share envmap b and view b, exactly the grouping of the reference's double loop
-    (models/drmnet.py:680-705), in one batched launch.  ``view_from`` is [B,3] or a list of B views.
+    (models/drmnet.py:680-705), in one batched launch.  ``view_from`` is [B,3] or a list of B views.  fp16 envmaps are
+    rendered in place and the renderer keeps the last one in fp16 (see ``render_batch``: fp16 ends at 65504).
 
     Like the loop it replaces, the call leaves its mark on the stateful renderer when ``new_scene`` is false: parameters
     that are not named come from the renderer's persistent BSDF, and afterwards the renderer holds the last envmap, the
@@ -62,7 +63,7 @@ def rendering_refmaps(renderer: B200RefMapRenderer, envmaps, z: torch.Tensor,
                        flip=torch.full((B * L,), bool(flip), device=device), res=renderer.refmap_res,
                        footprint_S=renderer.footprint_S, alpha_min=renderer.alpha_min or 0.0, channel_first=True)
     if not new_scene:
-        renderer._envmap = envmaps[-1].to(renderer.device, torch.float32)
+        renderer._envmap = envmaps[-1].to(renderer.device, _env_dtype(envmaps))
         renderer._bsdf = zz[-1].detach().clone()
         if view_from is not None:
             renderer._view = view[-1].detach().float().cpu()

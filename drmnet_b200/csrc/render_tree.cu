@@ -25,6 +25,7 @@
 //
 // The inner loops are bound by the FP32 / MUFU pipes (DESIGN.md 5): the envmap is read once by the pyramid build and
 // stays in L2 for the traversal.
+#include <cuda_fp16.h>
 #include <math.h>
 #include <string.h>
 
@@ -253,13 +254,20 @@ struct Mom {
     }
 };
 
+// Envmap texels are fp32 or fp16 (T = float or __half), 3 scalars a texel, converted where they are loaded.  fp16 -> fp32
+// is exact, so an fp16 envmap renders bit for bit like its fp32 upcast.  TreeArgs::env points to either; the kernels
+// that read texels cast it to T.
+__device__ __forceinline__ float texel_f(float x) { return x; }
+__device__ __forceinline__ float texel_f(__half x) { return __half2float(x); }
+
 // texel (r, c) of render rc / envmap e: half vector, v.h, Fresnel-weighted energy
-__device__ __forceinline__ void texel_spec(const TreeArgs& g, const TreeConst& rc, const float* __restrict__ env_b, int r,
+template <typename T>
+__device__ __forceinline__ void texel_spec(const TreeArgs& g, const TreeConst& rc, const T* __restrict__ env_b, int r,
                                            int c, float* h, float& vh, float* w) {
     const float st = g.sin_t[r], ct = g.cos_t[r], sp = g.sin_p[c], cp = g.cos_p[c];
     const float dx = st * sp, dy = ct, dz = -st * cp;
     const float dom = g.domega_k * st;
-    const float* e = env_b + ((size_t)r * g.We + c) * 3;
+    const T* e = env_b + ((size_t)r * g.We + c) * 3;
     // |v + d|^2 from its components: 2 + 2 v.d cancels at grazing reflection (d ~ -v), which the limb cells see
     const float sx = rc.vhat[0] + dx, sy = rc.vhat[1] + dy, sz = rc.vhat[2] + dz;
     const float len2 = fmaxf(sx * sx + sy * sy + sz * sz, 1e-12f);
@@ -270,18 +278,19 @@ __device__ __forceinline__ void texel_spec(const TreeArgs& g, const TreeConst& r
     const float mm = fminf(fmaxf(1.f - vh, 0.f), 1.f);
     const float sw = (mm * mm) * (mm * mm) * mm;
     const float a = (1.f - rc.m) * Fd + rc.m * sw, b = rc.m * (1.f - sw);  // F_c = a + b base_c
-    w[0] = e[0] * dom * (a + b * rc.base[0]);
-    w[1] = e[1] * dom * (a + b * rc.base[1]);
-    w[2] = e[2] * dom * (a + b * rc.base[2]);
+    w[0] = texel_f(e[0]) * dom * (a + b * rc.base[0]);
+    w[1] = texel_f(e[1]) * dom * (a + b * rc.base[1]);
+    w[2] = texel_f(e[2]) * dom * (a + b * rc.base[2]);
 }
 
-__device__ __forceinline__ void texel_diff(const TreeArgs& g, const float* __restrict__ env_b, int r, int c, float* d,
+template <typename T>
+__device__ __forceinline__ void texel_diff(const TreeArgs& g, const T* __restrict__ env_b, int r, int c, float* d,
                                            float* w) {
     const float st = g.sin_t[r], ct = g.cos_t[r], sp = g.sin_p[c], cp = g.cos_p[c];
     d[0] = st * sp; d[1] = ct; d[2] = -st * cp;
     const float dom = g.domega_k * st;
-    const float* e = env_b + ((size_t)r * g.We + c) * 3;
-    w[0] = e[0] * dom; w[1] = e[1] * dom; w[2] = e[2] * dom;
+    const T* e = env_b + ((size_t)r * g.We + c) * 3;
+    w[0] = texel_f(e[0]) * dom; w[1] = texel_f(e[1]) * dom; w[2] = texel_f(e[2]) * dom;
 }
 
 // level `lev` of a pyramid straight from the texels (lev = 1 for the specular pyramid of render blockIdx.y, the base
@@ -302,8 +311,8 @@ __global__ void tree_active_kernel(const TreeConst* __restrict__ rc, int n, int*
     }
 }
 
-template <bool SPEC>
-__global__ void pyr_from_texels_kernel(const TreeArgs g, int lev, float4* __restrict__ pyr) {
+template <bool SPEC, typename T>
+__device__ __forceinline__ void pyr_from_texels(const TreeArgs& g, int lev, float4* __restrict__ pyr) {
     const PyrGeom& G = SPEC ? g.gs : g.gd;
     const int Hl = G.H[lev], Wl = G.W[lev];
     const int cell = blockIdx.x * blockDim.x + threadIdx.x;
@@ -313,7 +322,7 @@ __global__ void pyr_from_texels_kernel(const TreeArgs g, int lev, float4* __rest
     const int R = cell / Wl, C = cell - R * Wl;
     const int e = 1 << lev;
     const TreeConst* rcp = SPEC ? &g.rc[k] : nullptr;
-    const float* env_b = g.env + (size_t)(SPEC ? rcp->env : k) * g.He * g.We * 3;
+    const T* env_b = reinterpret_cast<const T*>(g.env) + (size_t)(SPEC ? rcp->env : k) * g.He * g.We * 3;
     float4* rec = pyr + ((size_t)k * G.cells + G.off[lev] + cell) * REC4;
     if (SPEC && !rcp->has_spec) {
         for (int i = 0; i < REC4; ++i) rec[i] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -347,6 +356,15 @@ __global__ void pyr_from_texels_kernel(const TreeArgs g, int lev, float4* __rest
         out[0].w = sqrtf(rh) * 1.0001f + 1e-7f;
     }
     for (int i = 0; i < REC4; ++i) rec[i] = out[i];
+}
+
+template <bool SPEC>
+__global__ void pyr_from_texels_kernel(const TreeArgs g, int lev, float4* __restrict__ pyr) {
+    pyr_from_texels<SPEC, float>(g, lev, pyr);
+}
+template <bool SPEC>
+__global__ void pyr_from_texels_kernel_h(const TreeArgs g, int lev, float4* __restrict__ pyr) {
+    pyr_from_texels<SPEC, __half>(g, lev, pyr);
 }
 
 // level lev from level lev - 1 of every pyramid (blockIdx.y = pyramid)
@@ -588,10 +606,13 @@ struct WarpUni {
 };
 
 // ---- specular lobe, pass P (one instance per lattice 2^P) -------------------------------------------------------------
-template <int P>
-__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_kernel(const TreeArgs g) {
+// The bodies of the texel-reading kernels are device templates on T under fp32 and fp16 __global__ wrappers.  They take
+// threadIdx.x from the wrapper, where its range is known from the launch bounds, and this one takes TreeArgs by value:
+// either way the fp32 kernels compile to other (equivalent) code than when they held the body themselves.
+template <int P, typename T>
+__device__ __forceinline__ void tree_spec_pass(const TreeArgs g, int tid) {
     extern __shared__ __align__(16) unsigned char tree_smem[];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     int* stack = reinterpret_cast<int*>(tree_smem) + warp * STACK_CAP;
     float* buf1 = reinterpret_cast<float*>(tree_smem + TREE_WARPS * STACK_CAP * 4) + warp * (BUF1 / 2 * PAIR4 * 4);
     float4* buf0 = reinterpret_cast<float4*>(tree_smem + TREE_WARPS * STACK_CAP * 4 + TREE_WARPS * (BUF1 / 2) * PAIR4 * 16) + warp * (BUF0 * 2);
@@ -649,7 +670,7 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_ker
 
     if (live) {
         const float4* pyr = g.pyr_s + (size_t)k * g.gs.cells * REC4;
-        const float* env_b = g.env + (size_t)rc.env * g.He * g.We * 3;
+        const T* env_b = reinterpret_cast<const T*>(g.env) + (size_t)rc.env * g.He * g.We * 3;
         // input: the top level of the pyramid (pass 0) or the parent block's hand-over list
         const int nbJ = (NG + 7) / 8;
         const int bI = I0 >> 2, bJ = J0 >> 3;
@@ -1063,11 +1084,21 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_ker
     }
 }
 
+template <int P>
+__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_kernel(const TreeArgs g) {
+    tree_spec_pass<P, float>(g, threadIdx.x);
+}
+template <int P>
+__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_kernel_h(const TreeArgs g) {
+    tree_spec_pass<P, __half>(g, threadIdx.x);
+}
+
 // ---- diffuse lobe: one pass, writes `out`.  1x1 lattice whose node carries the covariance of the refmap cell (fourth
 // order in the cell size: cells up to 0.03 rad), or the render's own lattice for coarser refmaps ------------------------
-__global__ void __launch_bounds__(TREE_THREADS, DIFF_MINB) tree_diff_kernel(const TreeArgs g) {
+template <typename T>
+__device__ __forceinline__ void tree_diff(const TreeArgs& g, int tid) {
     extern __shared__ __align__(16) unsigned char tree_smem[];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     int* stack = reinterpret_cast<int*>(tree_smem) + warp * STACK_CAP;
     float4* buf1 = reinterpret_cast<float4*>(tree_smem + TREE_WARPS * STACK_CAP * 4) + warp * (BUF1 * SREC4);
     float* red = reinterpret_cast<float*>(tree_smem);
@@ -1087,7 +1118,7 @@ __global__ void __launch_bounds__(TREE_THREADS, DIFF_MINB) tree_diff_kernel(cons
     const bool live = rc.has_diff && warp_cone(g, p, nd, ax, ay, az, beta);
     if (live) {
         const float4* pyr = g.pyr_d + (size_t)rc.env * g.gd.cells * REC4;
-        const float* env_b = g.env + (size_t)rc.env * g.He * g.We * 3;
+        const T* env_b = reinterpret_cast<const T*>(g.env) + (size_t)rc.env * g.He * g.We * 3;
         const int in_n = g.gd.H[g.gd.L] * g.gd.W[g.gd.L];
         int in_pos = 0, sp = 0, n1 = 0;
         const float vx = rc.vhat[0], vy = rc.vhat[1], vz = rc.vhat[2];
@@ -1235,6 +1266,13 @@ __global__ void __launch_bounds__(TREE_THREADS, DIFF_MINB) tree_diff_kernel(cons
     tile_writeback(g, p, red, k, ti, tj, a0, a1, a2, true);
 }
 
+__global__ void __launch_bounds__(TREE_THREADS, DIFF_MINB) tree_diff_kernel(const TreeArgs g) {
+    tree_diff<float>(g, threadIdx.x);
+}
+__global__ void __launch_bounds__(TREE_THREADS, DIFF_MINB) tree_diff_kernel_h(const TreeArgs g) {
+    tree_diff<__half>(g, threadIdx.x);
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1349,27 +1387,41 @@ static_assert(BUF1 * SREC4 <= (BUF1 / 2) * PAIR4 + 8 * BUF0, "the diffuse pass s
 
 static constexpr int MAX_DEVICES = 64;
 
+// The kernels that read envmap texels, per texel type: fp32 (the kernels above) or fp16 (their _h twins).
+template <typename T> struct TexelKernels;
+template <> struct TexelKernels<float> {
+    template <int P> static constexpr void (*spec)(TreeArgs) = tree_spec_pass_kernel<P>;
+    static constexpr void (*diff)(TreeArgs) = tree_diff_kernel;
+    template <bool SPEC> static constexpr void (*pyr)(TreeArgs, int, float4*) = pyr_from_texels_kernel<SPEC>;
+};
+template <> struct TexelKernels<__half> {
+    template <int P> static constexpr void (*spec)(TreeArgs) = tree_spec_pass_kernel_h<P>;
+    static constexpr void (*diff)(TreeArgs) = tree_diff_kernel_h;
+    template <bool SPEC> static constexpr void (*pyr)(TreeArgs, int, float4*) = pyr_from_texels_kernel_h<SPEC>;
+};
+
 // Pass P on a persistent grid of (SMs x resident CTAs of this instance), at most one CTA per item.  The grid size is
-// queried once per device and instance.
-template <int P>
+// queried once per device and instance (fp32 and fp16 instances have their own slots).
+template <int P, typename T>
 static cudaError_t launch_spec_pass(const TreeArgs& a, long items, cudaStream_t st) {
     static int resident[MAX_DEVICES];
-    cudaError_t e = cudaFuncSetAttribute(tree_spec_pass_kernel<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM);
+    void (*kernel)(TreeArgs) = TexelKernels<T>::template spec<P>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM);
     if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(tree_spec_pass_kernel<P>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     int dev = 0;
     if (e == cudaSuccess) e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
     int per_sm = 0, sms = 0;
     int* slot = dev < MAX_DEVICES ? &resident[dev] : &per_sm;
     if (*slot == 0) {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tree_spec_pass_kernel<P>, TREE_THREADS, TREE_SMEM);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, TREE_THREADS, TREE_SMEM);
         if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         if (e != cudaSuccess) return e;
         *slot = max(per_sm, 1) * sms;
     }
     const int grid = (int)(items < *slot ? items : *slot);
-    tree_spec_pass_kernel<P><<<grid, TREE_THREADS, TREE_SMEM, st>>>(a);
+    kernel<<<grid, TREE_THREADS, TREE_SMEM, st>>>(a);
     return cudaGetLastError();
 }
 
@@ -1391,10 +1443,12 @@ extern "C" int drm_render_status(const void* workspace, int* status_host, void* 
     return DRM_OK;
 }
 
-extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, const int32_t* env_index, const float* z6,
-                                       const float* view3, const uint8_t* flip, int N, int res, int S, float alpha_min,
-                                       int channel_first, float* out, void* workspace, size_t workspace_bytes,
-                                       void* cuda_stream, const DrmRenderOptions* opts) {
+// drm_render_refmaps_opts (T = float) and drm_render_refmaps_half (T = __half): only the kernels that read texels differ
+template <typename T>
+static int render_refmaps(const T* env, int B, int He, int We, const int32_t* env_index, const float* z6,
+                          const float* view3, const uint8_t* flip, int N, int res, int S, float alpha_min,
+                          int channel_first, float* out, void* workspace, size_t workspace_bytes, void* cuda_stream,
+                          const DrmRenderOptions* opts) {
     DRM_REQUIRE(env && z6 && view3 && out, "render: null pointer");
     DRM_REQUIRE(N > 0 && B > 0 && He > 0 && We > 0 && res > 0, "render: N=%d B=%d He=%d We=%d res=%d must be positive", N, B, He, We, res);
     DRM_REQUIRE(S == 0 || log2_exact(S) >= 0, "render: footprint_S=%d must be 0 (per render) or 1, 2, 4, 8, 16", S);
@@ -1417,7 +1471,7 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
 
     TreeArgs g;
     memset(&g, 0, sizeof(g));
-    g.env = env; g.sin_t = L.sin_t; g.cos_t = L.cos_t; g.sin_p = L.sin_p; g.cos_p = L.cos_p;
+    g.env = reinterpret_cast<const float*>(env); g.sin_t = L.sin_t; g.cos_t = L.cos_t; g.sin_p = L.sin_p; g.cos_p = L.cos_p;
     g.pyr_s = L.pyr_s; g.pyr_d = L.pyr_d; g.status = L.status; g.env_used = L.env_used; g.act = L.act; g.nact = L.nact;
     g.gs = L.gs; g.gd = L.gd;
     g.B = B; g.He = He; g.We = We; g.res = res; g.pk = L.pk; g.channel_first = channel_first;
@@ -1447,7 +1501,7 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
     if (L.gd.L >= 1) {
         const int first = L.gd.base > 0 ? L.gd.base : 1;  // base 0: texels are read directly, level 1 is the first stored
         const int nb = L.gd.H[first] * L.gd.W[first];
-        pyr_from_texels_kernel<false><<<dim3((nb + tb - 1) / tb, B), tb, 0, st>>>(g, first, L.pyr_d);
+        TexelKernels<T>::template pyr<false><<<dim3((nb + tb - 1) / tb, B), tb, 0, st>>>(g, first, L.pyr_d);
         count_launches(1);
         for (int l = first + 1; l <= L.gd.L; ++l) {
             const int nl = L.gd.H[l] * L.gd.W[l];
@@ -1455,8 +1509,8 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
             count_launches(1);
         }
     }
-    DRM_CHECK_CUDA(cudaFuncSetAttribute(tree_diff_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM));
-    DRM_CHECK_CUDA(cudaFuncSetAttribute(tree_diff_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    DRM_CHECK_CUDA(cudaFuncSetAttribute(TexelKernels<T>::diff, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM));
+    DRM_CHECK_CUDA(cudaFuncSetAttribute(TexelKernels<T>::diff, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     // ---- renders, TREE_CHUNK at a time: specular pyramids, diffuse lobe (writes out), specular passes (add) ------------
     const size_t per_render_out = (size_t)res * res * 3;
     for (int k0 = 0; k0 < N; k0 += TREE_CHUNK) {
@@ -1469,7 +1523,7 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
         count_launches(1);
         if (L.gs.L >= 1) {
             const int n1 = L.gs.H[1] * L.gs.W[1];
-            pyr_from_texels_kernel<true><<<dim3((n1 + tb - 1) / tb, n), tb, 0, st>>>(a, 1, L.pyr_s);
+            TexelKernels<T>::template pyr<true><<<dim3((n1 + tb - 1) / tb, n), tb, 0, st>>>(a, 1, L.pyr_s);
             count_launches(1);
             for (int l = 2; l <= L.gs.L; ++l) {
                 const int nl = L.gs.H[l] * L.gs.W[l];
@@ -1481,7 +1535,7 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
             const int pd = a.diff_cov ? 0 : L.pk;  // grid for the finest lattice a render of this call may have
             const int NGd = res << pd;
             const int tiles = ((NGd + 15) / 16) * ((NGd + 15) / 16);
-            tree_diff_kernel<<<dim3(tiles, n), TREE_THREADS, TREE_SMEM, st>>>(a);
+            TexelKernels<T>::diff<<<dim3(tiles, n), TREE_THREADS, TREE_SMEM, st>>>(a);
             count_launches(1);
         }
         for (int p = 0; p <= L.pk; ++p) {
@@ -1498,17 +1552,33 @@ extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, 
             a.item_ctr = L.status + 44 + p;
             DRM_CHECK_CUDA(cudaMemsetAsync(a.item_ctr, 0, sizeof(int), st));
             switch (p) {
-                case 0: DRM_CHECK_CUDA(launch_spec_pass<0>(a, items, st)); break;
-                case 1: DRM_CHECK_CUDA(launch_spec_pass<1>(a, items, st)); break;
-                case 2: DRM_CHECK_CUDA(launch_spec_pass<2>(a, items, st)); break;
-                case 3: DRM_CHECK_CUDA(launch_spec_pass<3>(a, items, st)); break;
-                default: DRM_CHECK_CUDA(launch_spec_pass<4>(a, items, st)); break;
+                case 0: DRM_CHECK_CUDA((launch_spec_pass<0, T>(a, items, st))); break;
+                case 1: DRM_CHECK_CUDA((launch_spec_pass<1, T>(a, items, st))); break;
+                case 2: DRM_CHECK_CUDA((launch_spec_pass<2, T>(a, items, st))); break;
+                case 3: DRM_CHECK_CUDA((launch_spec_pass<3, T>(a, items, st))); break;
+                default: DRM_CHECK_CUDA((launch_spec_pass<4, T>(a, items, st))); break;
             }
             count_launches(1);
         }
     }
     DRM_CHECK_CUDA(cudaGetLastError());
     return DRM_OK;
+}
+
+extern "C" int drm_render_refmaps_opts(const float* env, int B, int He, int We, const int32_t* env_index, const float* z6,
+                                       const float* view3, const uint8_t* flip, int N, int res, int S, float alpha_min,
+                                       int channel_first, float* out, void* workspace, size_t workspace_bytes,
+                                       void* cuda_stream, const DrmRenderOptions* opts) {
+    return render_refmaps(env, B, He, We, env_index, z6, view3, flip, N, res, S, alpha_min, channel_first, out, workspace,
+                          workspace_bytes, cuda_stream, opts);
+}
+
+extern "C" int drm_render_refmaps_half(const void* env, int B, int He, int We, const int32_t* env_index, const float* z6,
+                                       const float* view3, const uint8_t* flip, int N, int res, int S, float alpha_min,
+                                       int channel_first, float* out, void* workspace, size_t workspace_bytes,
+                                       void* cuda_stream, const DrmRenderOptions* opts) {
+    return render_refmaps(static_cast<const __half*>(env), B, He, We, env_index, z6, view3, flip, N, res, S, alpha_min,
+                          channel_first, out, workspace, workspace_bytes, cuda_stream, opts);
 }
 
 extern "C" int drm_render_refmaps(const float* env, int B, int He, int We, const int32_t* env_index, const float* z6,

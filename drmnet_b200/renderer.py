@@ -60,24 +60,34 @@ def auto_footprint(roughness: float, res: int = 128, alpha_min: float = 1e-3) ->
     return 16
 
 
+def _env_dtype(envmap: torch.Tensor) -> torch.dtype:
+    """Storage type of an envmap on the device: fp16 stays fp16 (the render reads it natively), the rest becomes fp32."""
+    return torch.float16 if envmap.dtype == torch.float16 else torch.float32
+
+
 def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor, *,
                  env_index: Optional[torch.Tensor] = None, flip: Optional[torch.Tensor] = None,
                  brdf_param_names: Optional[Sequence[str]] = None, res: int = 128, footprint_S=1,
                  alpha_min: float = 0.0, channel_first: bool = True, out: Optional[torch.Tensor] = None,
                  options=None, flat: bool = False, check_status: bool = False) -> torch.Tensor:
-    """N renders in one launch.  envmaps [B,He,We,3] fp32 CUDA; z [N,P]; view_from [N,3]; env_index [N] int (default
-    arange, needs N == B); flip [N] bool; footprint_S 1, 2, 4, 8 or 16: an int, one per render, or None (chosen per
+    """N renders in one launch.  envmaps [B,He,We,3] fp32 or fp16 CUDA; z [N,P]; view_from [N,3]; env_index [N] int
+    (default arange, needs N == B); flip [N] bool; footprint_S 1, 2, 4, 8 or 16: an int, one per render, or None (chosen per
     render from its roughness by ``auto_footprint``).  Returns [N,3,res,res] (or [N,res,res,3]).
 
     ``options``: a ``_lib.RenderOptions`` (accuracy / cost constants, default ``_lib.default_render_options()``).
     ``flat=True`` evaluates the same sum pair by pair (``drm_render_refmaps_flat``, the validation path; any S in 1..16).
-    ``check_status=True`` synchronises and raises if a traversal list overflowed or an env_index was out of range."""
+    ``check_status=True`` synchronises and raises if a traversal list overflowed or an env_index was out of range.
+
+    An fp16 envmap is read in place (``drm_render_refmaps_half``: no fp32 copy) and gives bit for bit the result of its
+    fp32 upcast.  fp16 ends at 65504: brighter texels (a sun) become inf, so convert with ``env.clamp(max=65504).half()``.
+    ``flat=True`` and every other dtype render an fp32 copy."""
     if not (isinstance(envmaps, torch.Tensor) and envmaps.is_cuda):
         raise RuntimeError("envmaps must be a CUDA tensor: drmnet_b200 has no CPU path")
     if envmaps.dim() != 4 or envmaps.shape[-1] != 3:
         raise ValueError(f"envmaps {tuple(envmaps.shape)}: expected [B,He,We,3]")
     device = envmaps.device
-    envmaps = envmaps.contiguous().float()
+    half = envmaps.dtype == torch.float16 and not flat
+    envmaps = envmaps.contiguous() if half else envmaps.contiguous().float()
     B, He, We, _ = envmaps.shape
     z = z.to(device=device, dtype=torch.float32)
     if z.dim() != 2:
@@ -166,8 +176,9 @@ def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor
             ctypes.memmove(ctypes.byref(o), ctypes.byref(options if options is not None else _lib.default_render_options()),
                            ctypes.sizeof(o))
             o.footprint_per_render = per_render.data_ptr()
-        _lib.check(L.drm_render_refmaps_opts(*common_args(S_call, z6, view_from, env_index, flip, out, ws),
-                                             ctypes.byref(o) if o is not None else None))
+        render = L.drm_render_refmaps_half if half else L.drm_render_refmaps_opts
+        _lib.check(render(*common_args(S_call, z6, view_from, env_index, flip, out, ws),
+                          ctypes.byref(o) if o is not None else None))
         if check_status:
             st = (ctypes.c_int * 40)()
             _lib.check(L.drm_render_status(ws.data_ptr(), st, stream))
@@ -182,6 +193,9 @@ def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor
 
 class B200RefMapRenderer:
     """Same interface as MitsubaRefMapRenderer (utils/mitsuba3_utils.py:317-339, 411-430).
+
+    ``rendering`` keeps an fp16 envmap in fp16 (half the memory, the same image as its fp32 upcast; see ``render_batch``
+    for the 65504 limit) and converts every other dtype to fp32.
 
     Extra keywords: ``footprint_S`` (Gauss-Legendre sub-normals per cell and axis; None = chosen from the roughness of
     each call, which costs one device-to-host read of z) and ``alpha_min`` (None = max(1e-3, 1.25*pi/He)).  ``spp`` and
@@ -255,7 +269,7 @@ class B200RefMapRenderer:
         if new_scene:
             if envmap is None:
                 raise AttributeError("new_scene=True needs an envmap ('NoneType' object has no attribute 'cuda')")
-            env = envmap.to(self.device, torch.float32)
+            env = envmap.to(self.device, _env_dtype(envmap))
             if view_from is not None:
                 self._new_scene_view = torch.as_tensor(view_from, dtype=torch.float32).detach().cpu()
             if flip is not None:
@@ -264,7 +278,7 @@ class B200RefMapRenderer:
             z6 = self._compose_z6(z, names, torch.tensor(_SCENE_DEFAULTS, device=self.device))
         else:
             if envmap is not None:
-                self._envmap = envmap.to(self.device, torch.float32)
+                self._envmap = envmap.to(self.device, _env_dtype(envmap))
             if view_from is not None:
                 self._view = torch.as_tensor(view_from, dtype=torch.float32).detach().cpu()
             if flip is not None:

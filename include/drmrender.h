@@ -114,6 +114,17 @@ int drm_render_refmaps_opts(const float* env, int B, int He, int We,
                             float* out, void* workspace, size_t workspace_bytes, void* cuda_stream,
                             const DrmRenderOptions* opts);
 
+/* drm_render_refmaps_opts on an fp16 envmap: env is __half [B, He, We, 3] (IEEE binary16, device), read in place and
+ * converted to fp32 texel by texel.  The conversion is exact, so the result is bit for bit that of
+ * drm_render_refmaps_opts on the same map upcast to fp32, at half the envmap bytes.  Same arguments, validation,
+ * workspace (drm_render_workspace_bytes), status words (drm_render_status) and options.  fp16 ends at 65504: radiance
+ * above it (a sun) is +inf in the map and renders as inf or NaN, so convert with a clamp (torch: env.clamp(max=65504).half()). */
+int drm_render_refmaps_half(const void* env, int B, int He, int We,
+                            const int32_t* env_index, const float* z6, const float* view3, const uint8_t* flip,
+                            int N, int res, int footprint_S, float alpha_min, int channel_first,
+                            float* out, void* workspace, size_t workspace_bytes, void* cuda_stream,
+                            const DrmRenderOptions* opts);
+
 /* Copies the 40 status words of a finished (or enqueued: the copy is stream-ordered) render to status_host[40]:
  * [0] flags, 0 = clean: bit 0 = the pool of hand-over lists ran out (result incomplete), bit 1 = an env_index was out of
  * range, bit 2 = a traversal stack overflowed (result incomplete); [1] deepest traversal stack; [2..6] longest hand-over
