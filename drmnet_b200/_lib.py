@@ -68,6 +68,15 @@ def lib() -> ctypes.CDLL:
                                           ctypes.POINTER(RenderOptions)]
     L.drm_render_refmaps_half.restype = i32
     L.drm_render_refmaps_half.argtypes = L.drm_render_refmaps_opts.argtypes
+    L.drm_env_pyramid_bytes.restype = sz
+    L.drm_env_pyramid_bytes.argtypes = [i32] * 3
+    L.drm_env_pyramid_build.restype = i32
+    L.drm_env_pyramid_build.argtypes = [vp, i32, i32, i32, i32, vp, i32, vp, sz, vp]
+    L.drm_render_prepared_workspace_bytes.restype = sz
+    L.drm_render_prepared_workspace_bytes.argtypes = [i32] * 6
+    L.drm_render_refmaps_prepared.restype = i32
+    L.drm_render_refmaps_prepared.argtypes = [vp, i32, vp, sz, i32, i32, i32, vp, vp, vp, vp, i32, i32, i32, f32, i32,
+                                              vp, vp, sz, vp, ctypes.POINTER(RenderOptions)]
     L.drm_render_default_options.restype = None
     L.drm_render_default_options.argtypes = [ctypes.POINTER(RenderOptions)]
     L.drm_render_status.restype = i32
@@ -110,6 +119,8 @@ def check(code: int) -> None:
 
 EXPORTED_SYMBOLS = ["drm_version", "drm_last_error", "drm_launch_count", "drm_render_workspace_bytes", "drm_render_refmaps",
                     "drm_render_refmaps_opts", "drm_render_refmaps_half", "drm_render_default_options", "drm_render_status",
+                    "drm_env_pyramid_bytes", "drm_env_pyramid_build", "drm_render_prepared_workspace_bytes",
+                    "drm_render_refmaps_prepared",
                     "drm_render_flat_workspace_bytes", "drm_render_refmaps_flat",
                     "drm_img2refmap_workspace_bytes", "drm_img2refmap", "drm_img2refmap_status", "drm_normals_to_thetaphi",
                     "drm_refmap_postprocess", "drm_mirmap2envmap", "drm_refmap_lookup", "drm_normalized_log",

@@ -95,19 +95,26 @@ def refmap_postprocess(stacks: torch.Tensor, refmap_input_scaler: Optional[float
     return out, scale
 
 
-def synthesize_refmaps(renderer: B200RefMapRenderer, stacked_z: torch.Tensor, envmap: torch.Tensor,
+def synthesize_refmaps(renderer: B200RefMapRenderer, stacked_z: torch.Tensor, envmap,
                        view_from: torch.Tensor, cached: Optional[List[Optional[torch.Tensor]]] = None,
                        brdf_param_names: Optional[Sequence[str]] = None, refmap_input_scaler: Optional[float] = 0.12,
-                       transform: str = "log"):
+                       transform: str = "log", env_ids: Optional[torch.Tensor] = None):
     """Training-data synthesis of DRMNet.get_input (models/drmnet.py:523-569, 610-620) as two launches.
 
     stacked_z [G,B,P] (LrK, Lrk, Lrkm1[, r0]); envmap [B,He,We,3]; view_from [B,3]; ``cached[g]`` is either None or a
     [B,3,res,res] tensor whose entries with NaN at [b,0,0,0] are cache misses (the dataset's sentinel,
     dataset/parametricrefmap.py:174-193).  Only misses are rendered.  Returns (list of G transformed [B,3,res,res]
-    tensors, normalizing_scale [B], raw stacks [G,B,3,res,res])."""
+    tensors, normalizing_scale [B], raw stacks [G,B,3,res,res]).
+
+    ``envmap`` may also be an ``EnvmapBank`` of resident maps, with ``env_ids`` [B]: batch element b uses slot
+    ``env_ids[b]``, and no map is shipped or re-read per step.  ``env_ids`` applies to an [E,He,We,3] tensor too."""
     G, B = stacked_z.shape[0], stacked_z.shape[1]
     res = renderer.refmap_res
     device = envmap.device
+    if env_ids is not None:
+        env_ids = torch.as_tensor(env_ids).to(device=device, dtype=torch.int64).reshape(-1)
+        if env_ids.numel() != B:
+            raise ValueError(f"env_ids has {env_ids.numel()} entries for a batch of {B}")
     raw = torch.empty((G, B, 3, res, res), dtype=torch.float32, device=device)
     need = torch.ones((G, B), dtype=torch.bool, device=device)
     if cached is not None:
@@ -118,7 +125,8 @@ def synthesize_refmaps(renderer: B200RefMapRenderer, stacked_z: torch.Tensor, en
     idx = torch.nonzero(need.T)  # (batch_idx, stack_idx): the reference's iteration order (models/drmnet.py:561)
     if idx.numel():
         b_idx, g_idx = idx[:, 0], idx[:, 1]
-        out = render_batch(envmap, stacked_z.to(device)[g_idx, b_idx], view_from.to(device)[b_idx], env_index=b_idx,
+        out = render_batch(envmap, stacked_z.to(device)[g_idx, b_idx], view_from.to(device)[b_idx],
+                           env_index=b_idx if env_ids is None else env_ids[b_idx],
                            brdf_param_names=brdf_param_names or renderer.brdf_param_names, res=res,
                            footprint_S=renderer.footprint_S, alpha_min=renderer.alpha_min or 0.0, channel_first=True)
         raw[g_idx, b_idx] = out

@@ -300,6 +300,17 @@ __global__ void tree_mark_used_kernel(const TreeConst* __restrict__ rc, int N, i
     if (k < N && rc[k].has_diff) used[rc[k].env] = 1;
 }
 
+// drm_env_pyramid_build: mark the listed slots of a bank (ids == NULL: every slot); ids outside [0, B) are skipped
+__global__ void env_mark_slots_kernel(const int32_t* __restrict__ ids, int n, int B, int* __restrict__ used) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (!ids) {
+        if (i < B) used[i] = 1;
+    } else if (i < n) {
+        const int e = ids[i];
+        if (e >= 0 && e < B) used[e] = 1;
+    }
+}
+
 // per lattice pass p: the renders of this chunk whose own lattice is at least 2^p (one thread: a chunk has <= 64 renders)
 __global__ void tree_active_kernel(const TreeConst* __restrict__ rc, int n, int* __restrict__ act, int* __restrict__ nact) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
@@ -1338,19 +1349,26 @@ static int log2_exact(int S) {
     return -1;
 }
 
-// S: 1, 2, 4, 8, 16 = that footprint for every render; 0 = per render (given, or chosen on the device): sized for 16
-static size_t tree_layout(TreeLayout& L, void* ws, int N, int B, int He, int We, int res, int S) {
-    make_geom(L.gs, He, We, 1);
-    // the diffuse lobe reads no cell wider than ~0.03 rad: level 3 at 1000 rows, level 1 at 250 rows
+// the diffuse pyramid of an He x We envmap: the lobe reads no cell wider than ~0.03 rad, so the stored levels start at
+// level 3 at 1000 rows, level 1 at 250 rows
+static void make_diffuse_geom(PyrGeom& G, int He, int We) {
     int dbase = 0;
     while ((2 << dbase) * M_PI / He <= 0.03) ++dbase;
-    make_geom(L.gd, He, We, dbase);
+    make_geom(G, He, We, dbase);
+}
+
+// S: 1, 2, 4, 8, 16 = that footprint for every render; 0 = per render (given, or chosen on the device): sized for 16.
+// prepared: the diffuse pyramids come from the caller (drm_render_refmaps_prepared), so neither they nor the mask of
+// the envmaps in use take workspace.
+static size_t tree_layout(TreeLayout& L, void* ws, int N, int B, int He, int We, int res, int S, bool prepared = false) {
+    make_geom(L.gs, He, We, 1);
+    make_diffuse_geom(L.gd, He, We);
     L.pk = S > 0 ? log2_exact(S) : TREE_MAX_P;
     const int NC = N < TREE_CHUNK ? N : TREE_CHUNK;
     Carver c(ws);
     L.status = c.take<int>(64);
     L.rc = c.take<TreeConst>(N);
-    L.env_used = c.take<int>(B);
+    L.env_used = prepared ? nullptr : c.take<int>(B);
     L.act = c.take<int>((TREE_MAX_P + 1) * TREE_CHUNK);
     L.nact = c.take<int>(16);
     L.sin_t = c.take<float>(He);
@@ -1358,7 +1376,7 @@ static size_t tree_layout(TreeLayout& L, void* ws, int N, int B, int He, int We,
     L.sin_p = c.take<float>(We);
     L.cos_p = c.take<float>(We);
     L.pyr_s = c.take<float4>((size_t)NC * L.gs.cells * REC4);
-    L.pyr_d = c.take<float4>((size_t)B * L.gd.cells * REC4);
+    L.pyr_d = prepared ? nullptr : c.take<float4>((size_t)B * L.gd.cells * REC4);
     // hand-over lists: pass p writes nblocks[p] chains that pass p + 1 reads; two pools alternate, sized for the average
     // list (the longest ones, at the limb, reach ~3000 entries) with a factor 3 of slack
     size_t need[2] = {1, 1}, needh[2] = {1, 1};
@@ -1381,6 +1399,31 @@ static size_t tree_layout(TreeLayout& L, void* ws, int N, int B, int He, int We,
     return c.used();
 }
 
+// Buffer of drm_env_pyramid_build: the diffuse pyramids [B][gd.cells][REC4] at offset 0 (where the render reads them),
+// then the build's scratch: the direction tables of the texel rows and columns and the mask of the slots to build.
+struct EnvPyrLayout {
+    PyrGeom gd;
+    float4* pyr;
+    float *sin_t, *cos_t, *sin_p, *cos_p;
+    int* used;
+};
+
+static size_t env_pyr_layout(EnvPyrLayout& L, void* buf, int B, int He, int We) {
+    make_diffuse_geom(L.gd, He, We);
+    Carver c(buf);
+    L.pyr = c.take<float4>((size_t)B * L.gd.cells * REC4);
+    L.sin_t = c.take<float>(He);
+    L.cos_t = c.take<float>(He);
+    L.sin_p = c.take<float>(We);
+    L.cos_p = c.take<float>(We);
+    L.used = c.take<int>(B);
+    return c.used();
+}
+
+static bool env_sizes_ok(int B, int He, int We) {
+    return B > 0 && B <= 65535 && He > 0 && We > 0 && (long)He * We < (1L << 28);
+}
+
 static constexpr size_t TREE_SMEM = (size_t)TREE_WARPS * STACK_CAP * 4 + (size_t)TREE_WARPS * (BUF1 / 2) * PAIR4 * 16 +
                                     (size_t)TREE_WARPS * BUF0 * 2 * 16;
 static_assert(BUF1 * SREC4 <= (BUF1 / 2) * PAIR4 + 8 * BUF0, "the diffuse pass stages its records in the same region");
@@ -1399,6 +1442,25 @@ template <> struct TexelKernels<__half> {
     static constexpr void (*diff)(TreeArgs) = tree_diff_kernel_h;
     template <bool SPEC> static constexpr void (*pyr)(TreeArgs, int, float4*) = pyr_from_texels_kernel_h<SPEC>;
 };
+
+// the diffuse pyramids of the envmaps with g.env_used set (blockIdx.y = envmap; the others exit at once).  g needs env,
+// the direction tables, gd, He, We and domega_k.  Returns the kernels launched.
+template <typename T>
+static int launch_diffuse_pyramids(const TreeArgs& g, int B, float4* pyr, cudaStream_t st) {
+    if (g.gd.L < 1) return 0;
+    const int tb = 128;
+    const int first = g.gd.base > 0 ? g.gd.base : 1;  // base 0: texels are read directly, level 1 is the first stored
+    const int nb = g.gd.H[first] * g.gd.W[first];
+    int launches = 0;
+    TexelKernels<T>::template pyr<false><<<dim3((nb + tb - 1) / tb, B), tb, 0, st>>>(g, first, pyr);
+    ++launches;
+    for (int l = first + 1; l <= g.gd.L; ++l) {
+        const int nl = g.gd.H[l] * g.gd.W[l];
+        pyr_merge_kernel<<<dim3((nl + tb - 1) / tb, B), tb, 0, st>>>(g.gd, l, pyr, g.env_used);
+        ++launches;
+    }
+    return launches;
+}
 
 // Pass P on a persistent grid of (SMs x resident CTAs of this instance), at most one CTA per item.  The grid size is
 // queried once per device and instance (fp32 and fp16 instances have their own slots).
@@ -1436,6 +1498,55 @@ extern "C" size_t drm_render_workspace_bytes(int N, int B, int He, int We, int r
     return tree_layout(L, nullptr, N, B, He, We, res, S);
 }
 
+extern "C" size_t drm_render_prepared_workspace_bytes(int N, int B, int He, int We, int res, int S) {
+    if (N <= 0 || B <= 0 || He <= 0 || We <= 0 || res <= 0 || (S != 0 && log2_exact(S) < 0)) return 0;
+    if ((long)He * We >= (1L << 28)) return 0;
+    TreeLayout L;
+    return tree_layout(L, nullptr, N, B, He, We, res, S, true);
+}
+
+extern "C" size_t drm_env_pyramid_bytes(int B, int He, int We) {
+    if (!env_sizes_ok(B, He, We)) return 0;
+    EnvPyrLayout P;
+    return env_pyr_layout(P, nullptr, B, He, We);
+}
+
+template <typename T>
+static int env_pyramid_build(const T* env, int B, int He, int We, const int32_t* ids, int n_ids, void* pyramids,
+                             size_t pyramid_bytes, cudaStream_t st) {
+    EnvPyrLayout P;
+    const size_t need = env_pyr_layout(P, pyramids, B, He, We);
+    DRM_REQUIRE(pyramid_bytes >= need, "env_pyramid_build: pyramid buffer of %zu bytes needed for B=%d He=%d We=%d, %zu given",
+                need, B, He, We, pyramid_bytes);
+    if (ids && n_ids == 0) return DRM_OK;
+    TreeArgs g;
+    memset(&g, 0, sizeof(g));
+    g.env = reinterpret_cast<const float*>(env); g.sin_t = P.sin_t; g.cos_t = P.cos_t; g.sin_p = P.sin_p; g.cos_p = P.cos_p;
+    g.env_used = P.used; g.gd = P.gd;
+    g.B = B; g.He = He; g.We = We;
+    g.domega_k = (float)((2.0 * M_PI / We) * (M_PI / He));
+    const int tb = 128;
+    tree_tables_kernel<<<(max(He, We) + tb - 1) / tb, tb, 0, st>>>(P.sin_t, P.cos_t, P.sin_p, P.cos_p, He, We);
+    if (ids) DRM_CHECK_CUDA(cudaMemsetAsync(P.used, 0, sizeof(int) * B, st));
+    const int nmark = ids ? n_ids : B;
+    env_mark_slots_kernel<<<(nmark + tb - 1) / tb, tb, 0, st>>>(ids, n_ids, B, P.used);
+    count_launches(2 + launch_diffuse_pyramids<T>(g, B, P.pyr, st));
+    DRM_CHECK_CUDA(cudaGetLastError());
+    return DRM_OK;
+}
+
+extern "C" int drm_env_pyramid_build(const void* env, int env_half, int B, int He, int We, const int32_t* ids, int n_ids,
+                                     void* pyramids, size_t pyramid_bytes, void* cuda_stream) {
+    DRM_REQUIRE(env && pyramids, "env_pyramid_build: null pointer");
+    DRM_REQUIRE(env_sizes_ok(B, He, We), "env_pyramid_build: B=%d He=%d We=%d: sizes must be positive, B <= 65535 and "
+                "He * We < 2^28", B, He, We);
+    DRM_REQUIRE(!ids || n_ids >= 0, "env_pyramid_build: n_ids=%d must not be negative", n_ids);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    if (env_half)
+        return env_pyramid_build(static_cast<const __half*>(env), B, He, We, ids, n_ids, pyramids, pyramid_bytes, st);
+    return env_pyramid_build(static_cast<const float*>(env), B, He, We, ids, n_ids, pyramids, pyramid_bytes, st);
+}
+
 extern "C" int drm_render_status(const void* workspace, int* status_host, void* cuda_stream) {
     DRM_REQUIRE(workspace && status_host, "render_status: null pointer");
     DRM_CHECK_CUDA(cudaMemcpyAsync(status_host, workspace, 40 * sizeof(int), cudaMemcpyDeviceToHost,
@@ -1443,18 +1554,28 @@ extern "C" int drm_render_status(const void* workspace, int* status_host, void* 
     return DRM_OK;
 }
 
-// drm_render_refmaps_opts (T = float) and drm_render_refmaps_half (T = __half): only the kernels that read texels differ
+// drm_render_refmaps_opts (T = float) and drm_render_refmaps_half (T = __half): only the kernels that read texels differ.
+// prepared (drm_render_refmaps_prepared): the diffuse pyramids of the B envmaps are `pyramids`, built by
+// drm_env_pyramid_build; the call neither marks nor builds any.
 template <typename T>
 static int render_refmaps(const T* env, int B, int He, int We, const int32_t* env_index, const float* z6,
                           const float* view3, const uint8_t* flip, int N, int res, int S, float alpha_min,
                           int channel_first, float* out, void* workspace, size_t workspace_bytes, void* cuda_stream,
-                          const DrmRenderOptions* opts) {
+                          const DrmRenderOptions* opts, bool prepared = false, const void* pyramids = nullptr,
+                          size_t pyramid_bytes = 0) {
     DRM_REQUIRE(env && z6 && view3 && out, "render: null pointer");
+    DRM_REQUIRE(!prepared || pyramids, "render: null pointer (pyramids)");
     DRM_REQUIRE(N > 0 && B > 0 && He > 0 && We > 0 && res > 0, "render: N=%d B=%d He=%d We=%d res=%d must be positive", N, B, He, We, res);
     DRM_REQUIRE(S == 0 || log2_exact(S) >= 0, "render: footprint_S=%d must be 0 (per render) or 1, 2, 4, 8, 16", S);
     DRM_REQUIRE(res <= 4096, "render: res=%d too large", res);
     DRM_REQUIRE(B <= 65535, "render: at most 65535 envmaps per call (B=%d)", B);
     DRM_REQUIRE((long)He * We < (1L << 28), "render: envmap of %d x %d texels is too large", He, We);
+    if (prepared) {
+        EnvPyrLayout P;
+        const size_t pneed = env_pyr_layout(P, nullptr, B, He, We);
+        DRM_REQUIRE(pyramid_bytes >= pneed, "render: pyramid buffer of %zu bytes needed for B=%d He=%d We=%d, %zu given",
+                    pneed, B, He, We, pyramid_bytes);
+    }
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     DrmRenderOptions o;
     drm_render_default_options(&o);
@@ -1462,7 +1583,8 @@ static int render_refmaps(const T* env, int B, int He, int We, const int32_t* en
     const int32_t* S_per_render = o.footprint_per_render;
     const int S_layout = S_per_render ? 0 : S;
     TreeLayout L;
-    const size_t need = tree_layout(L, workspace, N, B, He, We, res, S_layout);
+    const size_t need = tree_layout(L, workspace, N, B, He, We, res, S_layout, prepared);
+    if (prepared) L.pyr_d = static_cast<float4*>(const_cast<void*>(pyramids));
     if (!workspace || workspace_bytes < need) {
         set_error("render: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
         return DRM_EWORKSPACE;
@@ -1494,20 +1616,12 @@ static int render_refmaps(const T* env, int B, int He, int We, const int32_t* en
                                                        o.level_scale * grow, (o.pixel_covariance ? o.level_scale0 : o.level_scale) * grow,
                                                        o.full_second_order ? o.alpha_full2 : 1e30f, o.pixel_covariance, o.flat_scale,
                                                        S, S_per_render, L.rc, L.status);
-    DRM_CHECK_CUDA(cudaMemsetAsync(L.env_used, 0, sizeof(int) * B, st));
-    tree_mark_used_kernel<<<(N + tb - 1) / tb, tb, 0, st>>>(L.rc, N, L.env_used);
-    count_launches(3);
+    count_launches(2);
     // ---- diffuse pyramids of the envmaps in use (view independent: shared by every render of an envmap) --------------
-    if (L.gd.L >= 1) {
-        const int first = L.gd.base > 0 ? L.gd.base : 1;  // base 0: texels are read directly, level 1 is the first stored
-        const int nb = L.gd.H[first] * L.gd.W[first];
-        TexelKernels<T>::template pyr<false><<<dim3((nb + tb - 1) / tb, B), tb, 0, st>>>(g, first, L.pyr_d);
-        count_launches(1);
-        for (int l = first + 1; l <= L.gd.L; ++l) {
-            const int nl = L.gd.H[l] * L.gd.W[l];
-            pyr_merge_kernel<<<dim3((nl + tb - 1) / tb, B), tb, 0, st>>>(L.gd, l, L.pyr_d, L.env_used);
-            count_launches(1);
-        }
+    if (!prepared) {
+        DRM_CHECK_CUDA(cudaMemsetAsync(L.env_used, 0, sizeof(int) * B, st));
+        tree_mark_used_kernel<<<(N + tb - 1) / tb, tb, 0, st>>>(L.rc, N, L.env_used);
+        count_launches(1 + launch_diffuse_pyramids<T>(g, B, L.pyr_d, st));
     }
     DRM_CHECK_CUDA(cudaFuncSetAttribute(TexelKernels<T>::diff, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM));
     DRM_CHECK_CUDA(cudaFuncSetAttribute(TexelKernels<T>::diff, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -1579,6 +1693,20 @@ extern "C" int drm_render_refmaps_half(const void* env, int B, int He, int We, c
                                        void* cuda_stream, const DrmRenderOptions* opts) {
     return render_refmaps(static_cast<const __half*>(env), B, He, We, env_index, z6, view3, flip, N, res, S, alpha_min,
                           channel_first, out, workspace, workspace_bytes, cuda_stream, opts);
+}
+
+extern "C" int drm_render_refmaps_prepared(const void* env, int env_half, const void* pyramids, size_t pyramid_bytes,
+                                           int B, int He, int We, const int32_t* env_index, const float* z6,
+                                           const float* view3, const uint8_t* flip, int N, int res, int S,
+                                           float alpha_min, int channel_first, float* out, void* workspace,
+                                           size_t workspace_bytes, void* cuda_stream, const DrmRenderOptions* opts) {
+    if (env_half)
+        return render_refmaps(static_cast<const __half*>(env), B, He, We, env_index, z6, view3, flip, N, res, S,
+                              alpha_min, channel_first, out, workspace, workspace_bytes, cuda_stream, opts, true,
+                              pyramids, pyramid_bytes);
+    return render_refmaps(static_cast<const float*>(env), B, He, We, env_index, z6, view3, flip, N, res, S, alpha_min,
+                          channel_first, out, workspace, workspace_bytes, cuda_stream, opts, true, pyramids,
+                          pyramid_bytes);
 }
 
 extern "C" int drm_render_refmaps(const float* env, int B, int He, int We, const int32_t* env_index, const float* z6,

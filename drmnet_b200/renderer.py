@@ -65,7 +65,77 @@ def _env_dtype(envmap: torch.Tensor) -> torch.dtype:
     return torch.float16 if envmap.dtype == torch.float16 else torch.float32
 
 
-def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor, *,
+class EnvmapBank:
+    """Envmaps resident on the device with their diffuse pyramids built once (``drm_env_pyramid_build``).
+
+    ``envmaps`` [B,He,We,3] CUDA: fp16 stays fp16 and every other dtype becomes fp32, as in ``render_batch``.  A map
+    that is already contiguous in that dtype is used in place, not copied.  Pass the bank to ``render_batch`` (or
+    ``synthesize_refmaps``) instead of the maps: ``env_index`` then holds bank slots, and the render reads the pyramids
+    instead of building those of the maps it uses on every call.  Its refmaps are bit for bit those of
+    ``render_batch`` on the plain maps, and its workspace does not grow with B.
+
+    The diffuse pyramid depends on the texels only, so a bank is built once per map set.  ``update(ids, maps)`` copies
+    new maps into slots, ``update(ids)`` re-reads slots changed in place, and both rebuild only those slots.  The bank
+    records the version counter of its maps: a render after an in-place change that no ``update`` followed raises
+    instead of reading a stale pyramid.  Builds run on the current stream; renders on another stream must wait for
+    them."""
+
+    def __init__(self, envmaps: torch.Tensor):
+        if not (isinstance(envmaps, torch.Tensor) and envmaps.is_cuda):
+            raise RuntimeError("envmaps must be a CUDA tensor: drmnet_b200 has no CPU path")
+        if envmaps.dim() != 4 or envmaps.shape[-1] != 3:
+            raise ValueError(f"envmaps {tuple(envmaps.shape)}: expected [B,He,We,3]")
+        self.maps = envmaps.to(_env_dtype(envmaps)).contiguous()
+        self.B, self.He, self.We = (int(s) for s in self.maps.shape[:3])
+        self.half = self.maps.dtype == torch.float16
+        self.device = self.maps.device
+        nbytes = _lib.lib().drm_env_pyramid_bytes(self.B, self.He, self.We)
+        if nbytes == 0:
+            raise ValueError(f"EnvmapBank: unsupported sizes B={self.B} He={self.He} We={self.We}")
+        self.pyramids = torch.empty(int(nbytes), dtype=torch.uint8, device=self.device)
+        self._build(None)
+
+    def _build(self, ids: Optional[torch.Tensor]) -> None:
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().drm_env_pyramid_build(
+                self.maps.data_ptr(), int(self.half), self.B, self.He, self.We,
+                ids.data_ptr() if ids is not None else None, ids.numel() if ids is not None else 0,
+                self.pyramids.data_ptr(), self.pyramids.numel(), torch.cuda.current_stream(self.device).cuda_stream))
+        self._version = self.maps._version
+
+    def update(self, ids, maps: Optional[torch.Tensor] = None) -> None:
+        """Rebuild the pyramids of slots ``ids`` (a list or an int tensor).  With ``maps``
+        [len(ids),He,We,3] the maps are first copied into those slots (converted to the bank's dtype); without, the
+        slots are re-read as they are, after the caller changed them in place.  ``update`` declares that no other slot
+        changed: the bank's version counter is taken as current afterwards."""
+        ids_host = torch.as_tensor(ids, dtype=torch.int64).reshape(-1).cpu()
+        if ids_host.numel() and (int(ids_host.min()) < 0 or int(ids_host.max()) >= self.B):
+            raise IndexError(f"EnvmapBank.update: slots must be in [0, {self.B})")
+        if ids_host.unique().numel() != ids_host.numel():
+            raise ValueError("EnvmapBank.update: repeated slot")
+        if ids_host.numel() == 0:  # an empty device tensor has a null pointer, which the build reads as "every slot"
+            self._version = self.maps._version
+            return
+        dev_ids = ids_host.to(self.device)
+        if maps is not None:
+            if tuple(maps.shape) != (ids_host.numel(), self.He, self.We, 3):
+                raise ValueError(f"EnvmapBank.update: maps {tuple(maps.shape)}, expected "
+                                 f"[{ids_host.numel()},{self.He},{self.We},3]")
+            self.maps.index_copy_(0, dev_ids, maps.to(self.device, self.maps.dtype))
+        self._build(dev_ids.to(torch.int32))
+
+    @property
+    def stale(self) -> bool:
+        """True when the maps changed in place since the last build or ``update``."""
+        return self.maps._version != self._version
+
+    def check_fresh(self) -> None:
+        if self.stale:
+            raise RuntimeError("EnvmapBank: the maps changed in place after the pyramids were built; call "
+                               "update(ids) with the changed slots before rendering")
+
+
+def render_batch(envmaps, z: torch.Tensor, view_from: torch.Tensor, *,
                  env_index: Optional[torch.Tensor] = None, flip: Optional[torch.Tensor] = None,
                  brdf_param_names: Optional[Sequence[str]] = None, res: int = 128, footprint_S=1,
                  alpha_min: float = 0.0, channel_first: bool = True, out: Optional[torch.Tensor] = None,
@@ -80,7 +150,16 @@ def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor
 
     An fp16 envmap is read in place (``drm_render_refmaps_half``: no fp32 copy) and gives bit for bit the result of its
     fp32 upcast.  fp16 ends at 65504: brighter texels (a sun) become inf, so convert with ``env.clamp(max=65504).half()``.
-    ``flat=True`` and every other dtype render an fp32 copy."""
+    ``flat=True`` and every other dtype render an fp32 copy.
+
+    ``envmaps`` may be an ``EnvmapBank``: ``env_index`` then holds its slots, and the render reads the bank's diffuse
+    pyramids (``drm_render_refmaps_prepared``) with the same result.  ``flat=True`` renders the bank's maps as before."""
+    bank = None
+    if isinstance(envmaps, EnvmapBank):
+        envmaps.check_fresh()
+        if not flat:
+            bank = envmaps
+        envmaps = envmaps.maps
     if not (isinstance(envmaps, torch.Tensor) and envmaps.is_cuda):
         raise RuntimeError("envmaps must be a CUDA tensor: drmnet_b200 has no CPU path")
     if envmaps.dim() != 4 or envmaps.shape[-1] != 3:
@@ -165,7 +244,8 @@ def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor
                 if part is not out:
                     out.index_copy_(0, ids, part)
             return out
-        nbytes = L.drm_render_workspace_bytes(N, B, He, We, int(res), 0 if per_render is not None else S_call)
+        ws_bytes = L.drm_render_prepared_workspace_bytes if bank is not None else L.drm_render_workspace_bytes
+        nbytes = ws_bytes(N, B, He, We, int(res), 0 if per_render is not None else S_call)
         if nbytes == 0:
             raise ValueError(f"render_batch: unsupported sizes N={N} B={B} He={He} We={We} res={res} S={footprint_S} "
                              "(footprints are 1, 2, 4, 8 or 16)")
@@ -176,9 +256,15 @@ def render_batch(envmaps: torch.Tensor, z: torch.Tensor, view_from: torch.Tensor
             ctypes.memmove(ctypes.byref(o), ctypes.byref(options if options is not None else _lib.default_render_options()),
                            ctypes.sizeof(o))
             o.footprint_per_render = per_render.data_ptr()
-        render = L.drm_render_refmaps_half if half else L.drm_render_refmaps_opts
-        _lib.check(render(*common_args(S_call, z6, view_from, env_index, flip, out, ws),
-                          ctypes.byref(o) if o is not None else None))
+        opts = ctypes.byref(o) if o is not None else None
+        if bank is not None:
+            _lib.check(L.drm_render_refmaps_prepared(envmaps.data_ptr(), int(half), bank.pyramids.data_ptr(),
+                                                     bank.pyramids.numel(),
+                                                     *common_args(S_call, z6, view_from, env_index, flip, out, ws)[1:],
+                                                     opts))
+        else:
+            render = L.drm_render_refmaps_half if half else L.drm_render_refmaps_opts
+            _lib.check(render(*common_args(S_call, z6, view_from, env_index, flip, out, ws), opts))
         if check_status:
             st = (ctypes.c_int * 40)()
             _lib.check(L.drm_render_status(ws.data_ptr(), st, stream))
@@ -195,7 +281,9 @@ class B200RefMapRenderer:
     """Same interface as MitsubaRefMapRenderer (utils/mitsuba3_utils.py:317-339, 411-430).
 
     ``rendering`` keeps an fp16 envmap in fp16 (half the memory, the same image as its fp32 upcast; see ``render_batch``
-    for the 65504 limit) and converts every other dtype to fp32.
+    for the 65504 limit) and converts every other dtype to fp32.  The persistent envmap is kept as an ``EnvmapBank`` of
+    one: its diffuse pyramid is built when an envmap is given or the persistent one changed in place, and calls with
+    ``envmap=None`` reuse it (the same image, fewer launches).  ``new_scene=True`` renders build it per call, as before.
 
     Extra keywords: ``footprint_S`` (Gauss-Legendre sub-normals per cell and axis; None = chosen from the roughness of
     each call, which costs one device-to-host read of z) and ``alpha_min`` (None = max(1e-3, 1.25*pi/He)).  ``spp`` and
@@ -222,6 +310,11 @@ class B200RefMapRenderer:
         self.device = torch.device(device)
         # persistent-scene state (mitsuba3_utils.py:229-243): envmap, sensor transform, flip, BSDF parameters
         self._envmap: Optional[torch.Tensor] = None
+        # the persistent envmap as a bank of one: its diffuse pyramid is built when the map is set or changed in place
+        # (identity and version counter of _envmap), not on every call
+        self._bank: Optional[EnvmapBank] = None
+        self._bank_src: Optional[torch.Tensor] = None
+        self._bank_version = -1
         self._view = torch.tensor(init_view_from, dtype=torch.float32)
         self._flip = False
         self._bsdf = torch.tensor(_SCENE_DEFAULTS, dtype=torch.float32)
@@ -279,6 +372,7 @@ class B200RefMapRenderer:
         else:
             if envmap is not None:
                 self._envmap = envmap.to(self.device, _env_dtype(envmap))
+                self._bank = None
             if view_from is not None:
                 self._view = torch.as_tensor(view_from, dtype=torch.float32).detach().cpu()
             if flip is not None:
@@ -286,12 +380,12 @@ class B200RefMapRenderer:
             if self._envmap is None:
                 # the reference would render its initial all-zero bitmap (mitsuba3_utils.py:112)
                 self._envmap = torch.zeros(*self.envmap_size, 3, device=self.device)
-            env, view, do_flip = self._envmap, self._view, self._flip
+            env, view, do_flip = self._persistent_bank(), self._view, self._flip
             # parameters that are not named keep their last value in the persistent scene
             self._bsdf = z6 = self._compose_z6(z, names, self._bsdf.to(self.device))
         res = self._film_res(sensor)
         S = self.footprint_S  # None: chosen on the device from the roughness (no host read of z)
-        img = render_batch(env[None], z6[None], view[None].to(self.device),
+        img = render_batch(env if isinstance(env, EnvmapBank) else env[None], z6[None], view[None].to(self.device),
                            flip=torch.tensor([do_flip], device=self.device), res=res, footprint_S=S,
                            alpha_min=self.alpha_min or 0.0, channel_first=channel_first)[0]
         if not self.return_normal and not self.return_depth:
@@ -302,6 +396,14 @@ class B200RefMapRenderer:
         if self.return_depth:
             outputs.append(self._depth_aov(res, channel_first))
         return outputs
+
+    def _persistent_bank(self) -> EnvmapBank:
+        """The bank of the persistent envmap, rebuilt when the envmap was replaced or changed in place."""
+        env = self._envmap
+        if self._bank is None or self._bank_src is not env or self._bank_version != env._version:
+            self._bank = EnvmapBank(env[None])
+            self._bank_src, self._bank_version = env, env._version
+        return self._bank
 
     # analytic AOVs of the sphere seen by the refmap sensor (cell centres), mitsuba3_utils.py:199-214
     def _normal_aov(self, res, do_flip, channel_first):

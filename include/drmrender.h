@@ -125,6 +125,37 @@ int drm_render_refmaps_half(const void* env, int B, int He, int We,
                             float* out, void* workspace, size_t workspace_bytes, void* cuda_stream,
                             const DrmRenderOptions* opts);
 
+/* Envmap banks: the diffuse pyramid of an envmap depends on its texels alone (not on the view, the BRDF or the refmap),
+ * so a caller that renders the same maps many times builds it once and renders by index.
+ *
+ * drm_env_pyramid_bytes: size of the buffer that holds the diffuse pyramids of B envmaps of He x We texels.  It starts
+ *   with the pyramids, [B][cells][5] float4 records (cells depends on He and We), and ends with the build's scratch
+ *   (direction tables and a mask of B ints).  0 for unsupported sizes (B > 65535, He * We >= 2^28).
+ * drm_env_pyramid_build: builds the pyramids of the listed slots of env [B, He, We, 3] (fp32, or __half when env_half
+ *   is nonzero) into `pyramids`.  ids [n_ids] int32 (device) lists the slots to build; ids outside [0, B) are skipped;
+ *   NULL builds every slot.  The other slots keep their records.  A pyramid is valid only for the texels, He and We it
+ *   was built from: rebuild a slot after its texels change.  Builds and renders that share a buffer must be ordered
+ *   (one stream, or events).
+ * drm_render_prepared_workspace_bytes / drm_render_refmaps_prepared: drm_render_refmaps_opts (drm_render_refmaps_half
+ *   when env_half is nonzero) reading the diffuse pyramids from `pyramids` instead of building those of the envmaps in
+ *   use in the workspace, so the workspace does not grow with B.  Bit for bit the result of drm_render_refmaps_opts on
+ *   the same maps; same validation, status words (drm_render_status) and options.
+ * Both entries check null pointers and sizes, and refuse a pyramid buffer smaller than drm_env_pyramid_bytes
+ * (DRM_EINVAL, with the size needed in drm_last_error), before any CUDA call. */
+size_t drm_env_pyramid_bytes(int B, int He, int We);
+
+int drm_env_pyramid_build(const void* env, int env_half, int B, int He, int We, const int32_t* ids, int n_ids,
+                          void* pyramids, size_t pyramid_bytes, void* cuda_stream);
+
+size_t drm_render_prepared_workspace_bytes(int N, int B, int He, int We, int res, int footprint_S);
+
+int drm_render_refmaps_prepared(const void* env, int env_half, const void* pyramids, size_t pyramid_bytes,
+                                int B, int He, int We,
+                                const int32_t* env_index, const float* z6, const float* view3, const uint8_t* flip,
+                                int N, int res, int footprint_S, float alpha_min, int channel_first,
+                                float* out, void* workspace, size_t workspace_bytes, void* cuda_stream,
+                                const DrmRenderOptions* opts);
+
 /* Copies the 40 status words of a finished (or enqueued: the copy is stream-ordered) render to status_host[40]:
  * [0] flags, 0 = clean: bit 0 = the pool of hand-over lists ran out (result incomplete), bit 1 = an env_index was out of
  * range, bit 2 = a traversal stack overflowed (result incomplete); [1] deepest traversal stack; [2..6] longest hand-over
