@@ -91,6 +91,12 @@ def lib() -> ctypes.CDLL:
     L.drm_img2refmap.argtypes = [vp, vp, i32, vp, i64, i32, i32, i32, f32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     L.drm_img2refmap_status.restype = i32
     L.drm_img2refmap_status.argtypes = [vp, i64, i32, i32, f32, ctypes.POINTER(ctypes.c_int32 * 2), vp]
+    L.drm_img2refmap_dense_workspace_bytes.restype = sz
+    L.drm_img2refmap_dense_workspace_bytes.argtypes = [i32, i32, i32, i32, f32]
+    L.drm_img2refmap_dense.restype = i32
+    i64p = ctypes.POINTER(i64)
+    L.drm_img2refmap_dense.argtypes = [vp, i64p, vp, i64p, vp, i32, i32, i32, i32, i32, f32, i32, i32, vp, vp, vp, vp, vp,
+                                       sz, vp]
     L.drm_refmap_postprocess.restype = i32
     L.drm_refmap_postprocess.argtypes = [vp, i32, i32, i32, f32, i32, vp, vp, vp]
     L.drm_mirmap2envmap.restype = i32
@@ -123,5 +129,6 @@ EXPORTED_SYMBOLS = ["drm_version", "drm_last_error", "drm_launch_count", "drm_re
                     "drm_render_refmaps_prepared",
                     "drm_render_flat_workspace_bytes", "drm_render_refmaps_flat",
                     "drm_img2refmap_workspace_bytes", "drm_img2refmap", "drm_img2refmap_status", "drm_normals_to_thetaphi",
+                    "drm_img2refmap_dense_workspace_bytes", "drm_img2refmap_dense",
                     "drm_refmap_postprocess", "drm_mirmap2envmap", "drm_refmap_lookup", "drm_normalized_log",
                     "drm_obsnet_condition", "drm_normalized_log_apply"]

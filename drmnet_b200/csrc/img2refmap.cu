@@ -15,6 +15,9 @@
 //   select  i2r_select_small  64 cells per CTA staged in shared memory, element-parallel rank counting
 //           i2r_select_big    warp per cell: cells above 1024 members, NaN-angle members, mean mode
 //
+// The passes that read pixels are templates on a pixel accessor: RowPixels reads the compacted rows of drm_img2refmap,
+// ImagePixels reads dense images under a mask in place (the *_dense instances, drm_img2refmap_dense).
+//
 // HBM-bound integer/compare work by its bytes (24 B per pixel in, 13 B per cell out), no tensor cores; what limits the
 // kernels today is instruction issue (acosf/atan2f and the window tests in pass 0, the rank counting in the select) and
 // the L2 transaction rate of the 8-byte scattered stores in pass 1 -- see DESIGN.md.
@@ -122,6 +125,16 @@ __device__ __forceinline__ uint32_t sum_key(const float* __restrict__ c, int C) 
     return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
 
+// sum_key of the channels c[0], c[cs], ..., c[(C-1)*cs]: the same sum in the same order
+__device__ __forceinline__ uint32_t sum_key_strided(const float* __restrict__ c, int64_t cs, int C) {
+    float s = c[0];
+    for (int k = 1; k < C; ++k) s = __fadd_rn(s, c[k * cs]);
+    if (isnan(s)) return KEY_NAN;
+    s = __fadd_rn(s, 0.0f);
+    uint32_t b = __float_as_uint(s);
+    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+
 // The cells of one axis whose window holds the angle x: centres are (arange + 0.5) * (pi / res) (img2refmap.py:16) and
 // the fp32 predicate |centre - x| <= thr (:27) alone decides membership.  The rounded difference is monotone in the
 // cell index, so the members are one run [lo, hi]: the candidates (+-1 cell for rounding) are trimmed from both ends.
@@ -159,29 +172,94 @@ static constexpr int SEL_CELLS = 64;  // cells per CTA of the select kernel: a p
 static constexpr int PIX_BITS = 26;   // ... above the pixel index, so one call takes up to 2^26 pixels
 static constexpr uint32_t PIX_MASK = (1u << PIX_BITS) - 1u;
 
+// ---- pixel accessors: how the passes reach pixel p's colour, geometry and image.  The pass bodies below are templates
+// on them; the compacted instances are the kernels of drm_img2refmap, the dense ones (*_dense) those of
+// drm_img2refmap_dense.
+//
+// RowPixels: compacted rows -- colors [n, C], normals [n, 3] or thetaphi [n, 2]; image b owns rows offsets[b] ..
+// offsets[b+1]-1 (pass 0 walks forward from block_image, the others search offsets).
+struct RowPixels {
+    __device__ __forceinline__ bool selected(const I2RArgs&, int64_t) const { return true; }
+    __device__ __forceinline__ void load_geom(const I2RArgs& a, int64_t p, float g[3]) const {
+        if (a.is_thetaphi) {
+            const float2 v = reinterpret_cast<const float2*>(a.geom)[p];
+            g[0] = v.x; g[1] = v.y; g[2] = 0.f;
+        } else {
+            g[0] = a.geom[3 * p]; g[1] = a.geom[3 * p + 1]; g[2] = a.geom[3 * p + 2];
+        }
+    }
+    __device__ __forceinline__ void load_rgb(const I2RArgs& a, int64_t p, float c[3]) const {
+        c[0] = a.colors[3 * p]; c[1] = a.colors[3 * p + 1]; c[2] = a.colors[3 * p + 2];
+    }
+    __device__ __forceinline__ void angles(const I2RArgs& a, int64_t p, float& th, float& ph) const { load_angles(a, p, th, ph); }
+    __device__ __forceinline__ uint32_t key(const float* colors, int C, int64_t p) const { return sum_key(colors + p * C, C); }
+    __device__ __forceinline__ float color(const float* colors, int C, int64_t p, int c) const { return colors[p * C + c]; }
+    __device__ __forceinline__ int image_in_block(const I2RArgs& a, unsigned blk, int64_t p) const {
+        int b = a.block_image[blk];
+        while (b + 1 < a.B && a.offsets[b + 1] <= p) ++b;
+        return b;
+    }
+    __device__ __forceinline__ int image(const I2RArgs& a, int64_t p) const { return image_of(a.offsets, a.B, p); }
+    __device__ __forceinline__ int64_t base(const I2RArgs& a, int b) const { return a.offsets[b]; }
+};
+
+// ImagePixels: dense images -- pixel p = (b * H + y) * W + x of B images of H x W, colour channel c at
+// colors[b*cs[0] + y*cs[1] + x*cs[2] + c*cs[3]] and normal component k likewise through ns (element strides, so any
+// [B,H,W,C] or [B,C,H,W] view), included when mask[p] != 0 (mask [B,H,W] contiguous, NULL = every pixel).  The image
+// of p is p / (H*W) and its first pixel b*H*W, so nan_list and sel_index hold the dense image-local index y*W + x.
+// B*H*W <= 2^26, so pixel ids and the divisions are 32-bit.
+struct ImagePixels {
+    const uint8_t* mask;
+    int64_t cs[4], ns[4];
+    uint32_t HW, W;
+    __device__ __forceinline__ int64_t at(const int64_t* s, int64_t p) const {
+        const uint32_t q = (uint32_t)p, b = q / HW, r = q - b * HW, y = r / W, x = r - y * W;
+        return (int64_t)b * s[0] + (int64_t)y * s[1] + (int64_t)x * s[2];
+    }
+    __device__ __forceinline__ bool selected(const I2RArgs&, int64_t p) const { return !mask || mask[p]; }
+    __device__ __forceinline__ void load_geom(const I2RArgs& a, int64_t p, float g[3]) const {
+        const float* n = a.geom + at(ns, p);
+        g[0] = n[0]; g[1] = n[ns[3]]; g[2] = n[2 * ns[3]];
+    }
+    __device__ __forceinline__ void load_rgb(const I2RArgs& a, int64_t p, float c[3]) const {
+        const float* v = a.colors + at(cs, p);
+        c[0] = v[0]; c[1] = v[cs[3]]; c[2] = v[2 * cs[3]];
+    }
+    __device__ __forceinline__ void angles(const I2RArgs& a, int64_t p, float& th, float& ph) const {
+        float g[3];
+        load_geom(a, p, g);
+        normal_to_thetaphi(g[0], g[1], g[2], th, ph);
+    }
+    __device__ __forceinline__ uint32_t key(const float* colors, int C, int64_t p) const {
+        return sum_key_strided(colors + at(cs, p), cs[3], C);
+    }
+    __device__ __forceinline__ float color(const float* colors, int, int64_t p, int c) const {
+        return colors[at(cs, p) + c * cs[3]];
+    }
+    __device__ __forceinline__ int image_in_block(const I2RArgs&, unsigned, int64_t p) const { return (int)((uint32_t)p / HW); }
+    __device__ __forceinline__ int image(const I2RArgs&, int64_t p) const { return (int)((uint32_t)p / HW); }
+    __device__ __forceinline__ int64_t base(const I2RArgs&, int b) const { return (int64_t)b * HW; }
+};
+
 // PASS 0: angles, window, sum key, histogram of the cells.  Each pixel keeps (first cell, key, rank inside that cell) so
 // that pass 1 places it without touching its normal or colour again.  A thread takes HIST_PX pixels (256 apart): all
 // their loads are issued first, and the rank that the histogram atomic returns is only consumed by the stores at the
-// end, so the latency of one pixel's atomic hides behind the arithmetic of the next.
+// end, so the latency of one pixel's atomic hides behind the arithmetic of the next.  A pixel outside the mask keeps
+// CELL_NONE and is not seen again.
 static constexpr int HIST_PX = 2;
-__global__ void __launch_bounds__(256) i2r_hist_pass(I2RArgs a) {
+template <class P>
+__device__ __forceinline__ void hist_pass_body(const I2RArgs& a, const P& px, unsigned tid) {
     int64_t p[HIST_PX];
-    bool in[HIST_PX];
+    bool in[HIST_PX], sel[HIST_PX];
     float g[HIST_PX][3], col[HIST_PX][3];
 #pragma unroll
     for (int u = 0; u < HIST_PX; ++u) {
-        p[u] = ((int64_t)blockIdx.x * HIST_PX + u) * 256 + threadIdx.x;
+        p[u] = ((int64_t)blockIdx.x * HIST_PX + u) * 256 + tid;
         in[u] = p[u] < a.total_n;
         const int64_t pc = in[u] ? p[u] : a.total_n - 1;
-        if (a.is_thetaphi) {
-            const float2 v = reinterpret_cast<const float2*>(a.geom)[pc];
-            g[u][0] = v.x; g[u][1] = v.y; g[u][2] = 0.f;
-        } else {
-            g[u][0] = a.geom[3 * pc]; g[u][1] = a.geom[3 * pc + 1]; g[u][2] = a.geom[3 * pc + 2];
-        }
-        if (a.C == 3) {
-            col[u][0] = a.colors[3 * pc]; col[u][1] = a.colors[3 * pc + 1]; col[u][2] = a.colors[3 * pc + 2];
-        }
+        sel[u] = px.selected(a, pc);
+        px.load_geom(a, pc, g[u]);
+        if (a.C == 3) px.load_rgb(a, pc, col[u]);
     }
     uint32_t cell0[HIST_PX], key[HIST_PX];
     int rank[HIST_PX];
@@ -190,16 +268,19 @@ __global__ void __launch_bounds__(256) i2r_hist_pass(I2RArgs a) {
         cell0[u] = CELL_NONE;
         rank[u] = 0;
         if (!in[u]) continue;
+        if (!sel[u]) {
+            key[u] = 0u;
+            continue;
+        }
         float th, ph;
         if (a.is_thetaphi) { th = g[u][0]; ph = g[u][1]; }
         else normal_to_thetaphi(g[u][0], g[u][1], g[u][2], th, ph);
-        key[u] = a.C == 3 ? sum_key(col[u], 3) : sum_key(a.colors + p[u] * a.C, a.C);
-        int b = a.block_image[blockIdx.x * HIST_PX + u];
-        while (b + 1 < a.B && a.offsets[b + 1] <= p[u]) ++b;
+        key[u] = a.C == 3 ? sum_key(col[u], 3) : px.key(a.colors, a.C, p[u]);
+        const int b = px.image_in_block(a, blockIdx.x * HIST_PX + u, p[u]);
         if (key[u] == KEY_NAN) a.nankey_flag[b] = 1;
         if (isnan(th) || isnan(ph)) {
             // 'NaN > thr' is False (img2refmap.py:27): the pixel is a member of every cell of its image
-            const int64_t base = a.offsets[b];
+            const int64_t base = px.base(a, b);
             const int slot = atomicAdd(&a.nan_count[b], 1);
             a.nan_list[base + slot] = (int32_t)(p[u] - base);
             continue;
@@ -224,6 +305,9 @@ __global__ void __launch_bounds__(256) i2r_hist_pass(I2RArgs a) {
     }
 }
 
+__global__ void __launch_bounds__(256) i2r_hist_pass(I2RArgs a) { hist_pass_body(a, RowPixels{}, threadIdx.x); }
+__global__ void __launch_bounds__(256) i2r_hist_pass_dense(I2RArgs a, ImagePixels px) { hist_pass_body(a, px, threadIdx.x); }
+
 __device__ __forceinline__ void place_pair(const I2RArgs& a, int64_t slot, int cell, uint32_t p, uint32_t key) {
     if (slot < a.pair_capacity) a.pairs[slot] = make_uint2(p | ((uint32_t)(cell % SEL_CELLS) << PIX_BITS), key);
     else atomicOr(a.status, 1);
@@ -232,7 +316,8 @@ __device__ __forceinline__ void place_pair(const I2RArgs& a, int64_t slot, int c
 // PASS 1: place (pixel, key) in the cell segments.  Four pixels per thread: the three record streams are read with
 // 16-byte loads and the four segment-offset gathers are in flight together (the pass is latency-bound otherwise).
 static constexpr int SCATTER_PX = 4;
-__global__ void __launch_bounds__(256) i2r_scatter_pass(I2RArgs a) {
+template <class P>
+__device__ __forceinline__ void scatter_pass_body(const I2RArgs& a, const P& px) {
     const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;  // quad of pixels
     const int64_t p0 = q * SCATTER_PX;
     if (p0 >= a.total_n) return;
@@ -267,9 +352,9 @@ __global__ void __launch_bounds__(256) i2r_scatter_pass(I2RArgs a) {
         if (c0[u] == CELL_NONE || !(c0[u] & CELL_MULTI)) continue;
         // the pixel's other cells: the same window arithmetic as pass 0; they fill the segment behind the first-cell pairs
         const int64_t p = p0 + u;
-        const int b = image_of(a.offsets, a.B, p);
+        const int b = px.image(a, p);
         float th, ph;
-        load_angles(a, p, th, ph);
+        px.angles(a, p, th, ph);
         int i0, i1, j0, j1;
         if (!(axis_cells(a, th, i0, i1) && axis_cells(a, ph, j0, j1))) continue;
         const int img0 = b * a.res2;
@@ -280,6 +365,9 @@ __global__ void __launch_bounds__(256) i2r_scatter_pass(I2RArgs a) {
             }
     }
 }
+
+__global__ void __launch_bounds__(256) i2r_scatter_pass(I2RArgs a) { scatter_pass_body(a, RowPixels{}); }
+__global__ void __launch_bounds__(256) i2r_scatter_pass_dense(I2RArgs a, ImagePixels px) { scatter_pass_body(a, px); }
 
 // ---- exclusive scan of cnt_first + cnt_other: ONE kernel.  Every CTA scans its tile of SCAN_TILE cells; the CTA that
 // finishes last (a ticket counter) scans the tile totals.  The consumers add the two levels (seg_offset).
@@ -347,6 +435,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) i2r_scan_kernel(const int32_t* _
 }
 
 // ---- selection of the lower median under the total order (sum key, pixel index) ----------------------------------
+template <class P>
 struct CellView {
     const uint2* seg;
     int nreg;
@@ -355,19 +444,21 @@ struct CellView {
     int64_t base;             // first pixel of the image
     const float* colors;      // global
     int C;
+    P px;
     __device__ __forceinline__ uint64_t get(int e) const {  // (key << 32) | global pixel index
         if (e < nreg) {
             uint2 pr = seg[e];
             return ((uint64_t)pr.y << 32) | (pr.x & PIX_MASK);
         }
         const int64_t idx = base + nan_list[e - nreg];
-        return ((uint64_t)sum_key(colors + idx * C, C) << 32) | (uint32_t)idx;
+        return ((uint64_t)px.key(colors, C, idx) << 32) | (uint32_t)idx;
     }
 };
 
-__device__ __forceinline__ void write_cell(const I2RArgs& a, int64_t gbin, int64_t base, bool filled, int cnt,
+template <class P>
+__device__ __forceinline__ void write_cell(const I2RArgs& a, const P& px, int64_t gbin, int64_t base, bool filled, int cnt,
                                            int64_t winner) {
-    for (int c = 0; c < a.C; ++c) a.refmap[gbin * a.C + c] = filled ? a.colors[winner * a.C + c] : 0.f;
+    for (int c = 0; c < a.C; ++c) a.refmap[gbin * a.C + c] = filled ? px.color(a.colors, a.C, winner, c) : 0.f;
     a.refmask[gbin] = filled ? 1 : 0;
     if (a.counts) a.counts[gbin] = cnt;
     if (a.sel_index) a.sel_index[gbin] = filled ? (int32_t)(winner - base) : -1;
@@ -398,7 +489,8 @@ __device__ __forceinline__ uint32_t add_if_less(uint32_t rank, uint64_t not_v, u
     return rank;
 }
 static constexpr int CELL_EMPTY = -1, CELL_QUEUED = -2;
-__global__ void __launch_bounds__(SEL_THREADS) i2r_select_small(I2RArgs a, int64_t M) {
+template <class P>
+__device__ __forceinline__ void select_small_body(const I2RArgs& a, const P& px, int64_t M) {
     __shared__ uint64_t buf[SEL_CAP];  // the staged pairs, complemented (see add_if_less)
     __shared__ int s_off[SEL_CELLS + 1];
     __shared__ int s_k[SEL_CELLS];         // median rank of the cell, or CELL_EMPTY / CELL_QUEUED
@@ -468,12 +560,18 @@ __global__ void __launch_bounds__(SEL_THREADS) i2r_select_small(I2RArgs a, int64
     if (tid < ncell) {
         const int k = s_k[tid];
         if (k == CELL_QUEUED) a.big_list[atomicAdd(a.big_count, 1)] = (int32_t)(g0 + tid);
-        else write_cell(a, g0 + tid, a.offsets[b], k >= 0, cnt, k >= 0 ? (int64_t)s_win[tid] : 0);
+        else write_cell(a, px, g0 + tid, px.base(a, b), k >= 0, cnt, k >= 0 ? (int64_t)s_win[tid] : 0);
     }
 }
 
+__global__ void __launch_bounds__(SEL_THREADS) i2r_select_small(I2RArgs a, int64_t M) { select_small_body(a, RowPixels{}, M); }
+__global__ void __launch_bounds__(SEL_THREADS) i2r_select_small_dense(I2RArgs a, ImagePixels px, int64_t M) {
+    select_small_body(a, px, M);
+}
+
 // one warp per queued cell
-__global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) {
+template <class P>
+__device__ __forceinline__ void select_big_body(const I2RArgs& a, const P& px) {
     const int lane = threadIdx.x & 31;
     const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -481,8 +579,8 @@ __global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) {
     for (int64_t q = warp0; q < nbig; q += nwarps) {
         const int64_t gbin = a.big_list[q];
         const int b = (int)(gbin / a.res2);
-        const int64_t base = a.offsets[b];
-        CellView cv;
+        const int64_t base = px.base(a, b);
+        CellView<P> cv;
         cv.nreg = seg_offset(a, (int)gbin + 1) - seg_offset(a, (int)gbin);
         cv.seg = a.pairs + seg_offset(a, (int)gbin);
         cv.nnan = a.nan_count[b];
@@ -490,6 +588,7 @@ __global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) {
         cv.base = base;
         cv.colors = a.colors;
         cv.C = a.C;
+        cv.px = px;
         const int cnt = cv.nreg + cv.nnan;
 
         int64_t winner = -1;
@@ -529,7 +628,7 @@ __global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) {
                         }
                     }
                     for (int d = 16; d; d >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, d));
-                    if (lane < a.C) acc = __fadd_rn(acc, cv.colors[best * a.C + lane]);
+                    if (lane < a.C) acc = __fadd_rn(acc, px.color(cv.colors, a.C, best, lane));
                     prev = best;
                 }
                 mean_c = __fdiv_rn(acc, (float)nvalid);
@@ -537,7 +636,7 @@ __global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) {
         }
         if (lane < a.C) {
             float v = 0.f;
-            if (filled) v = a.reduce_mode == 0 ? cv.colors[winner * a.C + lane] : mean_c;
+            if (filled) v = a.reduce_mode == 0 ? px.color(cv.colors, a.C, winner, lane) : mean_c;
             a.refmap[gbin * a.C + lane] = v;
         }
         if (lane == 0) {
@@ -547,6 +646,9 @@ __global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) {
         }
     }
 }
+
+__global__ void __launch_bounds__(256) i2r_select_big(I2RArgs a) { select_big_body(a, RowPixels{}); }
+__global__ void __launch_bounds__(256) i2r_select_big_dense(I2RArgs a, ImagePixels px) { select_big_body(a, px); }
 
 static int64_t pairs_per_pixel_bound(int res, float thr) {
     const double step = M_PI / res;
@@ -580,6 +682,24 @@ static size_t i2r_carve(I2RArgs& a, void* ws, int64_t total_n, int B, int res, f
     a.pairs = c.take<uint2>(a.pair_capacity > 0 ? a.pair_capacity : 1);
     a.block_image = c.take<int32_t>((npx + 255) / 256 + HIST_PX);
     return c.used();
+}
+
+// the sizes, window constants and outputs that both entries set alike
+static void i2r_set(I2RArgs& a, int B, int C, int res, float thr, int min_points, int reduce_mode, float* refmap,
+                    uint8_t* refmask, int32_t* counts, int32_t* sel_index) {
+    a.B = B; a.C = C; a.res = res; a.res2 = res * res;
+    a.thr = thr;
+    a.stepf = (float)(M_PI / res);  // python float pi/res rounded to fp32 once (img2refmap.py:16)
+    a.inv_step = (float)(res / M_PI);
+    a.R = (int)ceil((double)thr / (M_PI / res)) + 1;
+    if (a.R > res) a.R = res;
+    a.min_points = min_points; a.reduce_mode = reduce_mode;
+    a.refmap = refmap; a.refmask = refmask; a.counts = counts; a.sel_index = sel_index;
+}
+
+// cnt_first, cnt_other, cursor, nan_count, big_count, status are carved first and contiguous (each 256-aligned)
+static cudaError_t i2r_clear(const I2RArgs& a, cudaStream_t st) {
+    return cudaMemsetAsync(a.cnt_first, 0, (size_t)((char*)a.bin_offset - (char*)a.cnt_first), st);
 }
 
 }  // namespace drm
@@ -616,19 +736,9 @@ extern "C" int drm_img2refmap(const float* colors, const float* geom, int input_
         return DRM_EWORKSPACE;
     }
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    a.colors = colors; a.geom = geom; a.offsets = offsets; a.total_n = total_n;
-    a.B = B; a.C = C; a.res = res; a.res2 = res * res; a.is_thetaphi = input_is_thetaphi;
-    a.thr = thr;
-    a.stepf = (float)(M_PI / res);  // python float pi/res rounded to fp32 once (img2refmap.py:16)
-    a.inv_step = (float)(res / M_PI);
-    a.R = (int)ceil((double)thr / (M_PI / res)) + 1;
-    if (a.R > res) a.R = res;
-    a.min_points = min_points; a.reduce_mode = reduce_mode;
-    a.refmap = refmap; a.refmask = refmask; a.counts = counts; a.sel_index = sel_index;
-
-    // cnt_first, cnt_other, cursor, nan_count, big_count, status are carved first and contiguous (each 256-aligned)
-    const size_t zero_bytes = (size_t)((char*)a.bin_offset - (char*)a.cnt_first);
-    DRM_CHECK_CUDA(cudaMemsetAsync(a.cnt_first, 0, zero_bytes, st));
+    a.colors = colors; a.geom = geom; a.offsets = offsets; a.total_n = total_n; a.is_thetaphi = input_is_thetaphi;
+    i2r_set(a, B, C, res, thr, min_points, reduce_mode, refmap, refmask, counts, sel_index);
+    DRM_CHECK_CUDA(i2r_clear(a, st));
     const int64_t nblocks = (M + 1 + SCAN_TILE - 1) / SCAN_TILE;
     if (total_n > 0) {
         const int64_t nblk = (total_n + 255) / 256;
@@ -645,6 +755,71 @@ extern "C" int drm_img2refmap(const float* colors, const float* geom, int input_
     i2r_select_big<<<148 * 4, 256, 0, st>>>(a);
     DRM_CHECK_CUDA(cudaGetLastError());
     count_launches(total_n > 0 ? 6 : 3);
+    return DRM_OK;
+}
+
+// The dense entry runs the passes over all B*H*W pixels, so its workspace is that of drm_img2refmap at total_n = B*H*W
+// (and drm_img2refmap_status reads it with that total_n).
+extern "C" size_t drm_img2refmap_dense_workspace_bytes(int B, int H, int W, int res, float thr) {
+    if (B <= 0 || H <= 0 || W <= 0 || (int64_t)B * H * W > (1ll << PIX_BITS)) return 0;
+    return drm_img2refmap_workspace_bytes((int64_t)B * H * W, B, res, thr);
+}
+
+extern "C" int drm_img2refmap_dense(const float* colors, const int64_t colors_strides[4], const float* normals,
+                                    const int64_t normals_strides[4], const uint8_t* mask, int B, int H, int W, int C,
+                                    int res, float thr, int min_points, int reduce_mode, float* refmap, uint8_t* refmask,
+                                    int32_t* counts, int32_t* sel_index, void* workspace, size_t workspace_bytes,
+                                    void* cuda_stream) {
+    DRM_REQUIRE(colors && colors_strides && normals && normals_strides && refmap && refmask,
+                "img2refmap_dense: null pointer (colors %p, colors_strides %p, normals %p, normals_strides %p, refmap %p, "
+                "refmask %p)", (const void*)colors, (const void*)colors_strides, (const void*)normals,
+                (const void*)normals_strides, (void*)refmap, (void*)refmask);
+    DRM_REQUIRE(B > 0 && H > 0 && W > 0 && res > 0, "img2refmap_dense: B=%d H=%d W=%d res=%d must be positive", B, H, W, res);
+    DRM_REQUIRE(C >= 1 && C <= 4, "img2refmap_dense: C=%d not in 1..4", C);
+    DRM_REQUIRE(thr >= 0.f, "img2refmap_dense: angle threshold %g must be a non-negative number", (double)thr);
+    DRM_REQUIRE(reduce_mode == 0 || reduce_mode == 1, "img2refmap_dense: reduce_mode %d (0 = median, 1 = mean)", reduce_mode);
+    for (int k = 0; k < 4; ++k) {
+        DRM_REQUIRE(colors_strides[k] >= 0, "img2refmap_dense: colors_strides[%d] = %lld is negative", k,
+                    (long long)colors_strides[k]);
+        DRM_REQUIRE(normals_strides[k] >= 0, "img2refmap_dense: normals_strides[%d] = %lld is negative", k,
+                    (long long)normals_strides[k]);
+    }
+    const int64_t total_n = (int64_t)B * H * W, M = (int64_t)B * res * res;
+    DRM_REQUIRE(total_n <= (1ll << PIX_BITS), "img2refmap_dense: B*H*W = %lld pixels in one call, at most 2^26 (split the "
+                "batch)", (long long)total_n);
+    DRM_REQUIRE(M < (1ll << 31), "img2refmap_dense: B*res*res = %lld exceeds int32 cells", (long long)M);
+    const int64_t per_px = pairs_per_pixel_bound(res, thr);
+    if (total_n * per_px >= (1ll << 31)) {
+        set_error("img2refmap_dense: up to %lld (cell,pixel) pairs exceed the int32 segment offsets", (long long)(total_n * per_px));
+        return DRM_EUNSUPPORTED;
+    }
+    I2RArgs a{};
+    const size_t need = i2r_carve(a, workspace, total_n, B, res, thr);
+    if (!workspace || workspace_bytes < need) {
+        set_error("img2refmap_dense: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
+        return DRM_EWORKSPACE;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    a.colors = colors; a.geom = normals; a.offsets = nullptr; a.total_n = total_n; a.is_thetaphi = 0;
+    i2r_set(a, B, C, res, thr, min_points, reduce_mode, refmap, refmask, counts, sel_index);
+    ImagePixels px;
+    px.mask = mask;
+    for (int k = 0; k < 4; ++k) {
+        px.cs[k] = colors_strides[k];
+        px.ns[k] = normals_strides[k];
+    }
+    px.HW = (uint32_t)(H * W);
+    px.W = (uint32_t)W;
+    DRM_CHECK_CUDA(i2r_clear(a, st));
+    const int64_t nblk = (total_n + 255) / 256, nquad = (total_n + SCATTER_PX - 1) / SCATTER_PX;
+    i2r_hist_pass_dense<<<(unsigned)((nblk + HIST_PX - 1) / HIST_PX), 256, 0, st>>>(a, px);
+    i2r_scan_kernel<<<(unsigned)((M + 1 + SCAN_TILE - 1) / SCAN_TILE), SCAN_THREADS, 0, st>>>(
+        a.cnt_first, a.cnt_other, a.bin_offset, a.block_sums, a.scan_ticket, M + 1);
+    i2r_scatter_pass_dense<<<(unsigned)((nquad + 255) / 256), 256, 0, st>>>(a, px);
+    i2r_select_small_dense<<<(unsigned)((M + SEL_CELLS - 1) / SEL_CELLS), SEL_THREADS, 0, st>>>(a, px, M);
+    i2r_select_big_dense<<<148 * 4, 256, 0, st>>>(a, px);
+    DRM_CHECK_CUDA(cudaGetLastError());
+    count_launches(5);
     return DRM_OK;
 }
 

@@ -3,7 +3,8 @@
 ``refmap_mask_make`` (reference utils/img2refmap.py:6-37) bins masked object-image pixels by surface normal into a
 res x res refmap and copies, per cell, the pixel with the lower-median channel sum.  The work is done by
 ``drm_img2refmap`` in libdrmrender.so (hand-written sm_100a kernels, include/drmrender.h); tensors must live on a CUDA
-device -- there is no CPU path.
+device -- there is no CPU path.  ``img2refmap_batch`` scatters a batch of compacted pixel lists, ``img2refmap_images``
+a batch of dense images under a mask (``drm_img2refmap_dense``, read in place).
 """
 from __future__ import annotations
 
@@ -104,6 +105,91 @@ def img2refmap_batch(colors: torch.Tensor, normals: torch.Tensor, offsets: torch
                 raise RuntimeError("img2refmap: the (cell, pixel) pair buffer overflowed; outputs are invalid")
         ws.record_stream(torch.cuda.current_stream(device))
     return refmap, refmask, counts, sel
+
+
+def img2refmap_images(colors: torch.Tensor, normals: torch.Tensor, mask: torch.Tensor | None, res: int,
+                      angle_threshold: float, min_points: int = 0, *, channel_first: bool, reduce: str = "median",
+                      check_status: bool = False):
+    """``img2refmap_batch`` on dense images under a mask, read in place: no compaction, no copy, no host synchronisation.
+
+    colors [B,C,H,W] and normals [B,3,H,W] (``channel_first``) or [B,H,W,C] and [B,H,W,3], fp32, any strides (views
+    such as a channel slice or a permute are read through their strides); mask [B,H,W] bool, or None for every pixel.
+    A single image without the batch dimension is accepted, and its outputs then have none either.  Bit for bit::
+
+        img2refmap_batch(colors_hwc[mask], normals_hwc[mask], [0, cumsum(mask.sum((1, 2)))], res, angle_threshold, ...)
+
+    except ``sel_index``, which holds the dense image-local index y*W + x of the selected pixel (-1 where empty or in
+    mean mode).  Returns (refmap [B,res,res,C], refmask [B,res,res] bool, counts [B,res,res] int32, sel_index).
+    The mask is the caller's: build it with the expression the reference uses (e.g. ``normals.norm(dim=1) > 0.5``).
+    Batches of more than MAX_PIXELS_PER_CALL pixels (B*H*W, masked or not) are split by whole images on the host.
+    ``check_status`` as in ``img2refmap_batch`` (it synchronises).
+    """
+    _require_cuda(colors, "colors")
+    _require_cuda(normals, "normals")
+    if angle_threshold is None:
+        raise TypeError("'>' not supported between instances of 'Tensor' and 'NoneType'")
+    if colors.dtype != torch.float32 or normals.dtype != torch.float32:
+        raise TypeError("colors and normals must be float32")
+    single = colors.dim() == 3
+    if single:
+        colors, normals = colors.unsqueeze(0), normals.unsqueeze(0)
+        if mask is not None:
+            mask = mask.unsqueeze(0)
+    if colors.dim() != 4 or normals.dim() != 4:
+        raise ValueError(f"colors {tuple(colors.shape)} / normals {tuple(normals.shape)}: expected "
+                         f"{'[B,C,H,W] and [B,3,H,W]' if channel_first else '[B,H,W,C] and [B,H,W,3]'}")
+    if channel_first:
+        B, C, H, W = colors.shape
+        dims = (0, 2, 3, 1)  # the (b, y, x, c) strides of a [B,C,H,W] tensor
+    else:
+        B, H, W, C = colors.shape
+        dims = (0, 1, 2, 3)
+    if tuple(normals.shape) != ((B, 3, H, W) if channel_first else (B, H, W, 3)):
+        raise ValueError(f"normals {tuple(normals.shape)} do not match colors {tuple(colors.shape)}")
+    if normals.device != colors.device:
+        raise RuntimeError(f"normals are on {normals.device}, colors on {colors.device}")
+    if mask is not None:
+        _require_cuda(mask, "mask")
+        if mask.dtype != torch.bool:
+            raise TypeError("mask must be bool")
+        if tuple(mask.shape) != (B, H, W) or mask.device != colors.device:
+            raise ValueError(f"mask {tuple(mask.shape)} on {mask.device}: expected [{B},{H},{W}] on {colors.device}")
+    mode = {"median": 0, "mean": 1}[reduce]
+    if B * H * W > MAX_PIXELS_PER_CALL:
+        if H * W > MAX_PIXELS_PER_CALL:
+            raise ValueError(f"one image has {H * W} pixels; one image can hold at most {MAX_PIXELS_PER_CALL}")
+        step = MAX_PIXELS_PER_CALL // (H * W)
+        parts = [img2refmap_images(colors[b:b + step], normals[b:b + step], None if mask is None else mask[b:b + step],
+                                   res, angle_threshold, min_points, channel_first=channel_first, reduce=reduce,
+                                   check_status=check_status) for b in range(0, B, step)]
+        return tuple(torch.cat([p[i] for p in parts]) for i in range(4))
+    device = colors.device
+    L = _lib.lib()
+    cs = (ctypes.c_int64 * 4)(*(colors.stride(d) for d in dims))
+    ns = (ctypes.c_int64 * 4)(*(normals.stride(d) for d in dims))
+    with torch.cuda.device(device):
+        mask_u8 = None if mask is None else mask.contiguous().view(torch.uint8)
+        refmap = torch.empty((B, res, res, C), dtype=torch.float32, device=device)
+        refmask = torch.empty((B, res, res), dtype=torch.bool, device=device)  # the kernels store 0/1 bytes
+        counts = torch.empty((B, res, res), dtype=torch.int32, device=device)
+        sel = torch.empty((B, res, res), dtype=torch.int32, device=device)
+        nbytes = L.drm_img2refmap_dense_workspace_bytes(B, H, W, res, float(angle_threshold))
+        ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=device)
+        _lib.check(L.drm_img2refmap_dense(colors.data_ptr(), cs, normals.data_ptr(), ns,
+                                          None if mask_u8 is None else mask_u8.data_ptr(), B, H, W, C, int(res),
+                                          float(angle_threshold), int(min_points), mode, refmap.data_ptr(),
+                                          refmask.data_ptr(), counts.data_ptr(), sel.data_ptr(), ws.data_ptr(),
+                                          ws.numel(), _stream_ptr(device)))
+        if check_status:
+            st = (ctypes.c_int32 * 2)()
+            _lib.check(L.drm_img2refmap_status(ws.data_ptr(), B * H * W, B, int(res), float(angle_threshold),
+                                               ctypes.byref(st), _stream_ptr(device)))
+            img2refmap_images.last_status = (int(st[0]), int(st[1]))
+            if st[0] & 1:
+                raise RuntimeError("img2refmap: the (cell, pixel) pair buffer overflowed; outputs are invalid")
+        ws.record_stream(torch.cuda.current_stream(device))
+    out = (refmap, refmask, counts, sel)
+    return tuple(o[0] for o in out) if single else out
 
 
 def refmap_mask_make(colors: torch.Tensor, normals: torch.Tensor, res: int, angle_threshold: float = None,

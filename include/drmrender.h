@@ -192,6 +192,21 @@ int drm_render_refmaps_flat(const float* env, int B, int He, int We,
  * drm_img2refmap_status: after a call on the same workspace and arguments, status[0] = flags (bit 0: the pair buffer
  *   overflowed -- cannot happen while workspace_bytes is the value drm_img2refmap_workspace_bytes returns; the outputs
  *   are not to be used if it is set), status[1] = cells that took the warp-per-cell path.  Synchronises the stream.
+ *
+ * drm_img2refmap_dense: the same scatter of B dense images of H x W pixels under a mask, read in place -- no compaction,
+ *   no host read.  Bit for bit the outputs of drm_img2refmap on the compacted pixels (the masked pixels of each image in
+ *   row-major order, offsets = running sums of the mask), except sel_index:
+ *   colors     fp32, channel c of pixel (b, y, x) at colors[b*s[0] + y*s[1] + x*s[2] + c*s[3]], s = colors_strides
+ *              (elements, each >= 0: [B,H,W,C] and [B,C,H,W] views alike), C in 1..4 (device)
+ *   normals    fp32, component k of the normal likewise through normals_strides (device)
+ *   mask       [B, H, W] uint8, contiguous, nonzero = the pixel takes part (device); NULL = every pixel
+ *   sel_index  [B, res, res] int32 dense image-local index y*W + x of the selected pixel, -1 where empty or in mean mode
+ *   The other arguments and outputs are those of drm_img2refmap.  One call takes at most 2^26 pixels counted densely
+ *   (B*H*W, masked or not).  Null pointers, non-positive sizes, C outside 1..4, a negative stride and B*H*W > 2^26 are
+ *   refused (DRM_EINVAL), and a workspace below drm_img2refmap_dense_workspace_bytes (DRM_EWORKSPACE), before any CUDA
+ *   call; drm_last_error names the value.  The workspace is that of drm_img2refmap at total_n = B*H*W, so
+ *   drm_img2refmap_status(workspace, B*H*W, B, res, thr, ...) reads its status words.
+ *   drm_img2refmap_dense_workspace_bytes returns 0 for sizes the entry refuses.
  * ------------------------------------------------------------------------------------------------------------- */
 size_t drm_img2refmap_workspace_bytes(int64_t total_n, int B, int res, float thr);
 
@@ -202,6 +217,15 @@ int drm_img2refmap(const float* colors, const float* normals_or_thetaphi, int in
 
 int drm_img2refmap_status(const void* workspace, int64_t total_n, int B, int res, float thr, int32_t* status /* [2] */,
                           void* cuda_stream);
+
+size_t drm_img2refmap_dense_workspace_bytes(int B, int H, int W, int res, float thr);
+
+int drm_img2refmap_dense(const float* colors, const int64_t colors_strides[4], /* b, y, x, c in elements */
+                         const float* normals, const int64_t normals_strides[4],
+                         const uint8_t* mask /* [B,H,W] contiguous 0/1, NULL = every pixel */,
+                         int B, int H, int W, int C, int res, float thr, int min_points, int reduce_mode,
+                         float* refmap, uint8_t* refmask, int32_t* counts, int32_t* sel_index,
+                         void* workspace, size_t workspace_bytes, void* cuda_stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Callers either side of the render (SURVEY 8f N1, N2).
