@@ -22,7 +22,8 @@ class RenderOptions(ctypes.Structure):
                 ("pixel_covariance", ctypes.c_int), ("full_second_order", ctypes.c_int), ("alpha_full2", ctypes.c_float), ("hand_over", ctypes.c_float), ("limb_nv", ctypes.c_float),
                 ("limb_boost", ctypes.c_float), ("limb_x", ctypes.c_float), ("limb_cells", ctypes.c_float), ("limb_sub", ctypes.c_float), ("limb_hand", ctypes.c_float),
                 ("limb_ramp", ctypes.c_float), ("flat_scale", ctypes.c_float), ("footprint_per_render", ctypes.c_void_p), ("collect_stats", ctypes.c_int),
-                ("horizon_inner", ctypes.c_float), ("horizon_inner_nv", ctypes.c_float), ("horizon_finest", ctypes.c_float)]
+                ("horizon_inner", ctypes.c_float), ("horizon_inner_nv", ctypes.c_float), ("horizon_finest", ctypes.c_float),
+                ("spec_kernels", ctypes.c_int)]
 
 
 def default_render_options() -> "RenderOptions":

@@ -1104,6 +1104,513 @@ __global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass_ker
     tree_spec_pass<P, __half>(g, threadIdx.x);
 }
 
+// ---- specular lobe, pass P: the default instances ------------------------------------------------------------------
+// tree_spec_pass with evaluation loops that issue fewer packed FP32 instructions (eval0, eval1; DESIGN.md 5).
+// Traversal, decisions and staging are those of tree_spec_pass apart from constant factors folded into staged fields
+// (-v.h per texel; 2 m_c, 2 v.mu, 4 v Sigma v, 4 Sigma v per record); the sums are the same, re-rounded.
+// tree_spec_pass stays as it is, selected by DrmRenderOptions::spec_kernels = 1.
+
+template <int P, typename T>
+__device__ __forceinline__ void tree_spec_pass2(const TreeArgs g, int tid) {
+    extern __shared__ __align__(16) unsigned char tree_smem[];
+    const int lane = tid & 31, warp = tid >> 5;
+    int* stack = reinterpret_cast<int*>(tree_smem) + warp * STACK_CAP;
+    float* buf1 = reinterpret_cast<float*>(tree_smem + TREE_WARPS * STACK_CAP * 4) + warp * (BUF1 / 2 * PAIR4 * 4);
+    float4* buf0 = reinterpret_cast<float4*>(tree_smem + TREE_WARPS * STACK_CAP * 4 + TREE_WARPS * (BUF1 / 2) * PAIR4 * 16) + warp * (BUF0 * 2);
+    float* red = reinterpret_cast<float*>(tree_smem);  // reused after the traversal: [256][3]
+
+    constexpr int p = P;
+    const int NG = g.res << p;
+    const int tiles_x = (NG + 15) / 16;
+    const int n_items = g.nact[p] * tiles_x * tiles_x;
+    // barriers of the item loop; under collect_stats they also count the cycles the warp waits in them
+    const bool stats = g.stats;
+    long long t_warp = stats ? clock64() : 0, t_wait = 0;
+    auto tile_sync = [&]() {
+        const long long t = stats ? clock64() : 0;
+        __syncthreads();
+        if (stats) t_wait += clock64() - t;
+    };
+    // persistent CTAs: items = (active render, tile of 16 x 16 lattice nodes), tile-major so that the renders interleave,
+    // handed out by a counter in the order of tile_of (the rim tiles take several times longer than the others)
+    // the item's render record is read from shared memory where it is used: one copy per CTA instead of 34 registers
+    __shared__ int next_item, next_k;
+    __shared__ TreeConst rc;
+    __shared__ WarpUni wu_s[TREE_WARPS];
+    __shared__ int wst_s[TREE_WARPS][6];
+    WarpUni& wu = wu_s[warp];
+    while (true) {
+    if (warp == 0) {
+        int it = 0;
+        if (lane == 0) it = atomicAdd(g.item_ctr, 1);
+        it = __shfl_sync(0xffffffffu, it, 0);
+        if (it < n_items) {
+            const int kk = g.act[p * TREE_CHUNK + it % g.nact[p]];
+            const int* src = reinterpret_cast<const int*>(g.rc + kk);
+            int* dst = reinterpret_cast<int*>(&rc);
+            for (int i = lane; i < (int)(sizeof(TreeConst) / 4); i += 32) dst[i] = src[i];
+            if (lane == 0) next_k = kk;
+        }
+        if (lane == 0) next_item = it;
+    }
+    tile_sync();
+    const int item = next_item;
+    if (item >= n_items) break;
+    const int k = next_k;
+    const int tile = item / g.nact[p];
+    const int pk = rc.pk;
+    int ti, tj;
+    tile_of(tile, tiles_x, ti, tj);
+    const int I0 = ti * 16 + (warp >> 1) * 4, J0 = tj * 16 + (warp & 1) * 8;
+    float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+    const bool pixcov = g.pixcov && p == 0 && pk > 0;  // the 1x1 node of a finer footprint carries the cell's covariance
+
+    NodeT nd;
+    make_node(g, rc, p, pixcov, I0 + (lane >> 3), J0 + (lane & 7), true, nd);
+    float ax, ay, az, beta;
+    const bool live = rc.has_spec && warp_cone(g, p, nd, ax, ay, az, beta);
+
+    if (live) {
+        const float4* pyr = g.pyr_s + (size_t)k * g.gs.cells * REC4;
+        const T* env_b = reinterpret_cast<const T*>(g.env) + (size_t)rc.env * g.He * g.We * 3;
+        // input: the top level of the pyramid (pass 0) or the parent block's hand-over list
+        const int nbJ = (NG + 7) / 8;
+        const int bI = I0 >> 2, bJ = J0 >> 3;
+        const int* in_list = nullptr;  // entries of the current chunk
+        int in_n, in_pos = 0, in_next = -1;
+        if constexpr (p == 0) {
+            in_n = g.gs.H[g.gs.L] * g.gs.W[g.gs.L];
+        } else {
+            const int nbJp = ((g.res << (p - 1)) + 7) / 8;
+            const int nbIp = ((g.res << (p - 1)) + 3) / 4;
+            const size_t pb = (size_t)k * nbIp * nbJp + (size_t)(bI >> 1) * nbJp + (bJ >> 1);
+            in_next = g.heads_in[pb];
+            in_n = 0;
+        }
+        int out_cur = -1, out_fill = 0, out_head = -1;
+        int sp = 0, n1 = 0, n0 = 0;
+        // collect_stats counters [0..3] and the high-water marks of the stack [4] and of the hand-over list [5] in the
+        // warp's shared slot, not in registers through the traversal (lane 0 keeps them)
+        int* st = wst_s[warp];
+        if (lane == 0) st[0] = st[1] = st[2] = st[3] = st[4] = st[5] = 0;
+        // at the limb (n.v -> 0) the lobe sits on the horizon of the normal and the cell average converges later
+        const float nv_min = -warp_max(nd.active ? -nd.nv : -1.f);
+        // ... and n.d = 2 (v.h)(n.h) - n.v moves by the cell's own spread of n.v, so where n.v comes within a few alpha of
+        // zero the view factor and the shadowing ramp G1(n.d) vary across the cell however far the half vector is: blocks
+        // that touch this rim (the outermost cells of the refmap for a sharp lobe) accept nothing that comes near on the
+        // coarse lattices: it all goes down to the render's own lattice.
+        // (a lattice whose sub-cells are narrower than limb_sub * alpha resolves that ramp: no rim rule on it)
+        const float subw = g.cell / (float)(1 << p);
+        const bool limb = nv_min < fmaxf(g.limb_nv, fminf(g.limb_x * sqrtf(rc.alpha2), g.limb_cells * g.cell)) &&
+                          subw * subw > g.limb_sub * g.limb_sub * rc.alpha2;
+        const float thr_p = rc.thr[p] * (limb ? g.limb_boost : 1.f);
+        const float hand_p = limb ? g.limb_hand : g.hand;
+        // the horizon ramp matters most where the lobe itself sits on it: n.v within a few lobe widths of zero
+        const float hz_p = (limb || nv_min < g.hz_nv * sqrtf(rc.alpha2)) ? (p == pk && rc.full2 ? g.hz_fin : g.hz) : g.hz_in;
+        const float xthr = g.limb_ramp * sqrtf(rc.alpha2);
+        const float kappa2 = g.kappa * g.kappa;
+        // wide cells need the second-order terms of G1(n.d) whatever the lobe: without them the cap is half as large
+        const float rcap = rc.full2 ? g.rcap : g.rcap_simple;
+        if (lane == 0) wu = WarpUni{ax, ay, az, beta, thr_p, hand_p, hz_p, xthr, rcap, kappa2, limb};
+        __syncwarp();
+
+        // Staged pairs as in tree_spec_pass, except fields 14-19: 2 m_R, 2 m_B; 20: 2 v.mu; 21: 4 v Sigma v;
+        // 22-24: 4 Sigma v.
+        const f2 NX = F2(nd.nx), NY = F2(nd.ny), NZ = F2(nd.nz), NV = F2(-nd.nv);
+        const f2 Q0 = F2(nd.q0), Q1 = F2(nd.q1), Q2 = F2(nd.q2), Q3 = F2(0.5f * nd.q3), Q4 = F2(0.5f * nd.q4), Q5 = F2(0.5f * nd.q5);
+        const f2 TRP = F2(nd.P0 + nd.P1 + nd.P2);
+        // The loops below evaluate the sums of tree_spec_pass in the same order.  Their cost is the FP32 pipe, where a
+        // packed FFMA2 / FMUL2 / FADD2 takes the cycles of two scalar instructions, so they save packed instructions
+        // and leave the clamps to FMNMX (integer/ALU pipe) and reciprocals and square roots to MUFU:
+        //  * q = 1 + CI sin^2 = 1 + CI u (1 - u/4) as fma(u, fma(u, -CI/4, CI), 1);
+        //  * sq as one sqrt, not arg * rsqrt(arg); the sharp lobe's D G1-ratio as rq^2 xm / (xm + sq);
+        //  * constant factors 2 and 4 folded into staged fields and into 2 a, 2 CI.
+        // The results differ from tree_spec_pass by rounding only.
+        auto eval1 = [&]() {
+            const float ci = rc.inv_a2m1;
+            const f2 CI = F2(ci), CQ = F2(-0.25f * ci), CI2 = F2(2.f * ci), OMA = F2(rc.one_m_a2), A2 = F2(rc.alpha2);
+            if (n1 & 1) {  // pad the last pair with a record of zero weight
+                float* s = buf1 + ((n1 >> 1) * 26) * 2 + 1;
+                if (lane < 26) s[lane * 2] = lane == 3 ? 1.f : 0.f;
+                __syncwarp();
+            }
+            const int np = (n1 + 1) >> 1;
+            f2 cR = F2(0.f), cG = F2(0.f), cB = F2(0.f);
+            const float4* b4 = reinterpret_cast<const float4*>(buf1);
+            if (!rc.full2) {
+                for (int j = 0; j < np; ++j) {
+                    const float4* s = b4 + j * PAIR4;
+                    const float4 v0 = s[0], v1 = s[1];
+                    const f2 ex = sub2(NX, lo(v0)), ey = sub2(NY, hi(v0)), ez = sub2(NZ, lo(v1));
+                    f2 u = fma2(ez, ez, fma2(ey, ey, fma2(ex, ex, hi(v1))));
+                    f2 nmu = fma2(u, F2(-0.5f), F2(1.f));
+                    if (pixcov) {  // the normal's spread over the cell also moves the mean of 2 - 2 n.h: + tr P (n.h)
+                        u = fma2(TRP, nmu, u);
+                        nmu = fma2(u, F2(-0.5f), F2(1.f));
+                    }
+                    const float4 v2 = s[2], v3 = s[3], v4 = s[4];
+                    f2 nSn = mul2(Q0, lo(v2));
+                    nSn = fma2(Q1, hi(v2), nSn); nSn = fma2(Q2, lo(v3), nSn);
+                    nSn = fma2(Q3, hi(v3), nSn); nSn = fma2(Q4, lo(v4), nSn); nSn = fma2(Q5, hi(v4), nSn);
+                    if (pixcov) {
+                        const f2 mx = lo(v0), my = hi(v0), mz = lo(v1);
+                        f2 pp = mul2(mul2(mx, mx), F2(nd.P0));
+                        pp = fma2(mul2(my, my), F2(nd.P1), pp); pp = fma2(mul2(mz, mz), F2(nd.P2), pp);
+                        pp = fma2(mul2(mx, my), F2(nd.P3), pp); pp = fma2(mul2(mx, mz), F2(nd.P4), pp);
+                        pp = fma2(mul2(my, mz), F2(nd.P5), pp);
+                        nSn = add2(nSn, pp);
+                    }
+                    const float4 v5 = s[5];
+                    f2 x = fma2(lo(v5), nmu, NV);
+                    x = max2(x, 0.f);
+                    const f2 q = fma2(u, fma2(u, CQ, CI), F2(1.f));
+                    const f2 xs = add2(x, sqrt2(fma2(mul2(x, x), OMA, A2)));
+                    const f2 rq = rcp2(q);
+                    const f2 Dg = mul2(mul2(rq, rq), mul2(x, rcp2(xs)));
+                    const f2 ciq = mul2(rq, CI2);
+                    const f2 a = mul2(nmu, ciq);                              // 2 a
+                    const f2 K = mul2(Dg, fma2(nSn, fma2(mul2(a, a), F2(3.f), ciq), F2(1.f)));  // Dg (1 + 2 nSn t)
+                    const f2 cn = mul2(Dg, a);
+                    const float4 v6 = s[6], v7 = s[7], v8 = s[8], v9 = s[9];
+                    const f2 nmR = fma2(NZ, lo(v8), fma2(NY, hi(v7), mul2(NX, lo(v7))));
+                    const f2 nmB = fma2(NZ, hi(v9), fma2(NY, lo(v9), mul2(NX, hi(v8))));
+                    cR = fma2(cn, nmR, fma2(K, hi(v5), cR));
+                    cG = fma2(cn, make_float2(-nmR.x - nmB.x, -nmR.y - nmB.y), fma2(K, lo(v6), cG));
+                    cB = fma2(cn, nmB, fma2(K, hi(v6), cB));
+                }
+            } else {
+                for (int j = 0; j < np; ++j) {
+                    const float4* s = b4 + j * PAIR4;
+                    const float4 v0 = s[0], v1 = s[1];
+                    const f2 ex = sub2(NX, lo(v0)), ey = sub2(NY, hi(v0)), ez = sub2(NZ, lo(v1));
+                    f2 u = fma2(ez, ez, fma2(ey, ey, fma2(ex, ex, hi(v1))));
+                    f2 nmu = fma2(u, F2(-0.5f), F2(1.f));
+                    if (pixcov) {  // the normal's spread over the cell also moves the mean of 2 - 2 n.h: + tr P (n.h)
+                        u = fma2(TRP, nmu, u);
+                        nmu = fma2(u, F2(-0.5f), F2(1.f));
+                    }
+                    const float4 v2 = s[2], v3 = s[3], v4 = s[4];
+                    f2 nSn = mul2(Q0, lo(v2));
+                    nSn = fma2(Q1, hi(v2), nSn); nSn = fma2(Q2, lo(v3), nSn);
+                    nSn = fma2(Q3, hi(v3), nSn); nSn = fma2(Q4, lo(v4), nSn); nSn = fma2(Q5, hi(v4), nSn);
+                    f2 pS = nSn;
+                    if (pixcov) {
+                        const f2 mx = lo(v0), my = hi(v0), mz = lo(v1);
+                        f2 pp = mul2(mul2(mx, mx), F2(nd.P0));
+                        pp = fma2(mul2(my, my), F2(nd.P1), pp); pp = fma2(mul2(mz, mz), F2(nd.P2), pp);
+                        pp = fma2(mul2(mx, my), F2(nd.P3), pp); pp = fma2(mul2(mx, mz), F2(nd.P4), pp);
+                        pp = fma2(mul2(my, mz), F2(nd.P5), pp);
+                        pS = add2(nSn, pp);
+                    }
+                    const float4 v10 = s[10], v11 = s[11], v12 = s[12];
+                    const f2 vmu = lo(v10), vSv = hi(v10);                   // 2 v.mu, 4 v Sigma v
+                    const f2 nSv = fma2(NZ, lo(v12), fma2(NY, hi(v11), mul2(NX, lo(v11))));  // 4 n Sigma v
+                    // mean and variance of n.d over the cell; the clamp at the horizon acts on that distribution
+                    f2 x = fma2(vmu, nmu, fma2(nSv, F2(0.5f), NV));
+                    const f2 vn = mul2(vmu, nSn);
+                    f2 varx = mul2(mul2(nmu, nmu), vSv);
+                    varx = fma2(mul2(nmu, vmu), nSv, varx);
+                    varx = max2(fma2(vmu, vn, varx), 0.f);                   // 4 var(n.d)
+                    const f2 w = sqrt2(mul2(varx, F2(3.f)));
+                    const bool st0 = x.x < w.x, st1 = x.y < w.y;
+                    const f2 xe = max2(add2(x, w), 0.f);
+                    const f2 xs2 = mul2(mul2(xe, xe), rcp2(max2(mul2(w, F2(4.f)), 1e-30f)));
+                    x.x = st0 ? xs2.x : x.x;
+                    x.y = st1 ? xs2.y : x.y;
+                    const f2 xm = max2(x, 0.f);
+                    const f2 q = fma2(u, fma2(u, CQ, CI), F2(1.f));
+                    const f2 rq = rcp2(q);
+                    const f2 D = mul2(rq, rq);
+                    const f2 arg = fma2(mul2(xm, xm), OMA, A2);
+                    const f2 rsq = rsqrt2(arg);
+                    const f2 sq = mul2(arg, rsq);
+                    const f2 rxs = rcp2(add2(xm, sq));
+                    const f2 ciq = mul2(rq, CI2);                             // 2 CI rq
+                    const f2 a = mul2(nmu, ciq);                              // 2 a
+                    const f2 Dg = mul2(D, mul2(xm, rxs));
+                    f2 K = mul2(Dg, fma2(pS, fma2(mul2(a, a), F2(3.f), ciq), F2(1.f)));
+                    const f2 gx = mul2(mul2(A2, rsq), mul2(rxs, rxs));
+                    const f2 spx = mul2(mul2(xm, OMA), rsq);
+                    const f2 gxx = mul2(gx, fma2(spx, rsq, mul2(mul2(add2(spx, F2(1.f)), F2(2.f)), rxs)));  // = -g_xx
+                    const f2 T2 = mul2(mul2(mul2(D, a), gx), fma2(vn, F2(2.f), mul2(nmu, nSv)));
+                    f2 T3 = mul2(mul2(D, gxx), mul2(varx, F2(-0.5f)));
+                    T3.x = st0 ? 0.f : T3.x;
+                    T3.y = st1 ? 0.f : T3.y;
+                    K = add2(K, add2(T2, T3));
+                    const f2 cn = mul2(Dg, a);
+                    const float4 v5 = s[5], v6 = s[6], v7 = s[7], v8 = s[8], v9 = s[9];
+                    const f2 nmR = fma2(NZ, lo(v8), fma2(NY, hi(v7), mul2(NX, lo(v7))));
+                    const f2 nmB = fma2(NZ, hi(v9), fma2(NY, lo(v9), mul2(NX, hi(v8))));
+                    cR = fma2(cn, nmR, fma2(K, hi(v5), cR));
+                    cG = fma2(cn, make_float2(-nmR.x - nmB.x, -nmR.y - nmB.y), fma2(K, lo(v6), cG));
+                    cB = fma2(cn, nmB, fma2(K, hi(v6), cB));
+                }
+            }
+            a0 += nd.mult * (cR.x + cR.y);
+            a1 += nd.mult * (cG.x + cG.y);
+            a2 += nd.mult * (cB.x + cB.y);
+            n1 = 0;
+        };
+        // Staged texels, two per float4 pair like the records: texels 2j, 2j+1 sit at buf0[4 j .. 4 j + 3] as
+        // (hx0,hx1,hy0,hy1) (hz0,hz1,2vh0,2vh1) (wR0,wR1,wG0,wG1) (wB0,wB1,-vh0,-vh1); -v.h turns n.d into one FMA.
+        // The loop takes four texels (two pairs A, B) an iteration.
+        const f2 NVp = F2(nd.nv);
+        auto eval0 = [&]() {
+            const float ci = rc.inv_a2m1;
+            const f2 CI = F2(ci), CQ = F2(-0.25f * ci), OMA = F2(rc.one_m_a2), A2 = F2(rc.alpha2);
+            if (n0 & 3) {  // pad to whole quads with texels of zero weight at the node itself
+                const int slot = n0 + (lane >> 3), f = lane & 7;
+                if (slot < ((n0 + 3) & ~3)) {
+                    float* s = reinterpret_cast<float*>(buf0 + (slot >> 1) * 4) + (slot & 1);
+                    s[f * 2] = f == 0 ? nd.nx : f == 1 ? nd.ny : f == 2 ? nd.nz : 0.f;
+                }
+                __syncwarp();
+            }
+            const int nq = (n0 + 3) >> 2;
+            f2 bR = F2(0.f), bG = F2(0.f), bB = F2(0.f);
+            for (int j = 0; j < nq; ++j) {
+                const float4* s = buf0 + 8 * j;
+                const float4 v0 = s[0], v1 = s[1], v3 = s[3];
+                f2 ex = sub2(NX, lo(v0)), ey = sub2(NY, hi(v0)), ez = sub2(NZ, lo(v1));
+                const f2 uA = fma2(ez, ez, fma2(ey, ey, mul2(ex, ex)));   // 2 (1 - n.h), no cancellation
+                f2 xA = sub2(fma2(uA, hi(v3), hi(v1)), NVp);               // n.d = |v+d| (1 - u/2) - n.v
+                xA = max2(xA, 0.f);
+                const f2 qA = fma2(uA, fma2(uA, CQ, CI), F2(1.f));
+                const f2 dA = mul2(mul2(qA, qA), add2(xA, sqrt2(fma2(mul2(xA, xA), OMA, A2))));
+                const float4 w0 = s[4], w1 = s[5], w3 = s[7];
+                ex = sub2(NX, lo(w0)); ey = sub2(NY, hi(w0)); ez = sub2(NZ, lo(w1));
+                const f2 uB = fma2(ez, ez, fma2(ey, ey, mul2(ex, ex)));
+                f2 xB = sub2(fma2(uB, hi(w3), hi(w1)), NVp);
+                xB = max2(xB, 0.f);
+                const f2 qB = fma2(uB, fma2(uB, CQ, CI), F2(1.f));
+                const f2 dB = mul2(mul2(qB, qB), add2(xB, sqrt2(fma2(mul2(xB, xB), OMA, A2))));
+                const f2 wsA = mul2(xA, rcp2(dA)), wsB = mul2(xB, rcp2(dB));
+                const float4 v2 = s[2], w2 = s[6];
+                bR = fma2(wsA, lo(v2), bR); bG = fma2(wsA, hi(v2), bG); bB = fma2(wsA, lo(v3), bB);
+                bR = fma2(wsB, lo(w2), bR); bG = fma2(wsB, hi(w2), bG); bB = fma2(wsB, lo(w3), bB);
+            }
+            a0 += nd.mult * (bR.x + bR.y); a1 += nd.mult * (bG.x + bG.y); a2 += nd.mult * (bB.x + bB.y);
+            n0 = 0;
+        };
+
+        bool done = false;
+        while (true) {
+            unsigned ent = 0;
+            int ntake;
+            if (sp > 0) {
+                ntake = min(32, sp);
+                if (lane < ntake) ent = (unsigned)stack[sp - 1 - lane];
+                sp -= ntake;
+            } else {
+                if (p > 0 && in_pos >= in_n && in_next >= 0) {  // next chunk of the parent's list
+                    const int* ch = g.pool_in + (size_t)in_next * CHUNK;
+                    in_next = ch[0];
+                    in_n = ch[1];
+                    in_list = ch + 2;
+                    in_pos = 0;
+                }
+                if (in_pos < in_n) {
+                    ntake = min(32, in_n - in_pos);
+                    if (lane < ntake) ent = p == 0 ? (((unsigned)g.gs.L << 28) | (unsigned)(in_pos + lane)) : (unsigned)in_list[in_pos + lane];
+                    in_pos += ntake;
+                } else {
+                    ntake = 0;
+                    done = true;  // one more turn of the loop flushes the staged records
+                }
+            }
+            const bool has = lane < ntake;
+            if (stats && lane == 0) { st[0] += ntake; st[1] += 1; }
+            __syncwarp();
+            // ---- decide ----
+            int act = ACT_DROP;
+            const int lev = (int)(ent >> 28), id = (int)(ent & 0x0fffffffu);
+            float h[3], vh = 0.f, w3[3];
+            if (has) {
+                float mx, my, mz, rha, wsum, vmu, im;
+                if (lev > 0) {
+                    // the verdict needs the mean, radius and energy; staging reads the rest of the record again
+                    const float4* rp = pyr + (g.gs.off[lev] + id) * REC4;
+                    const float4 r0 = rp[0], r2 = rp[2], r3 = rp[3];
+                    mx = r0.x; my = r0.y; mz = r0.z;
+                    wsum = r2.z + r2.w + r3.x;
+                    const float m2 = fmaxf(mx * mx + my * my + mz * mz, 1e-30f);
+                    im = fast_rsqrt(m2);
+                    rha = fast_radius_angle(r0.w + fmaxf(1.f - m2 * im, 0.f));
+                    vmu = rc.vhat[0] * mx + rc.vhat[1] * my + rc.vhat[2] * mz;
+                } else {
+                    const int r = id / g.We, c = id - r * g.We;
+                    texel_spec(g, rc, env_b, r, c, h, vh, w3);
+                    mx = h[0]; my = h[1]; mz = h[2];
+                    wsum = w3[0] + w3[1] + w3[2];
+                    im = 1.f; rha = 0.f; vmu = vh;
+                }
+                if (wsum > 0.f) {
+                    const float ax = wu.ax, ay = wu.ay, az = wu.az, beta = wu.beta;
+                    const float hx = mx * im - ax, hy = my * im - ay, hz = mz * im - az;
+                    const float ang = fast_chord_angle(hx * hx + hy * hy + hz * hz);
+                    const float dmin = fmaxf(ang - beta - rha, 0.f);
+                    // direction of the cell d = 2 (v.h) h - v and its angular radius <= 2 rha: visibility, horizon
+                    const float t2 = 2.f * vmu * im * im;
+                    const float adc = ax * (t2 * mx - rc.vhat[0]) + ay * (t2 * my - rc.vhat[1]) + az * (t2 * mz - rc.vhat[2]);
+                    const float spread = beta + 2.f * rha + 1e-3f;
+                    const float ss = __sinf(fminf(spread, 1.5607f));
+                    if (spread < 1.5607f && adc <= -ss) act = ACT_DROP;
+                    // near for this lattice: small cells go to the child blocks, large ones are refined here so that
+                    // their far parts stay on this lattice
+                    else if (p < pk && dmin < wu.thr_p) act = (lev == 0 || rha <= wu.hand_p * wu.thr_p) ? ACT_HAND : ACT_REFINE;
+                    // rim blocks: what lies within the shadowing ramp of their horizon goes down as well, in pieces of
+                    // at most 0.05 rad
+                    else if (p < pk && wu.limb && spread < 1.5607f &&
+                             adc * __cosf(spread) - sqrtf(fmaxf(1.f - adc * adc, 0.f)) * ss < wu.xthr)
+                        act = (lev == 0 || rha <= 0.05f) ? ACT_HAND : ACT_REFINE;
+                    else if (lev > 0 && (rha > wu.rcap || rha * rha > wu.kappa2 * (rc.alpha2 + dmin * dmin) ||
+                                         (2.f * rha > wu.hz_p && fabsf(adc) < ss))) act = ACT_REFINE;
+                    else act = ACT_ACCEPT;
+                }
+            }
+            // ---- hand over to the child blocks of the next pass ----
+            {
+                const unsigned mh = __ballot_sync(0xffffffffu, act == ACT_HAND);
+                if (mh) {
+                    const int cnt = __popc(mh);
+                    if (out_cur < 0 || out_fill + cnt > CHUNK - 2) {  // close the current chunk, take a new one from the pool
+                        int nc = 0;
+                        if (lane == 0) nc = atomicAdd(g.pool_ctr, 1);
+                        nc = __shfl_sync(0xffffffffu, nc, 0);
+                        if (nc >= g.pool_cap) {
+                            if (lane == 0) atomicOr(g.status, 1);  // pool exhausted: the result is incomplete
+                            nc = -1;
+                        }
+                        if (lane == 0) {
+                            if (out_cur >= 0) {
+                                g.pool_out[(size_t)out_cur * CHUNK] = nc;
+                                g.pool_out[(size_t)out_cur * CHUNK + 1] = out_fill;
+                            }
+                        }
+                        if (out_cur < 0) out_head = nc;
+                        out_cur = nc;
+                        out_fill = 0;
+                    }
+                    if (act == ACT_HAND && out_cur >= 0)
+                        g.pool_out[(size_t)out_cur * CHUNK + 2 + out_fill + __popc(mh & ((1u << lane) - 1u))] = (int)ent;
+                    if (out_cur >= 0) out_fill += cnt;
+                    if (lane == 0) st[5] += cnt;
+                }
+            }
+            // ---- refine: children onto the stack ----
+            {
+                int nch = 0, cr = 0, cc = 0, Wc = 0;
+                if (act == ACT_REFINE) {
+                    const int Wl = g.gs.W[lev];
+                    const int r = id / Wl, c = id - r * Wl;
+                    Wc = lev == 1 ? g.We : g.gs.W[lev - 1];
+                    const int Hc = lev == 1 ? g.He : g.gs.H[lev - 1];
+                    cr = 2 * r; cc = 2 * c;
+                    nch = (cr + 1 < Hc ? 2 : 1) * (cc + 1 < Wc ? 2 : 1);
+                }
+                int inc = nch;
+                for (int d = 1; d < 32; d <<= 1) {
+                    const int t = __shfl_up_sync(0xffffffffu, inc, d);
+                    if (lane >= d) inc += t;
+                }
+                const int total = __shfl_sync(0xffffffffu, inc, 31);
+                if (total) {
+                    if (sp + total > STACK_CAP) {
+                        atomicOr(g.status, 4);  // traversal stack full
+                    } else if (nch) {
+                        int pos = sp + inc - nch;
+                        const int two_c = (nch == 4) || (nch == 2 && cc + 1 < Wc);
+                        const int two_r = (nch == 4) || (nch == 2 && !two_c);
+                        const int tag = (int)((unsigned)(lev - 1) << 28);
+                        stack[pos++] = tag | (cr * Wc + cc);
+                        if (two_c) stack[pos++] = tag | (cr * Wc + cc + 1);
+                        if (two_r) stack[pos++] = tag | ((cr + 1) * Wc + cc);
+                        if (two_r && two_c) stack[pos++] = tag | ((cr + 1) * Wc + cc + 1);
+                    }
+                    if (sp + total <= STACK_CAP) sp += total;
+                    if (lane == 0) st[4] = max(st[4], sp);
+                }
+            }
+            // ---- accept: stage the record for the evaluation ----
+            {
+                const unsigned m1 = __ballot_sync(0xffffffffu, act == ACT_ACCEPT && lev > 0);
+                const unsigned m0 = __ballot_sync(0xffffffffu, act == ACT_ACCEPT && lev == 0);
+                if (done || n1 + __popc(m1) > BUF1) { __syncwarp(); eval1(); __syncwarp(); }
+                if (done || n0 + __popc(m0) > BUF0) { __syncwarp(); eval0(); __syncwarp(); }
+                if (done) break;
+                if (act == ACT_ACCEPT) {
+                    if (lev > 0) {
+                        const int slot = n1 + __popc(m1 & ((1u << lane) - 1u));
+                        float* s = buf1 + ((slot >> 1) * 26) * 2 + (slot & 1);
+                        const float4* rp = pyr + (g.gs.off[lev] + id) * REC4;
+                        const float4 r0 = rp[0], r1 = rp[1], r2 = rp[2], r3 = rp[3], r4 = rp[4];
+                        const float Sxx = r1.x, Syy = r1.y, Szz = r1.z, Sxy = r1.w, Sxz = r2.x, Syz = r2.y;
+                        const float vx = rc.vhat[0], vy = rc.vhat[1], vz = rc.vhat[2];
+                        const float vmu = vx * r0.x + vy * r0.y + vz * r0.z;
+                        const float trS = Sxx + Syy + Szz;
+                        const float svx = Sxx * vx + Sxy * vy + Sxz * vz, svy = Sxy * vx + Syy * vy + Syz * vz,
+                                    svz = Sxz * vx + Syz * vy + Szz * vz;
+                        s[0] = r0.x; s[2] = r0.y; s[4] = r0.z; s[6] = trS;
+                        s[8] = Sxx; s[10] = Syy; s[12] = Szz; s[14] = 2.f * Sxy; s[16] = 2.f * Sxz; s[18] = 2.f * Syz;
+                        s[20] = 2.f * vmu / fmaxf(1.f - trS, 1e-12f);
+                        s[22] = r2.z; s[24] = r2.w; s[26] = r3.x;
+                        s[28] = 2.f * r3.y; s[30] = 2.f * r3.z; s[32] = 2.f * r3.w;
+                        s[34] = 2.f * r4.x; s[36] = 2.f * r4.y; s[38] = 2.f * r4.z;
+                        s[40] = 2.f * vmu; s[42] = 4.f * (vx * svx + vy * svy + vz * svz);
+                        s[44] = 4.f * svx; s[46] = 4.f * svy; s[48] = 4.f * svz; s[50] = 0.f;
+                    } else {
+                        const int slot = n0 + __popc(m0 & ((1u << lane) - 1u));
+                        float* s = reinterpret_cast<float*>(buf0 + (slot >> 1) * 4) + (slot & 1);
+                        s[0] = h[0]; s[2] = h[1]; s[4] = h[2]; s[6] = 2.f * vh;
+                        s[8] = w3[0]; s[10] = w3[1]; s[12] = w3[2]; s[14] = -vh;
+                    }
+                }
+                n1 += __popc(m1);
+                n0 += __popc(m0);
+                if (stats && lane == 0) { st[2] += __popc(m0); st[3] += __popc(m1); }
+            }
+            __syncwarp();
+        }
+        if (p < pk && lane == 0) {
+            const int nbI = (NG + 3) / 4;
+            if (out_cur >= 0) {
+                g.pool_out[(size_t)out_cur * CHUNK] = -1;
+                g.pool_out[(size_t)out_cur * CHUNK + 1] = out_fill;
+            }
+            g.heads_out[(size_t)k * nbI * nbJ + (size_t)bI * nbJ + bJ] = out_head;
+        }
+        if (lane == 0 && g.stats) {
+            atomicAdd(g.status + 16 + 4 * p, st[0]); atomicAdd(g.status + 17 + 4 * p, st[1]);
+            atomicAdd(g.status + 18 + 4 * p, st[2]); atomicAdd(g.status + 19 + 4 * p, st[3]);
+        }
+        if (lane == 0) {  // high-water marks (drm_render_status)
+            if (st[4] > g.status[1]) atomicMax(g.status + 1, st[4]);
+            if (st[5] > g.status[2 + p]) atomicMax(g.status + 2 + p, st[5]);
+        }
+    } else if (p < pk && lane == 0) {
+        const int nbJ = (NG + 7) / 8, nbI = (NG + 3) / 4;
+        const int bI = I0 >> 2, bJ = J0 >> 3;
+        if (bI < nbI && bJ < nbJ) g.heads_out[(size_t)k * nbI * nbJ + (size_t)bI * nbJ + bJ] = -1;
+    }
+    tile_sync();  // stacks and buffers are dead: the reduction reuses the memory
+    tile_writeback(g, p, red, k, ti, tj, a0, a1, a2, false);
+    tile_sync();  // ... and the next item's traversal reuses it again
+    }
+    if (stats && lane == 0) {
+        atomicAdd(g.status + STAT_TILE_WAIT + p, (int)(t_wait >> 10));
+        atomicAdd(g.status + STAT_WARP_CYCLES + p, (int)((clock64() - t_warp) >> 10));
+    }
+}
+
+template <int P>
+__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass2_kernel(const TreeArgs g) {
+    tree_spec_pass2<P, float>(g, threadIdx.x);
+}
+template <int P>
+__global__ void __launch_bounds__(TREE_THREADS, SPEC_MINB[P]) tree_spec_pass2_kernel_h(const TreeArgs g) {
+    tree_spec_pass2<P, __half>(g, threadIdx.x);
+}
+
 // ---- diffuse lobe: one pass, writes `out`.  1x1 lattice whose node carries the covariance of the refmap cell (fourth
 // order in the cell size: cells up to 0.03 rad), or the render's own lattice for coarser refmaps ------------------------
 template <typename T>
@@ -1434,11 +1941,13 @@ static constexpr int MAX_DEVICES = 64;
 template <typename T> struct TexelKernels;
 template <> struct TexelKernels<float> {
     template <int P> static constexpr void (*spec)(TreeArgs) = tree_spec_pass_kernel<P>;
+    template <int P> static constexpr void (*spec2)(TreeArgs) = tree_spec_pass2_kernel<P>;
     static constexpr void (*diff)(TreeArgs) = tree_diff_kernel;
     template <bool SPEC> static constexpr void (*pyr)(TreeArgs, int, float4*) = pyr_from_texels_kernel<SPEC>;
 };
 template <> struct TexelKernels<__half> {
     template <int P> static constexpr void (*spec)(TreeArgs) = tree_spec_pass_kernel_h<P>;
+    template <int P> static constexpr void (*spec2)(TreeArgs) = tree_spec_pass2_kernel_h<P>;
     static constexpr void (*diff)(TreeArgs) = tree_diff_kernel_h;
     template <bool SPEC> static constexpr void (*pyr)(TreeArgs, int, float4*) = pyr_from_texels_kernel_h<SPEC>;
 };
@@ -1463,11 +1972,11 @@ static int launch_diffuse_pyramids(const TreeArgs& g, int B, float4* pyr, cudaSt
 }
 
 // Pass P on a persistent grid of (SMs x resident CTAs of this instance), at most one CTA per item.  The grid size is
-// queried once per device and instance (fp32 and fp16 instances have their own slots).
-template <int P, typename T>
+// queried once per device and instance (fp32 and fp16, default and pinned instances have their own slots).
+template <int P, typename T, bool PINNED>
 static cudaError_t launch_spec_pass(const TreeArgs& a, long items, cudaStream_t st) {
     static int resident[MAX_DEVICES];
-    void (*kernel)(TreeArgs) = TexelKernels<T>::template spec<P>;
+    void (*kernel)(TreeArgs) = PINNED ? TexelKernels<T>::template spec<P> : TexelKernels<T>::template spec2<P>;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_SMEM);
     if (e == cudaSuccess)
         e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -1590,6 +2099,8 @@ static int render_refmaps(const T* env, int B, int He, int We, const int32_t* en
         return DRM_EWORKSPACE;
     }
     if (!(alpha_min > 0.f)) alpha_min = fmaxf(1e-3f, (float)(1.25 * M_PI / He));
+    DRM_REQUIRE(o.spec_kernels == 0 || o.spec_kernels == 1, "render: spec_kernels=%d must be 0 or 1", o.spec_kernels);
+    const bool pinned = o.spec_kernels == 1;
 
     TreeArgs g;
     memset(&g, 0, sizeof(g));
@@ -1665,12 +2176,22 @@ static int render_refmaps(const T* env, int B, int He, int We, const int32_t* en
             const long items = (long)((NG + 15) / 16) * ((NG + 15) / 16) * n;  // upper bound: the active renders are fewer
             a.item_ctr = L.status + 44 + p;
             DRM_CHECK_CUDA(cudaMemsetAsync(a.item_ctr, 0, sizeof(int), st));
-            switch (p) {
-                case 0: DRM_CHECK_CUDA((launch_spec_pass<0, T>(a, items, st))); break;
-                case 1: DRM_CHECK_CUDA((launch_spec_pass<1, T>(a, items, st))); break;
-                case 2: DRM_CHECK_CUDA((launch_spec_pass<2, T>(a, items, st))); break;
-                case 3: DRM_CHECK_CUDA((launch_spec_pass<3, T>(a, items, st))); break;
-                default: DRM_CHECK_CUDA((launch_spec_pass<4, T>(a, items, st))); break;
+            if (pinned) {
+                switch (p) {
+                    case 0: DRM_CHECK_CUDA((launch_spec_pass<0, T, true>(a, items, st))); break;
+                    case 1: DRM_CHECK_CUDA((launch_spec_pass<1, T, true>(a, items, st))); break;
+                    case 2: DRM_CHECK_CUDA((launch_spec_pass<2, T, true>(a, items, st))); break;
+                    case 3: DRM_CHECK_CUDA((launch_spec_pass<3, T, true>(a, items, st))); break;
+                    default: DRM_CHECK_CUDA((launch_spec_pass<4, T, true>(a, items, st))); break;
+                }
+            } else {
+                switch (p) {
+                    case 0: DRM_CHECK_CUDA((launch_spec_pass<0, T, false>(a, items, st))); break;
+                    case 1: DRM_CHECK_CUDA((launch_spec_pass<1, T, false>(a, items, st))); break;
+                    case 2: DRM_CHECK_CUDA((launch_spec_pass<2, T, false>(a, items, st))); break;
+                    case 3: DRM_CHECK_CUDA((launch_spec_pass<3, T, false>(a, items, st))); break;
+                    default: DRM_CHECK_CUDA((launch_spec_pass<4, T, false>(a, items, st))); break;
+                }
             }
             count_launches(1);
         }
@@ -1744,4 +2265,5 @@ extern "C" void drm_render_default_options(DrmRenderOptions* o) {
     o->limb_cells = 1.3f;
     o->limb_hand = 32.f;
     o->limb_ramp = 0.f;
+    o->spec_kernels = 0;
 }

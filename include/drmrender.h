@@ -103,6 +103,8 @@ typedef struct DrmRenderOptions {
     float horizon_finest;   /* the horizon width near the limb on the render's own lattice (its nodes are the exact normals)
                                for the lobes that carry the per-cell horizon clamp (alpha >= alpha_full2); same scaling
                                with the cell size */
+    int spec_kernels;       /* 0 (default): the specular lattice passes with the shorter evaluation loops; 1: the earlier
+                               pass kernels (tree_spec_pass_kernel<P>), whose results differ by rounding only */
 } DrmRenderOptions;
 
 void drm_render_default_options(DrmRenderOptions* opts);

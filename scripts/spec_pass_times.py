@@ -70,7 +70,7 @@ def main():
             p = None
             if name.startswith("tree_diff_kernel"):
                 pass_idx = -1
-            elif name.startswith("tree_spec_pass_kernel"):
+            elif re.match(r"tree_spec_pass2?_kernel", name):
                 pass_idx += 1
                 m = re.search(r"<(\d+)>", name)
                 p = int(m.group(1)) if m else pass_idx
