@@ -104,6 +104,8 @@ def lib() -> ctypes.CDLL:
     L.drm_mirmap2envmap.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.drm_refmap_lookup.restype = i32
     L.drm_refmap_lookup.argtypes = [vp, vp, vp, i64, i32, i32, i32, i32, vp, vp]
+    L.drm_refmap_lookup_dense.restype = i32
+    L.drm_refmap_lookup_dense.argtypes = [vp, i32, i32, vp, i64p, vp, i32, i32, i32, i32, vp, i64p, vp]
     L.drm_normalized_log.restype = i32
     L.drm_normalized_log.argtypes = [vp, vp, i32, i32, i32, i32, f32, vp, vp, vp, vp]
     L.drm_obsnet_condition.restype = i32
@@ -131,5 +133,6 @@ EXPORTED_SYMBOLS = ["drm_version", "drm_last_error", "drm_launch_count", "drm_re
                     "drm_render_flat_workspace_bytes", "drm_render_refmaps_flat",
                     "drm_img2refmap_workspace_bytes", "drm_img2refmap", "drm_img2refmap_status", "drm_normals_to_thetaphi",
                     "drm_img2refmap_dense_workspace_bytes", "drm_img2refmap_dense",
-                    "drm_refmap_postprocess", "drm_mirmap2envmap", "drm_refmap_lookup", "drm_normalized_log",
+                    "drm_refmap_postprocess", "drm_mirmap2envmap", "drm_refmap_lookup", "drm_refmap_lookup_dense",
+                    "drm_normalized_log",
                     "drm_obsnet_condition", "drm_normalized_log_apply"]

@@ -6,15 +6,20 @@ step instead of one synchronous render per (sample, BRDF vector).
                             :610-620; dataset/basedataset.py:52-53), NaN-sentinel protocol included
 * ``refmap_postprocess`` <- models/drmnet.py:610-620 alone
 * ``mirmap2envmap`` / ``r0toenvmap`` <- utils/transform.py:106-144 / DRMNet.r0toenvmap (models/drmnet.py:931-941)
+* ``obsnet_inputs``      <- the render + object image + scatter + conditioning part of ObsNetDiffusion.get_input
+                            (models/obsnet.py:139-413), the object image shaded by ``refmap_lookup_images``
 """
 from __future__ import annotations
 
+import ctypes
+import math
 from typing import List, Optional, Sequence, Tuple
 
 import torch
 
 from . import _lib
-from .renderer import B200RefMapRenderer, _env_dtype, _slots, render_batch
+from .img2refmap import img2refmap_images
+from .renderer import B200RefMapRenderer, EnvmapBank, _env_dtype, _slots, render_batch
 
 
 def _stream(device) -> int:
@@ -23,27 +28,36 @@ def _stream(device) -> int:
 
 def rendering_refmaps(renderer: B200RefMapRenderer, envmaps, z: torch.Tensor,
                       brdf_param_names: Optional[Sequence[str]] = None, view_from=None,
-                      new_scene: bool = False) -> torch.Tensor:
+                      new_scene: bool = False, env_ids: Optional[torch.Tensor] = None) -> torch.Tensor:
     """envmaps [B,He,We,3] (a tensor, or a list of [He,We,3] tensors), z [L,B,P] -> [L,B,3,res,res]: the L BRDF vectors
     of sample b share envmap b and view b, exactly the grouping of the reference's double loop
     (models/drmnet.py:680-705), in one batched launch.  ``view_from`` is [B,3] or a list of B views.  fp16 envmaps are
     rendered in place and the renderer keeps the last one in fp16 (see ``render_batch``: fp16 ends at 65504).
 
+    ``envmaps`` may also be an ``EnvmapBank`` of resident maps, with ``env_ids`` [B]: sample b uses slot ``env_ids[b]``,
+    bit for bit as ``bank.maps[env_ids]`` would.  ``env_ids`` applies to an [E,He,We,3] tensor too.
+
     Like the loop it replaces, the call leaves its mark on the stateful renderer when ``new_scene`` is false: parameters
     that are not named come from the renderer's persistent BSDF, and afterwards the renderer holds the last envmap, the
     last view and the last BRDF vector (utils/mitsuba3_utils.py:411-430 called with envmap/view only at list_idx 0)."""
-    assert len(envmaps) == z.size(1)
+    if env_ids is None:
+        assert (envmaps.B if isinstance(envmaps, EnvmapBank) else len(envmaps)) == z.size(1)
     if isinstance(envmaps, (list, tuple)):
         if isinstance(envmaps[0], str):
             # the reference's branch for names (models/drmnet.py:685-689) empties the list it iterates and cannot work;
             # EXR reading is outside the render path
             raise NotImplementedError("envmap names are not supported: pass the [He,We,3] tensors")
         envmaps = torch.stack([torch.as_tensor(e) for e in envmaps])
+    maps = envmaps.maps if isinstance(envmaps, EnvmapBank) else envmaps
+    if env_ids is not None:
+        env_ids = torch.as_tensor(env_ids).to(device=maps.device, dtype=torch.int64).reshape(-1)
+        if env_ids.numel() != z.size(1):
+            raise ValueError(f"env_ids has {env_ids.numel()} entries for a batch of {z.size(1)}")
     if isinstance(view_from, (list, tuple)):
         view_from = torch.stack([torch.as_tensor(v, dtype=torch.float32) for v in view_from])
     L, B = z.shape[0], z.shape[1]
     names = brdf_param_names or renderer.brdf_param_names
-    device = envmaps.device
+    device = maps.device
     if view_from is None:
         view = (renderer._new_scene_view if new_scene else renderer._view).to(device)[None].expand(B, 3)
     else:
@@ -58,12 +72,13 @@ def rendering_refmaps(renderer: B200RefMapRenderer, envmaps, z: torch.Tensor,
         zz, names_arg = z6, None
     else:
         names_arg = names
-    env_index = torch.arange(B, device=device).repeat_interleave(L)
+    env_index = (torch.arange(B, device=device) if env_ids is None else env_ids).repeat_interleave(L)
     out = render_batch(envmaps, zz, view.repeat_interleave(L, dim=0), env_index=env_index, brdf_param_names=names_arg,
                        flip=torch.full((B * L,), bool(flip), device=device), res=renderer.refmap_res,
                        footprint_S=renderer.footprint_S, alpha_min=renderer.alpha_min or 0.0, channel_first=True)
     if not new_scene:
-        renderer._envmap = envmaps[-1].to(renderer.device, _env_dtype(envmaps))
+        last = maps[-1] if env_ids is None else maps.index_select(0, env_ids[-1:])[0]
+        renderer._envmap = last.to(renderer.device, _env_dtype(maps))
         renderer._bsdf = zz[-1].detach().clone()
         if view_from is not None:
             renderer._view = view[-1].detach().float().cpu()
@@ -169,7 +184,8 @@ def refmap_lookup(refmap: torch.Tensor, normals: torch.Tensor, offsets: Optional
     """Shade pixels by their normals: colors [n,C] = bilinear lookup of refmap [B,C,H,W] (or [C,H,W]) at the (theta, phi)
     of normals [n,3]; image b owns rows offsets[b]:offsets[b+1].  The arithmetic of refmap2refimg_torch
     (utils/transform.py:170-198) for arbitrary object normals -- the stand-in for the reference's mesh path tracer in
-    the parametric_img2refmap flow (SURVEY 8f N3)."""
+    the parametric_img2refmap flow (SURVEY 8f N3).  For dense normal maps under a mask, ``refmap_lookup_images`` gives
+    the same colours without compacting them first."""
     if not refmap.is_cuda:
         raise RuntimeError("refmap must be a CUDA tensor: drmnet_b200 has no CPU path")
     if refmap.dim() == 3:
@@ -187,6 +203,88 @@ def refmap_lookup(refmap: torch.Tensor, normals: torch.Tensor, offsets: Optional
         _lib.check(_lib.lib().drm_refmap_lookup(refmap.data_ptr(), normals.data_ptr(), offsets.data_ptr(), n, B, C, H, W,
                                                 colors.data_ptr(), _stream(refmap.device)))
     return colors
+
+
+def refmap_lookup_images(refmap: torch.Tensor, normals: torch.Tensor, mask: Optional[torch.Tensor] = None, *,
+                         channel_first: bool) -> torch.Tensor:
+    """``refmap_lookup`` on dense normal maps under a mask, read in place: no compaction, no copy, no host
+    synchronisation (``drm_refmap_lookup_dense``).
+
+    refmap [B,C,Hr,Wr] (C in 1..4); normals [B,3,H,W] (``channel_first``) or [B,H,W,3], fp32, any strides (a permuted
+    or sliced view is read through its strides); mask [B,H,W] bool, or None for every pixel.  Returns the image
+    [B,C,H,W] (``channel_first``) or [B,H,W,C], contiguous: masked pixels hold bit for bit the colours ``refmap_lookup``
+    gives for the compacted normals ``normals_hwc[mask]``, every other pixel is 0."""
+    if not refmap.is_cuda or not normals.is_cuda:
+        raise RuntimeError("refmap and normals must be CUDA tensors: drmnet_b200 has no CPU path")
+    if normals.dtype != torch.float32:
+        raise TypeError("normals must be float32")
+    refmap = refmap.contiguous().float()
+    if refmap.dim() != 4 or normals.dim() != 4:
+        raise ValueError(f"refmap {tuple(refmap.shape)} / normals {tuple(normals.shape)}: expected [B,C,Hr,Wr] and "
+                         f"{'[B,3,H,W]' if channel_first else '[B,H,W,3]'}")
+    B, C, Hr, Wr = refmap.shape
+    if channel_first:
+        H, W = normals.shape[2], normals.shape[3]
+        dims = (0, 2, 3, 1)  # the (b, y, x, k) strides of a [B,3,H,W] tensor
+    else:
+        H, W = normals.shape[1], normals.shape[2]
+        dims = (0, 1, 2, 3)
+    if tuple(normals.shape) != ((B, 3, H, W) if channel_first else (B, H, W, 3)):
+        raise ValueError(f"normals {tuple(normals.shape)} do not match refmap {tuple(refmap.shape)}")
+    if normals.device != refmap.device:
+        raise RuntimeError(f"normals are on {normals.device}, refmap on {refmap.device}")
+    if mask is not None:
+        if mask.dtype != torch.bool:
+            raise TypeError("mask must be bool")
+        if tuple(mask.shape) != (B, H, W) or mask.device != refmap.device:
+            raise ValueError(f"mask {tuple(mask.shape)} on {mask.device}: expected [{B},{H},{W}] on {refmap.device}")
+        mask = mask.contiguous().view(torch.uint8)
+    out = torch.empty((B, C, H, W) if channel_first else (B, H, W, C), dtype=torch.float32, device=refmap.device)
+    ns = (ctypes.c_int64 * 4)(*(normals.stride(d) for d in dims))
+    os_ = (ctypes.c_int64 * 4)(*(out.stride(d) for d in dims))
+    with torch.cuda.device(refmap.device):
+        _lib.check(_lib.lib().drm_refmap_lookup_dense(refmap.data_ptr(), Hr, Wr, normals.data_ptr(), ns,
+                                                      None if mask is None else mask.data_ptr(), B, H, W, C,
+                                                      out.data_ptr(), os_, _stream(refmap.device)))
+    return out
+
+
+def obsnet_inputs(renderer: B200RefMapRenderer, zK: torch.Tensor, envmap, view_from: torch.Tensor,
+                  normals: torch.Tensor, mask: Optional[torch.Tensor], *, env_ids: Optional[torch.Tensor] = None,
+                  angle_threshold: float = math.pi / 128 / 2, noisy_observe: float = 0.0, padding_mode: str = "zeros",
+                  observe_noise: Optional[torch.Tensor] = None, padding_noise: Optional[torch.Tensor] = None):
+    """ObsNet's training inputs (models/obsnet.py:139-413) in one call on the device: no nonzero, no boolean indexing,
+    no host read, so the stream is not synchronised.
+
+    zK [B,P] (``renderer.brdf_param_names``); envmap [B,He,We,3] fp32 or fp16, or an ``EnvmapBank`` with ``env_ids``
+    [B] (``env_ids`` applies to an [E,He,We,3] tensor too); view_from [B,3]; normals [B,3,H,W] fp32 normal maps (any
+    strides); mask [B,H,W] bool (e.g. ``normals.norm(dim=1) > 0.5``), or None for every pixel.  In order:
+
+    1. LrK [B,3,res,res] = ``render_batch`` of zK, as ``synthesize_refmaps`` renders LrK (the renderer's res,
+       footprint, chosen on the device when ``renderer.footprint_S`` is None, and alpha_min);
+    2. image [B,3,H,W] = ``refmap_lookup_images(LrK, normals, mask)``: the object image, shaded by refmap lookup -- the
+       stand-in for the reference's mesh path tracer, not a render of a mesh;
+    3. raw_refmap [B,res,res,3] -> [B,3,res,res] and raw_refmask [B,res,res] bool = ``img2refmap_images(image, normals,
+       mask, res, angle_threshold)``;
+    4. cond, mask, params = ``obsnet_condition(raw_refmap, raw_refmask, ...)`` with the noise arguments as there;
+    5. LrK_transformed = ``normalized_log_apply(LrK, params)`` (models/obsnet.py:368-371).
+
+    Returns (cond [B,3,res,res], mask [B,1,res,res] float, LrK_transformed [B,3,res,res], params (log10min [B],
+    log10max [B]), raw_refmap [B,3,res,res], raw_refmask [B,res,res] bool, image [B,3,H,W])."""
+    B = zK.shape[0]
+    if env_ids is not None:
+        env_ids = torch.as_tensor(env_ids).to(device=envmap.device, dtype=torch.int64).reshape(-1)
+        if env_ids.numel() != B:
+            raise ValueError(f"env_ids has {env_ids.numel()} entries for a batch of {B}")
+    res = renderer.refmap_res
+    LrK = render_batch(envmap, zK, view_from, env_index=env_ids, brdf_param_names=renderer.brdf_param_names, res=res,
+                       footprint_S=renderer.footprint_S, alpha_min=renderer.alpha_min or 0.0, channel_first=True)
+    image = refmap_lookup_images(LrK, normals, mask, channel_first=True)
+    refmap, refmask, _, _ = img2refmap_images(image, normals, mask, res, angle_threshold, channel_first=True)
+    raw_refmap = refmap.permute(0, 3, 1, 2).contiguous()
+    cond, cmask, params = obsnet_condition(raw_refmap, refmask, noisy_observe=noisy_observe, observe_noise=observe_noise,
+                                           padding_mode=padding_mode, padding_noise=padding_noise)
+    return cond, cmask, normalized_log_apply(LrK, params), params, raw_refmap, refmask, image
 
 
 def normalized_log_transform(x: torch.Tensor, mask: torch.Tensor, lowerbound: float = 1e-6):

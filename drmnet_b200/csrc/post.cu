@@ -101,7 +101,27 @@ __global__ void mirmap2envmap_kernel(const float* __restrict__ mir, const float*
 
 // N3: shade pixels by a bilinear refmap lookup at the (theta, phi) of their normals -- the arithmetic of
 // refmap2refimg_torch (utils/transform.py:170-198: xyz2thetaphi(normal,[0,1,0],[-1,0,0]) -> uv = (phi, theta) * 2/pi - 1
-// -> grid_sample bilinear / border / align_corners=False), for arbitrary normal lists (object images), batched by offsets.
+// -> grid_sample bilinear / border / align_corners=False).  One pixel of image b (refmap b of [B, C, H, W]): store(c, v)
+// receives channel c.  Both lookup kernels inline it, so they shade a normal bit for bit alike.
+template <typename Store>
+__device__ __forceinline__ void refmap_lookup_pixel(const float* __restrict__ refmap, int b, int C, int H, int W, float x,
+                                                    float y, float z, Store store) {
+    const float th = acosf(y), ph = atan2f(z, -x + 0.f);
+    const float u = ph * (float)(2.0 / M_PI) - 1.f, v = th * (float)(2.0 / M_PI) - 1.f;
+    float ix = ((u + 1.f) * W - 1.f) * 0.5f, iy = ((v + 1.f) * H - 1.f) * 0.5f;
+    ix = fminf(fmaxf(ix, 0.f), (float)(W - 1));
+    iy = fminf(fmaxf(iy, 0.f), (float)(H - 1));
+    const float fx0 = floorf(ix), fy0 = floorf(iy);
+    const int x0 = (int)fx0, y0 = (int)fy0, x1 = min(x0 + 1, W - 1), y1 = min(y0 + 1, H - 1);
+    const float wx1 = ix - fx0, wy1 = iy - fy0, wx0 = 1.f - wx1, wy0 = 1.f - wy1;
+    for (int c = 0; c < C; ++c) {
+        const float* m = refmap + ((size_t)b * C + c) * H * W;
+        store(c, m[y0 * W + x0] * (wx0 * wy0) + m[y0 * W + x1] * (wx1 * wy0) + m[y1 * W + x0] * (wx0 * wy1) +
+                     m[y1 * W + x1] * (wx1 * wy1));
+    }
+}
+
+// compacted normal lists [total_n, 3] -> colors [total_n, C], image b owning rows offsets[b] .. offsets[b+1]-1
 __global__ void refmap_lookup_kernel(const float* __restrict__ refmap, const float* __restrict__ normals,
                                      const int64_t* __restrict__ offsets, int64_t total_n, int B, int C, int H, int W,
                                      float* __restrict__ colors) {
@@ -112,19 +132,33 @@ __global__ void refmap_lookup_kernel(const float* __restrict__ refmap, const flo
         int mid = (lo + hi) >> 1;
         if (offsets[mid] <= p) lo = mid; else hi = mid;
     }
-    const float x = normals[3 * p], y = normals[3 * p + 1], z = normals[3 * p + 2];
-    const float th = acosf(y), ph = atan2f(z, -x + 0.f);
-    const float u = ph * (float)(2.0 / M_PI) - 1.f, v = th * (float)(2.0 / M_PI) - 1.f;
-    float ix = ((u + 1.f) * W - 1.f) * 0.5f, iy = ((v + 1.f) * H - 1.f) * 0.5f;
-    ix = fminf(fmaxf(ix, 0.f), (float)(W - 1));
-    iy = fminf(fmaxf(iy, 0.f), (float)(H - 1));
-    const float fx0 = floorf(ix), fy0 = floorf(iy);
-    const int x0 = (int)fx0, y0 = (int)fy0, x1 = min(x0 + 1, W - 1), y1 = min(y0 + 1, H - 1);
-    const float wx1 = ix - fx0, wy1 = iy - fy0, wx0 = 1.f - wx1, wy0 = 1.f - wy1;
-    for (int c = 0; c < C; ++c) {
-        const float* m = refmap + ((size_t)lo * C + c) * H * W;
-        colors[p * C + c] = m[y0 * W + x0] * (wx0 * wy0) + m[y0 * W + x1] * (wx1 * wy0) + m[y1 * W + x0] * (wx0 * wy1) +
-                            m[y1 * W + x1] * (wx1 * wy1);
+    refmap_lookup_pixel(refmap, lo, C, H, W, normals[3 * p], normals[3 * p + 1], normals[3 * p + 2],
+                        [&](int c, float v) { colors[p * C + c] = v; });
+}
+
+// (b, y, x, channel) element strides of a dense image, each >= 0
+struct ImageStrides {
+    int64_t s[4];
+};
+
+// dense normal maps under a mask -> dense images: pixel (b, y, x) of B images of HW = H * W pixels.  blockIdx.y walks the
+// images (grid-stride, gridDim.y <= 65535); a pixel whose mask byte is 0 gets zeros and its normal is not read.
+__global__ void refmap_lookup_dense_kernel(const float* __restrict__ refmap, int Hr, int Wr,
+                                           const float* __restrict__ normals, ImageStrides ns,
+                                           const uint8_t* __restrict__ mask, int B, int HW, int W, int C,
+                                           float* __restrict__ out, ImageStrides os) {
+    const int64_t qq = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (qq >= HW) return;
+    const int q = (int)qq, py = q / W, px = q - py * W;
+    for (int b = blockIdx.y; b < B; b += gridDim.y) {
+        float* o = out + b * os.s[0] + py * os.s[1] + px * os.s[2];
+        if (mask && !mask[(size_t)b * HW + q]) {
+            for (int c = 0; c < C; ++c) o[c * os.s[3]] = 0.f;
+            continue;
+        }
+        const float* n = normals + b * ns.s[0] + py * ns.s[1] + px * ns.s[2];
+        refmap_lookup_pixel(refmap, b, C, Hr, Wr, n[0], n[ns.s[3]], n[2 * ns.s[3]],
+                            [&](int c, float v) { o[c * os.s[3]] = v; });
     }
 }
 
@@ -265,6 +299,36 @@ extern "C" int drm_refmap_lookup(const float* refmap, const float* normals, cons
     if (total_n == 0) return DRM_OK;
     refmap_lookup_kernel<<<(unsigned)((total_n + 255) / 256), 256, 0, static_cast<cudaStream_t>(cuda_stream)>>>(
         refmap, normals, offsets, total_n, B, C, H, W, colors);
+    DRM_CHECK_CUDA(cudaGetLastError());
+    count_launches(1);
+    return DRM_OK;
+}
+
+extern "C" int drm_refmap_lookup_dense(const float* refmap, int Hr, int Wr, const float* normals,
+                                       const int64_t normals_strides[4], const uint8_t* mask, int B, int H, int W, int C,
+                                       float* out, const int64_t out_strides[4], void* cuda_stream) {
+    DRM_REQUIRE(refmap && normals && normals_strides && out && out_strides,
+                "refmap_lookup_dense: null pointer (refmap %p, normals %p, normals_strides %p, out %p, out_strides %p)",
+                (const void*)refmap, (const void*)normals, (const void*)normals_strides, (void*)out,
+                (const void*)out_strides);
+    DRM_REQUIRE(B > 0 && H > 0 && W > 0 && Hr > 0 && Wr > 0,
+                "refmap_lookup_dense: B=%d H=%d W=%d Hr=%d Wr=%d must be positive", B, H, W, Hr, Wr);
+    DRM_REQUIRE(C >= 1 && C <= 4, "refmap_lookup_dense: C=%d not in 1..4", C);
+    DRM_REQUIRE((int64_t)H * W < (1ll << 31), "refmap_lookup_dense: H*W = %lld pixels per image, below 2^31 required",
+                (long long)H * W);
+    ImageStrides ns, os;
+    for (int k = 0; k < 4; ++k) {
+        DRM_REQUIRE(normals_strides[k] >= 0, "refmap_lookup_dense: normals_strides[%d] = %lld is negative", k,
+                    (long long)normals_strides[k]);
+        DRM_REQUIRE(out_strides[k] >= 0, "refmap_lookup_dense: out_strides[%d] = %lld is negative", k,
+                    (long long)out_strides[k]);
+        ns.s[k] = normals_strides[k];
+        os.s[k] = out_strides[k];
+    }
+    const int HW = H * W;
+    const dim3 grid((unsigned)(((int64_t)HW + 255) / 256), (unsigned)(B < 65535 ? B : 65535));
+    refmap_lookup_dense_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(cuda_stream)>>>(refmap, Hr, Wr, normals, ns, mask,
+                                                                                        B, HW, W, C, out, os);
     DRM_CHECK_CUDA(cudaGetLastError());
     count_launches(1);
     return DRM_OK;

@@ -16,6 +16,7 @@ models/drmnet.py:561-569 and :680-691.
 from __future__ import annotations
 
 import ctypes
+import functools
 import math
 from typing import List, Optional, Sequence
 
@@ -36,6 +37,14 @@ def _slots(names: Sequence[str]) -> List[int]:
                                       "(the parameters DRMNet's configs drive)")
         out.append(_SLOT[n])
     return out
+
+
+@functools.lru_cache(maxsize=None)
+def _z6_template(names: tuple, device: torch.device):
+    """The scene defaults [6] and the slots of ``names`` as tensors on ``device``, copied there once: composing z6 from
+    them needs no host-to-device copy, so a render does not synchronise the stream."""
+    return (torch.tensor(_SCENE_DEFAULTS, dtype=torch.float32, device=device),
+            torch.tensor(_slots(names), dtype=torch.int64, device=device))
 
 
 def default_alpha_min(He: int) -> float:
@@ -177,9 +186,9 @@ def render_batch(envmaps, z: torch.Tensor, view_from: torch.Tensor, *,
             raise ValueError("z must have 6 columns when brdf_param_names is not given")
         z6 = z.contiguous()
     else:
-        slots = _slots(brdf_param_names)
-        z6 = torch.tensor(_SCENE_DEFAULTS, device=device).repeat(N, 1)
-        z6[:, slots] = z[:, :len(slots)]
+        defaults, slots = _z6_template(tuple(brdf_param_names), device)
+        z6 = defaults.repeat(N, 1)
+        z6.index_copy_(1, slots, z[:, :slots.numel()])
     view_from = view_from.to(device=device, dtype=torch.float32).reshape(-1, 3)
     if view_from.shape[0] == 1 and N > 1:
         view_from = view_from.expand(N, 3)

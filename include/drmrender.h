@@ -247,9 +247,26 @@ int drm_mirmap2envmap(const float* mirmap, const float* basis, int B, int C, int
                       float* out, void* cuda_stream);
 
 /* N3: colors[p, :] = bilinear lookup of refmap[b] (refmap [B, C, H, W]) at the (theta, phi) of normals[p] for the pixels
- * p of image b (offsets [B+1] int64) -- refmap2refimg_torch (utils/transform.py:170-198) for arbitrary normal lists. */
+ * p of image b (offsets [B+1] int64) -- refmap2refimg_torch (utils/transform.py:170-198) for arbitrary normal lists.
+ * Dense normal maps go to drm_refmap_lookup_dense without compaction. */
 int drm_refmap_lookup(const float* refmap, const float* normals, const int64_t* offsets, int64_t total_n,
                       int B, int C, int H, int W, float* colors, void* cuda_stream);
+
+/* N3 on dense normal maps, read in place -- no compaction, no host read: every pixel (b, y, x) of B images of H x W
+ * pixels whose mask byte is nonzero is shaded with the arithmetic of drm_refmap_lookup (bit for bit the colours it gives
+ * for the compacted pixels), every other pixel is set to 0 in every channel.
+ *   refmap   [B, C, Hr, Wr] fp32, contiguous (device)
+ *   normals  fp32, component k of the normal of pixel (b, y, x) at normals[b*s[0] + y*s[1] + x*s[2] + k*s[3]],
+ *            s = normals_strides (elements, each >= 0: [B,H,W,3] and [B,3,H,W] views alike) (device)
+ *   mask     [B, H, W] uint8, contiguous, nonzero = shade the pixel (device); NULL = every pixel
+ *   out      fp32, channel c of pixel (b, y, x) at out[b*o[0] + y*o[1] + x*o[2] + c*o[3]], o = out_strides (each >= 0),
+ *            C in 1..4 (device)
+ * Null pointers, non-positive sizes, C outside 1..4, H*W >= 2^31 and a negative stride are refused (DRM_EINVAL) before
+ * any CUDA call; drm_last_error names the value. */
+int drm_refmap_lookup_dense(const float* refmap, int Hr, int Wr, const float* normals,
+                            const int64_t normals_strides[4], /* b, y, x, k in elements */
+                            const uint8_t* mask, int B, int H, int W, int C, float* out,
+                            const int64_t out_strides[4] /* b, y, x, c in elements */, void* cuda_stream);
 
 /* N4: ObsNet conditioning transform `0p1tom1p1_normalizedLogarithmic_lowerbound<lb>` with dynamic normalisation under a
  * mask (dataset/basedataset.py:56-76, models/obsnet.py:224,370): x [B, C, H, W], mask [B, H, W] float 0/1;
