@@ -25,11 +25,25 @@ __device__ __forceinline__ float block_sum(float v, float* sh) {
     return t;
 }
 
-// in/out: [G, N, 3, res, res]; sample n = blockIdx.x
-__global__ void __launch_bounds__(POST_THREADS) refmap_postprocess_kernel(const float* __restrict__ in, int G, int N,
-                                                                          int res, float target, int transform,
-                                                                          float* __restrict__ scale_out,
-                                                                          float* __restrict__ out) {
+// max / min that return NaN when either operand is NaN, as torch's clamp, amax and amin do (PTX max.NaN / min.NaN);
+// fmaxf / fminf return the other operand instead.  Equal to fmaxf / fminf on every other input.
+__device__ __forceinline__ float fmax_nan(float a, float b) {
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
+
+__device__ __forceinline__ float fmin_nan(float a, float b) {
+    float r;
+    asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
+
+// in/out: [G, N, 3, res, res]; sample n = blockIdx.x.  in may equal out (no __restrict__): each element is read and then
+// written by one thread, and the block has read all of its LrK (the sums end in __syncthreads) before any write.
+__global__ void __launch_bounds__(POST_THREADS) refmap_postprocess_kernel(const float* in, int G, int N, int res,
+                                                                          float target, int transform,
+                                                                          float* __restrict__ scale_out, float* out) {
     __shared__ float sh[POST_THREADS / 32];
     const int n = blockIdx.x;
     const int P = res * res;
@@ -42,6 +56,8 @@ __global__ void __launch_bounds__(POST_THREADS) refmap_postprocess_kernel(const 
             if (L > 0.f) {
                 s += logf(fmaxf(L, 1e-5f));
                 c += 1.f;
+            } else if (L != L) {
+                s += L;  // the reference's log(clip(L)) * (L > 0) is NaN * 0: the scale of the sample is NaN
             }
         }
         s = block_sum(s, sh);
@@ -49,12 +65,26 @@ __global__ void __launch_bounds__(POST_THREADS) refmap_postprocess_kernel(const 
         scale = target / expf(s / c);  // c == 0 -> NaN, as the reference's 0/0
     }
     if (scale_out && threadIdx.x == 0) scale_out[n] = scale;
+    // four loads in flight per thread before its four stores: without __restrict__ the compiler may not hoist a load
+    // above the previous iteration's store itself
+    constexpr int K = 4;
     for (int gidx = 0; gidx < G; ++gidx) {
         const size_t base = ((size_t)gidx * N + n) * 3 * P;
-        for (int e = threadIdx.x; e < 3 * P; e += POST_THREADS) {
-            float v = in[base + e] * scale;
-            if (transform == 1) v = log10f(v + 0.1f) + 1.f;
-            out[base + e] = v;
+        for (int e0 = threadIdx.x; e0 < 3 * P; e0 += K * POST_THREADS) {
+            float v[K];
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+                const int e = e0 + k * POST_THREADS;
+                if (e < 3 * P) v[k] = in[base + e];
+            }
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+                const int e = e0 + k * POST_THREADS;
+                if (e >= 3 * P) break;
+                float w = v[k] * scale;
+                if (transform == 1) w = log10f(w + 0.1f) + 1.f;
+                out[base + e] = w;
+            }
         }
     }
 }
@@ -162,13 +192,14 @@ __global__ void refmap_lookup_dense_kernel(const float* __restrict__ refmap, int
     }
 }
 
+// NaN if any thread's v is NaN, as torch's amax
 __device__ __forceinline__ float block_max(float v, float* sh) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int d = 16; d; d >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, d));
+    for (int d = 16; d; d >>= 1) v = fmax_nan(v, __shfl_xor_sync(0xffffffffu, v, d));
     if (lane == 0) sh[w] = v;
     __syncthreads();
     float t = sh[0];
-    for (int i = 1; i < POST_THREADS / 32; ++i) t = fmaxf(t, sh[i]);
+    for (int i = 1; i < POST_THREADS / 32; ++i) t = fmax_nan(t, sh[i]);
     __syncthreads();
     return t;
 }
@@ -176,6 +207,7 @@ __device__ __forceinline__ float block_max(float v, float* sh) {
 // N4: ObsNet's conditioning transform chain `0p1tom1p1_normalizedLogarithmic_lowerbound<lb>` with dynamic_normalize
 // (dataset/basedataset.py:56-76 applied right to left; models/obsnet.py:224,370): y = clip(x, lb);
 // max = amax(y * mask), min = amin(y * mask + (1 - mask) * max) per sample; out = 2 (log10 y - log10 min)/(log10 max - log10 min) - 1.
+// NaN propagates as there: a NaN in x, or +inf in x under mask 0 (inf * 0), makes the parameters and the whole sample NaN.
 __global__ void __launch_bounds__(POST_THREADS) normalized_log_kernel(const float* __restrict__ x,
                                                                       const float* __restrict__ mask, int C, int P,
                                                                       float lowerbound, float* __restrict__ out,
@@ -186,12 +218,12 @@ __global__ void __launch_bounds__(POST_THREADS) normalized_log_kernel(const floa
     const float* xs = x + (size_t)n * C * P;
     const float* ms = mask + (size_t)n * P;
     float mx = -INFINITY;
-    for (int e = threadIdx.x; e < C * P; e += POST_THREADS) mx = fmaxf(mx, fmaxf(xs[e], lowerbound) * ms[e % P]);
+    for (int e = threadIdx.x; e < C * P; e += POST_THREADS) mx = fmax_nan(mx, fmax_nan(xs[e], lowerbound) * ms[e % P]);
     mx = block_max(mx, sh);
     float mn = -INFINITY;  // max of the negated values = -min
     for (int e = threadIdx.x; e < C * P; e += POST_THREADS) {
         const float m = ms[e % P];
-        mn = fmaxf(mn, -(fmaxf(xs[e], lowerbound) * m + (1.f - m) * mx));
+        mn = fmax_nan(mn, -(fmax_nan(xs[e], lowerbound) * m + (1.f - m) * mx));
     }
     mn = -block_max(mn, sh);
     const float lmax = log10f(mx), lmin = log10f(mn);
@@ -201,7 +233,7 @@ __global__ void __launch_bounds__(POST_THREADS) normalized_log_kernel(const floa
     }
     const float inv = 1.f / (lmax - lmin);
     for (int e = threadIdx.x; e < C * P; e += POST_THREADS)
-        out[(size_t)n * C * P + e] = (log10f(fmaxf(xs[e], lowerbound)) - lmin) * inv * 2.f - 1.f;
+        out[(size_t)n * C * P + e] = (log10f(fmax_nan(xs[e], lowerbound)) - lmin) * inv * 2.f - 1.f;
 }
 
 // N4 remainder: ObsNet's conditioning (models/obsnet.py:672-691, training path :368-371).  One CTA per sample:
@@ -219,12 +251,12 @@ __global__ void __launch_bounds__(POST_THREADS) obsnet_condition_kernel(const fl
     const float* xs = x + base;
     const float* ms = mask + (size_t)n * P;
     float mx = -INFINITY;
-    for (int e = threadIdx.x; e < C * P; e += POST_THREADS) mx = fmaxf(mx, fmaxf(xs[e], lowerbound) * ms[e % P]);
+    for (int e = threadIdx.x; e < C * P; e += POST_THREADS) mx = fmax_nan(mx, fmax_nan(xs[e], lowerbound) * ms[e % P]);
     mx = block_max(mx, sh);
     float mn = -INFINITY;
     for (int e = threadIdx.x; e < C * P; e += POST_THREADS) {
         const float m = ms[e % P];
-        mn = fmaxf(mn, -(fmaxf(xs[e], lowerbound) * m + (1.f - m) * mx));
+        mn = fmax_nan(mn, -(fmax_nan(xs[e], lowerbound) * m + (1.f - m) * mx));
     }
     mn = -block_max(mn, sh);
     const float lmax = log10f(mx), lmin = log10f(mn);
@@ -235,7 +267,7 @@ __global__ void __launch_bounds__(POST_THREADS) obsnet_condition_kernel(const fl
     const float inv = 1.f / (lmax - lmin);
     for (int e = threadIdx.x; e < C * P; e += POST_THREADS) {
         const float m = ms[e % P];
-        float c = ((log10f(fmaxf(xs[e], lowerbound)) - lmin) * inv * 2.f - 1.f) * m;
+        float c = ((log10f(fmax_nan(xs[e], lowerbound)) - lmin) * inv * 2.f - 1.f) * m;
         if (n1) c = sigma * n1[base + e] + c;
         if (n2) c += (1.f - m) * n2[base + e];
         cond[base + e] = c;
@@ -243,7 +275,8 @@ __global__ void __launch_bounds__(POST_THREADS) obsnet_condition_kernel(const fl
 }
 
 // the same transform with parameters fixed by an earlier dynamic call (dynamic_normalize=False, dataset/basedataset.py:68-72)
-// and its inverse, BaseDataset.rescale (:98-110): x -> (x + 1) / 2 -> 10 ^ min(x (max - min) + min, clamp)
+// and its inverse, BaseDataset.rescale (:98-110): x -> (x + 1) / 2 -> 10 ^ min(x (max - min) + min, clamp).  A NaN element
+// stays NaN both ways, as torch's clip and clamp keep it.
 __global__ void normalized_log_apply_kernel(const float* __restrict__ x, const float* __restrict__ lmin,
                                             const float* __restrict__ lmax, int64_t per_sample, int64_t total,
                                             float lowerbound, int inverse, float clamp_before_exp, float* __restrict__ out) {
@@ -252,10 +285,10 @@ __global__ void normalized_log_apply_kernel(const float* __restrict__ x, const f
     const int n = (int)(e / per_sample);
     const float a = lmin[n], b = lmax[n];
     if (!inverse) {
-        out[e] = (log10f(fmaxf(x[e], lowerbound)) - a) / (b - a) * 2.f - 1.f;
+        out[e] = (log10f(fmax_nan(x[e], lowerbound)) - a) / (b - a) * 2.f - 1.f;
     } else {
         float y = (x[e] + 1.f) / 2.f * (b - a) + a;
-        if (clamp_before_exp != 0.f) y = fminf(y, clamp_before_exp);
+        if (clamp_before_exp != 0.f) y = fmin_nan(y, clamp_before_exp);
         out[e] = powf(10.f, y);
     }
 }

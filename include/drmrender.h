@@ -235,7 +235,8 @@ int drm_img2refmap_dense(const float* colors, const int64_t colors_strides[4], /
  * drm_refmap_postprocess: in/out [G, N, 3, res, res] fp32 (stack 0 = LrK).  target > 0: every stack of sample n is
  *   multiplied by target / geometric-mean luminance of LrK[n] over L > 0 (models/drmnet.py:610-617; 0.12 in the shipped
  *   configs), scale_out [N] receives the factor (may be NULL).  transform 1 applies log10(x + 0.1) + 1
- *   (dataset/basedataset.py:52-53), 0 none.  in may equal out.
+ *   (dataset/basedataset.py:52-53), 0 none.  in may equal out.  As in the reference, a NaN luminance in LrK[n] (and an
+ *   LrK[n] without L > 0, 0/0) makes the factor and every output of sample n NaN.
  * drm_mirmap2envmap: mirror refmap [B, C, H, W] -> lat-long envmap [B, C, OH, OW] with the defaults of
  *   utils/transform.py:106-144 (view (0,0,1), bilinear, border); basis [C, H, W] (may be NULL) divides the refmap first
  *   (DRMNet.r0toenvmap, models/drmnet.py:939-940).
@@ -270,7 +271,9 @@ int drm_refmap_lookup_dense(const float* refmap, int Hr, int Wr, const float* no
 
 /* N4: ObsNet conditioning transform `0p1tom1p1_normalizedLogarithmic_lowerbound<lb>` with dynamic normalisation under a
  * mask (dataset/basedataset.py:56-76, models/obsnet.py:224,370): x [B, C, H, W], mask [B, H, W] float 0/1;
- * log10min_out / log10max_out [B] receive the per-sample parameters (may be NULL). */
+ * log10min_out / log10max_out [B] receive the per-sample parameters (may be NULL).  NaN propagates as in the reference's
+ * clip / amax / amin: a NaN anywhere in x[b], or +inf where the mask is 0 (inf * 0), makes both parameters and all of
+ * out[b] NaN. */
 int drm_normalized_log(const float* x, const float* mask, int B, int C, int H, int W, float lowerbound,
                        float* out, float* log10min_out, float* log10max_out, void* cuda_stream);
 
@@ -278,14 +281,16 @@ int drm_normalized_log(const float* x, const float* mask, int B, int C, int H, i
  * above of raw_refmap [B, C, H, W] under raw_refmask [B, H, W] (float 0/1), then, in the reference's order,
  *   cond = t(raw) * mask;  cond = noisy_observe * observe_noise + cond (if noisy_observe > 0);
  *   cond += (1 - mask) * padding_noise (padding_mode "noise"; NULL = "zeros").
- * The noise tensors [B, C, H, W] are drawn by the caller (torch.randn_like in the reference). */
+ * The noise tensors [B, C, H, W] are drawn by the caller (torch.randn_like in the reference).  Non-finite inputs as
+ * drm_normalized_log: such a sample's parameters and cond are NaN. */
 int drm_obsnet_condition(const float* raw_refmap, const float* raw_refmask, int B, int C, int H, int W,
                          float lowerbound, float noisy_observe, const float* observe_noise, const float* padding_noise,
                          float* cond, float* log10min_out, float* log10max_out, void* cuda_stream);
 
 /* N4: the same transform with the parameters of an earlier dynamic call (dynamic_normalize=False,
  * dataset/basedataset.py:68-72; LrK at models/obsnet.py:371), inverse = 0; or BaseDataset.rescale (:98-110), inverse = 1:
- * 10 ^ min((x + 1) / 2 * (max - min) + min, clamp_before_exp) (clamp_before_exp 0 = no clamp). */
+ * 10 ^ min((x + 1) / 2 * (max - min) + min, clamp_before_exp) (clamp_before_exp 0 = no clamp).  A NaN element of x gives
+ * NaN both ways (the clip and the clamp keep it), so a NaN in a rendered LrK stays visible in its transform. */
 int drm_normalized_log_apply(const float* x, const float* log10min, const float* log10max, int B, int C, int H, int W,
                              float lowerbound, int inverse, float clamp_before_exp, float* out, void* cuda_stream);
 

@@ -37,19 +37,29 @@ def test_normalized_log_oracle_matches_reference_code():
 
 
 def test_postprocess_oracle_matches_torch_formulas():
-    """The same expressions evaluated with torch ops (models/drmnet.py:610-620, dataset/basedataset.py:52-53)."""
+    """The same expressions evaluated with torch ops (models/drmnet.py:610-620, dataset/basedataset.py:52-53), on finite
+    samples and on samples whose LrK holds NaN (scale NaN), +inf (scale 0), -inf (L < 0, excluded) or is all zero (0/0)."""
     g = torch.Generator().manual_seed(0)
-    stacks = torch.rand(3, 4, 3, 16, 16, generator=g) * 3
+    stacks = torch.rand(3, 9, 3, 16, 16, generator=g) * 3
     stacks[0, 1, :, :4] = 0  # L == 0 pixels are excluded from the mean
+    stacks[0, 4, 1, 3, 5] = float("nan")
+    stacks[0, 5, 0, 7, 7] = float("inf")
+    stacks[0, 6, 2, 2, 9] = -float("inf")
+    stacks[0, 7] = 0
+    stacks[2, 8, 0, 0, 0] = float("nan")  # outside LrK: that element only
     LrK = stacks[0]
     L = 0.212671 * LrK[:, 0] + 0.715160 * LrK[:, 1] + 0.072169 * LrK[:, 2]
     m = L > 0
     Lmean = torch.exp((torch.log(L.clip(1e-5)) * m).sum(dim=(1, 2)) / m.sum(dim=(1, 2)))
     scale = 0.12 / Lmean
     ref = torch.log10(stacks * scale[None, :, None, None, None] + 1e-1) + 1
-    ours, s = postprocess_oracle(stacks.numpy())
-    assert np.allclose(s, scale.numpy(), rtol=1e-5)
-    assert np.allclose(ours, ref.numpy(), rtol=1e-5, atol=1e-6)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        ours, s = postprocess_oracle(stacks.numpy())
+    assert np.array_equal(np.isnan(s), [False] * 4 + [True, False, False, True, False]) and s[5] == 0
+    assert np.allclose(s, scale.numpy(), rtol=1e-5, equal_nan=True)
+    assert np.array_equal(np.isnan(ours), torch.isnan(ref).numpy()) and np.isnan(ours[:, [4, 7]]).all()
+    assert np.isnan(ours[:, 8]).sum() == 1 and np.isnan(ours[:, :4]).sum() == 0
+    assert np.allclose(ours, ref.numpy(), rtol=1e-5, atol=1e-6, equal_nan=True)
 
 
 def test_refmap_lookup_oracle_matches_reference_refmap2refimg(golden_mirmap):
@@ -63,20 +73,29 @@ def test_refmap_lookup_oracle_matches_reference_refmap2refimg(golden_mirmap):
 
 
 def test_normalized_log_oracle_matches_torch_formulas():
-    """dataset/basedataset.py:56-76 evaluated with torch ops, chain lowerbound1e-6 -> normalizedLogarithmic -> 0p1tom1p1."""
+    """dataset/basedataset.py:56-76 evaluated with torch ops, chain lowerbound1e-6 -> normalizedLogarithmic -> 0p1tom1p1.
+    Samples 3-6 hold +inf in a masked cell, +inf in an unmasked one (inf * 0), NaN in a masked and in an unmasked cell:
+    torch's clip, amax and amin keep the NaN, so each of those samples is NaN throughout; sample 7 has an empty mask."""
     from oracle.callers_oracle import normalized_log_oracle
     g = torch.Generator().manual_seed(2)
-    x = torch.exp(torch.randn(3, 3, 16, 16, generator=g) * 2)
+    x = torch.exp(torch.randn(8, 3, 16, 16, generator=g) * 2)
     x[0, 0, 0, 0] = 0.0
-    mask = (torch.rand(3, 1, 16, 16, generator=g) > 0.3).float()
+    mask = (torch.rand(8, 1, 16, 16, generator=g) > 0.3).float()
+    mask[3:7, :, 5, 6], mask[3:7, :, 7, 8], mask[7] = 1, 0, 0
+    x[3, 2, 5, 6], x[4, 0, 7, 8], x[5, 0, 5, 6], x[6, 2, 7, 8] = float("inf"), float("inf"), float("nan"), float("nan")
     y = torch.clip(x, 1e-6)
     linearmax = (y * mask).amax(dim=(-1, -2, -3), keepdim=True)
     log10max = torch.log10(linearmax)
     log10min = torch.log10((y * mask + (1 - mask) * linearmax).amin(dim=(-1, -2, -3), keepdim=True))
     ref = (torch.log10(y) - log10min) / (log10max - log10min) * 2 - 1
-    ours, lmin, lmax = normalized_log_oracle(x.numpy(), mask.numpy())
-    assert np.allclose(ours, ref.numpy(), rtol=1e-5, atol=1e-5)
-    assert np.allclose(lmin, log10min.reshape(-1).numpy(), atol=1e-6) and np.allclose(lmax, log10max.reshape(-1).numpy(), atol=1e-6)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        ours, lmin, lmax = normalized_log_oracle(x.numpy(), mask.numpy())
+    assert torch.isnan(ref[3:8]).all() and not torch.isnan(ref[:3]).any() and np.isnan(lmin[3:7]).all()
+    assert np.isneginf(lmin[7]) and np.isneginf(lmax[7])
+    assert np.array_equal(np.isnan(ours), torch.isnan(ref).numpy())
+    assert np.allclose(ours, ref.numpy(), rtol=1e-5, atol=1e-5, equal_nan=True)
+    assert np.allclose(lmin, log10min.reshape(-1).numpy(), atol=1e-6, equal_nan=True)
+    assert np.allclose(lmax, log10max.reshape(-1).numpy(), atol=1e-6, equal_nan=True)
 
 
 def test_obsnet_condition_oracles_match_reference_code():
